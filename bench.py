@@ -31,7 +31,6 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 METRIC = "decoded_ascii_GBps"
 UNIT = "GB/s"
-CACHE = os.environ.get("NAFBENCH_CACHE", "/tmp/nafbench_cache")
 
 
 def log(*a):
@@ -53,16 +52,7 @@ def emit(line: dict):
 # workload: cfg2 archives, generated with the oracle's restatement of the reference encoder (+ mask section)
 def make_archive(seed, n_res, level):
     import _cases as K
-    os.makedirs(CACHE, exist_ok=True)
-    path = os.path.join(CACHE, f"cfg2_s{seed}_n{n_res}_l{level}.naf")
-    if os.path.exists(path):
-        return open(path, "rb").read()
-    data = K.genome(seed, n_res, level=level, mask=True, records=1)
-    tmp = path + f".{os.getpid()}.tmp"
-    with open(tmp, "wb") as f:
-        f.write(data)
-    os.replace(tmp, path)
-    return data
+    return K.cached(f"cfg2_s{seed}_n{n_res}_l{level}.naf", lambda: K.genome(seed, n_res, level=level, mask=True, records=1))[0]
 
 
 def make_workload(unique, n_res, level, rank):
@@ -165,28 +155,42 @@ def workload_config(args, batch):
             "l2": "batch working set (compressed + packed + ASCII) exceeds the 126 MB L2; device-resident timing also overwrites a 256 MB buffer before every timed iteration"}
 
 
+DUMP_SEED = 20261020
+DUMP_SEQUENCE_SAMPLES = 8 << 20            # float32: 32 MiB, the largest of the files
+
+
+def dump_outputs(out_dir, results):
+    """What a caller of the timed decode receives for the batch, as exact float arrays: n_records per archive, every record
+    length (float64), the ids and comments blobs (NUL-terminated, archives concatenated) and the sequence bytes of each
+    archive, whole if it fits its share of DUMP_SEQUENCE_SAMPLES, else at a fixed seeded sample of positions (the batch is
+    1.28 GB of ASCII at the default sizes; float32)."""
+    import numpy as np
+
+    def view(ptr, n, ctype):
+        return np.ctypeslib.as_array(C.cast(ptr, C.POINTER(ctype)), shape=(n,)) if ptr and n else np.zeros(0, np.dtype(ctype))
+
+    n_arc = len(results)
+    per_archive = DUMP_SEQUENCE_SAMPLES // n_arc
+    out = {"n_records": [], "lengths": [], "ids": [], "comments": [], "sequence_sample": []}
+    for i, r in enumerate(results):
+        assert r.status == 0, (i, r.status)
+        out["n_records"].append(np.array([r.n_records], np.float64))
+        out["lengths"].append(view(r.lengths, r.n_lengths, C.c_uint64).astype(np.float64))
+        for name, blob, offsets, n in (("ids", r.ids, r.id_offsets, r.n_ids), ("comments", r.comments, r.comment_offsets, r.n_comments)):
+            size = int(view(offsets, n + 1, C.c_uint64)[-1]) if blob else 0
+            out[name].append(view(blob, size, C.c_uint8).astype(np.float32))
+        seq = view(r.sequence, r.total_residues, C.c_uint8)
+        if len(seq) > per_archive:
+            seq = seq[np.sort(np.random.default_rng([DUMP_SEED, i]).integers(0, len(seq), size=per_archive))]
+        out["sequence_sample"].append(seq.astype(np.float32))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, parts in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.concatenate(parts))
+    log(f"[dump] {len(out)} arrays of the last timed step written to {out_dir}")
+
 
 # ------------------------------------------------------------------------------------------------------------------
 # BASELINE.json configs at their stated sizes, each: parity gate vs the oracle, host prepare, device time, roofline, e2e
-BENCH_CACHE = os.path.join(ROOT, "bench_cache")          # in-tree, git-ignored: travels to the GPU box with the snapshot
-
-
-def cached(name, make):
-    """Archives that take minutes to generate (250 Mbp at zstd level 19: ~3 min on one core) are kept in bench_cache/."""
-    for d in (BENCH_CACHE, CACHE):
-        path = os.path.join(d, name)
-        if os.path.exists(path):
-            return open(path, "rb").read(), f"cached ({os.path.relpath(path, ROOT) if d == BENCH_CACHE else path})"
-    t0 = time.perf_counter()
-    data = make()
-    os.makedirs(CACHE, exist_ok=True)
-    tmp = os.path.join(CACHE, name + f".{os.getpid()}.tmp")
-    with open(tmp, "wb") as f:
-        f.write(data)
-    os.replace(tmp, os.path.join(CACHE, name))
-    return data, f"generated in {time.perf_counter() - t0:.0f} s"
-
-
 def pin(lib, blobs):
     """Pinned host copies + parsed archive structs (the e2e legs copy from pinned memory)."""
     from nafcodec_b200 import _ffi
@@ -311,7 +315,7 @@ def run_configs(args, ctx, lib, peak, uniq_cfg2):
     if args.cfg3_residues > 0:
         def cfg3():
             nm = f"cfg3_n{args.cfg3_residues}_s3_l19.naf"
-            data, how = cached(nm, lambda: K.cfg3_chromosome(args.cfg3_residues, workers=0))
+            data, how = K.cached(nm, lambda: K.cfg3_chromosome(args.cfg3_residues, workers=0))
             r = measure_config(ctx, lib, "cfg3", [data], want, peak, ALL,
                                f"cfg3: synthetic {args.cfg3_residues / 1e6:g} Mbp chromosome, ONE record / one zstd frame per section, level 19 (8 MiB window), "
                                f"N telomeres + centromere + 20 gaps, ~50 % soft-masked (mean run 300); archive {how}", iters=5)
@@ -330,7 +334,7 @@ def run_configs(args, ctx, lib, peak, uniq_cfg2):
         def cfg5():
             t0 = time.perf_counter()
             with ThreadPoolExecutor(max_workers=os.cpu_count() or 1) as ex:
-                blobs = list(ex.map(lambda i: cached(f"cfg5_i{i}_l19.naf", lambda: K.cfg5_member(i))[0], range(args.cfg5_archives)))
+                blobs = list(ex.map(lambda i: K.cached(f"cfg5_i{i}_l19.naf", lambda: K.cfg5_member(i))[0], range(args.cfg5_archives)))
             gen_s = time.perf_counter() - t0
             r = measure_config(ctx, lib, "cfg5", blobs, want, peak, ALL,
                                f"cfg5: RefSeq-collection shape, {args.cfg5_archives} UNIQUE archives in one job (of the 20 000 / 8 GPUs = 2500 per GPU), N uniform 2-6 Mbp, "
@@ -356,6 +360,8 @@ def main():
     ap.add_argument("--cfg4-reads", type=int, default=1_000_000, help="configs[3]: FASTQ reads (BASELINE says 10 M: 450 MB archive, ~2 min to generate; 0 = skip)")
     ap.add_argument("--cfg5-archives", type=int, default=512, help="configs[4]: unique 2-6 Mbp archives in one job (0 = skip)")
     ap.add_argument("--no-configs", action="store_true", help="only the headline workload (cfg2 x batch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step decoded (rank 0) to DIR/<name>.npy, "
+                                                          "so that two builds can be compared output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
@@ -429,7 +435,9 @@ def main():
     dev_ms = ctx.time_runs(args.steps, True)
     barrier()
     dev_ms = max_over_ranks(dev_ms)
-    ctx.fetch_raw()                        # (outside the timed region) brings back the LZ round statistics of the last run
+    res = ctx.fetch_raw()                  # (outside the timed region) the last run's results and its LZ round statistics
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res)
     st = ctx.stats()                       # kernel_launches is filled by the runs
     lz_rounds = int(st.lz_rounds)
     ascii_bytes = st.ascii_bytes

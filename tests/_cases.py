@@ -1,9 +1,36 @@
 """Parity archives produced by the oracle's restatement of the reference encoder (deterministic)."""
+import os
 import struct
+import tempfile
+import time
 
 import numpy as np
 
 import _oracle as O
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+TREE_CACHE = os.path.join(ROOT, "bench_cache")
+# Per user: on a shared host another user's cache directory would be unwritable, and its archives not ours to trust.
+CACHE = os.environ.get("NAFBENCH_CACHE") or os.path.join(tempfile.gettempdir(), f"nafbench_cache_{os.getuid()}")
+
+
+def cached(name, make):
+    """(archive, where it came from).  Archives that take minutes to generate (250 Mbp at zstd level 19: ~3 min on one core)
+    are read from bench_cache/ in the tree when someone put them there, else from CACHE, else generated into CACHE.  A new
+    file is written under a temporary name and renamed, so an interrupted run leaves no truncated archive behind."""
+    for d in (TREE_CACHE, CACHE):
+        path = os.path.join(d, name)
+        if os.path.exists(path):
+            with open(path, "rb") as f:
+                return f.read(), f"cached ({os.path.relpath(path, ROOT) if d == TREE_CACHE else path})"
+    t0 = time.perf_counter()
+    data = make()
+    os.makedirs(CACHE, exist_ok=True)
+    tmp = os.path.join(CACHE, f"{name}.{os.getpid()}.tmp")
+    with open(tmp, "wb") as f:
+        f.write(data)
+    os.replace(tmp, os.path.join(CACHE, name))
+    return data, f"generated in {time.perf_counter() - t0:.0f} s"
 
 
 def _rng(seed):
