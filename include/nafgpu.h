@@ -270,6 +270,48 @@ int nafgpu_pack(nafgpu_ctx* ctx, const nafgpu_pack_input* in, nafgpu_pack_result
 /* Device pointers of the last run's outputs, for callers that keep results in HBM (device-resident variant). */
 int nafgpu_job_device_result(nafgpu_ctx* ctx, uint32_t archive, const uint8_t** sequence_dev, uint64_t* capacity_bytes);
 
+/* ---- device-resident export -------------------------------------------------------------------------------------------
+ * The decoded job, from the context's arena into DEVICE memory the caller owns, as tokens: every decoded byte goes through a
+ * 256-entry table (identity = ASCII; the soft mask is the case of the ASCII).  Records are numbered across the job: archive 0's
+ * n_lengths records first, then archive 1's, and so on; an archive whose status is nonzero contributes none.
+ * After nafgpu_job_run; the job stays in device memory until the next prepare / run on the context, so one decode serves
+ * any number of exports. */
+
+/* Per-archive counters of the job that was run (read once per run: one small D2H and a synchronise, as for
+ * nafgpu_job_fetch_window). */
+typedef struct nafgpu_counts {
+    uint64_t n_records, n_ids, n_comments, n_lengths, total_residues;
+    uint64_t id_bytes, comment_bytes;     /* decoded size of the ids / comments streams: what a FLAT export of that field writes */
+    uint64_t first_bad_record;            /* as in nafgpu_result */
+    int32_t record_status, status;        /* as in nafgpu_result: a failed archive has status != 0 and contributes no records */
+} nafgpu_counts;
+int nafgpu_job_counts(nafgpu_ctx* ctx, nafgpu_counts* out, uint32_t n);
+
+/* FLAT    one field of every archive, concatenated in job order: sequence / quality total_residues bytes per archive, ids /
+ *         comments id_bytes / comment_bytes (NUL-terminated strings).  An archive without that section contributes no bytes.
+ * ROWS    uint8 [n_rows, row_length]: row i holds residues [start, start + row_length) of job record `record` of the sequence or
+ *         quality, for (record, start) = rows[2i], rows[2i + 1]; `pad` past the record's end.  A row whose record is out of
+ *         range or lacks the field, or whose start is negative or not below the record's length, is all `pad`.
+ * OFFSETS int64 [N + 1] job-global exclusive record offsets (N = the job's records); lengths are their differences. */
+enum { NAFGPU_EXPORT_FLAT = 0, NAFGPU_EXPORT_ROWS = 1, NAFGPU_EXPORT_OFFSETS = 2 };
+typedef struct nafgpu_export {
+    int32_t field;                 /* NAFGPU_SEC_ID | _COMMENT | _SEQUENCE | _QUALITY (FLAT); _SEQUENCE | _QUALITY (ROWS); ignored (OFFSETS) */
+    int32_t layout;
+    uint8_t table[256];            /* out byte = table[decoded byte]; by value, so no copy and no lifetime */
+    uint8_t pad;                   /* ROWS */
+    uint8_t _pad[7];
+    void* out;                     /* DEVICE memory of the caller (8-byte aligned for OFFSETS) */
+    uint64_t out_bytes;            /* its capacity: checked against what the export writes */
+    const int64_t* rows;           /* DEVICE, ROWS: n_rows (record, start) pairs */
+    uint64_t n_rows, row_length;
+} nafgpu_export;
+/* Enqueues the export on `stream` (a cudaStream_t; NULL = the context's stream).  The kernels wait for the job's run (an event
+ * on the context's stream), and the context's next call waits for them (an event on `stream`), so the caller may prepare
+ * the next job right away.  Asynchronous: no host sync unless the counters have not been read for this run yet.
+ * NAFGPU_ERR_ARGUMENT: no run, a field that was not requested (want bits), ROWS of ids / comments, out_bytes too small,
+ * rows NULL with n_rows > 0.  An empty job, or an archive without records, exports zero bytes (OFFSETS: the one entry 0). */
+int nafgpu_job_export(nafgpu_ctx* ctx, const nafgpu_export* spec, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

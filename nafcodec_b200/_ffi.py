@@ -19,6 +19,8 @@ N_SECTIONS = 6
 NO_RECORD = 2 ** 64 - 1
 TEXT_AUTO, TEXT_FASTA, TEXT_FASTQ = 0, 1, 2
 LINE_LENGTH_FROM_HEADER = 2 ** 64 - 1
+SEC_ID, SEC_COMMENT, SEC_LENGTH, SEC_MASK, SEC_SEQUENCE, SEC_QUALITY = range(6)
+EXPORT_FLAT, EXPORT_ROWS, EXPORT_OFFSETS = 0, 1, 2
 
 
 class Header(C.Structure):
@@ -69,13 +71,25 @@ class JobStats(C.Structure):
                 ("lz_flow", C.c_uint32), ("_pad", C.c_uint32)]
 
 
+class Counts(C.Structure):
+    _fields_ = [("n_records", C.c_uint64), ("n_ids", C.c_uint64), ("n_comments", C.c_uint64), ("n_lengths", C.c_uint64),
+                ("total_residues", C.c_uint64), ("id_bytes", C.c_uint64), ("comment_bytes", C.c_uint64),
+                ("first_bad_record", C.c_uint64), ("record_status", C.c_int32), ("status", C.c_int32)]
+
+
+class Export(C.Structure):
+    _fields_ = [("field", C.c_int32), ("layout", C.c_int32), ("table", C.c_uint8 * 256), ("pad", C.c_uint8), ("_pad", C.c_uint8 * 7),
+                ("out", C.c_void_p), ("out_bytes", C.c_uint64), ("rows", C.c_void_p), ("n_rows", C.c_uint64), ("row_length", C.c_uint64)]
+
+
 # every symbol include/nafgpu.h declares (tests check the library exports all of them)
 SYMBOLS = ["nafgpu_parse_archive", "nafgpu_variable_u64", "nafgpu_strerror", "nafgpu_version", "nafgpu_ctx_create",
            "nafgpu_ctx_destroy", "nafgpu_last_error", "nafgpu_host_alloc", "nafgpu_host_free", "nafgpu_decode",
            "nafgpu_decode_batch", "nafgpu_job_prepare", "nafgpu_job_run", "nafgpu_job_fetch", "nafgpu_job_fetch_window", "nafgpu_job_sync",
            "nafgpu_job_get_stats", "nafgpu_job_time", "nafgpu_job_run_profiled", "nafgpu_stage_name",
            "nafgpu_job_device_result", "nafgpu_zstd_decompress", "nafgpu_job_format", "nafgpu_format_batch", "nafgpu_pack", "nafgpu_pipeline_create", "nafgpu_pipeline_destroy", "nafgpu_pipeline_submit",
-           "nafgpu_pipeline_wait", "nafgpu_pipeline_release", "nafgpu_pipeline_last_error", "nafgpu_pipeline_lanes", "nafgpu_pipeline_lane_stats"]
+           "nafgpu_pipeline_wait", "nafgpu_pipeline_release", "nafgpu_pipeline_last_error", "nafgpu_pipeline_lanes", "nafgpu_pipeline_lane_stats",
+           "nafgpu_job_counts", "nafgpu_job_export"]
 
 
 class Library:
@@ -130,6 +144,8 @@ class Library:
         L.nafgpu_pipeline_lane_stats.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(JobStats)]
         L.nafgpu_pack.argtypes = [C.c_void_p, C.POINTER(PackInput), C.POINTER(PackResult)]
         L.nafgpu_job_device_result.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
+        L.nafgpu_job_counts.argtypes = [C.c_void_p, C.POINTER(Counts), C.c_uint32]
+        L.nafgpu_job_export.argtypes = [C.c_void_p, C.POINTER(Export), C.c_void_p]
 
     def strerror(self, code):
         return self.dll.nafgpu_strerror(code).decode()

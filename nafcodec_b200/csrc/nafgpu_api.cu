@@ -21,6 +21,7 @@
 #include "../../include/nafgpu.h"
 #include "cuda_compat.h"
 #include "frame_walk.h"
+#include "naf_export.cuh"
 #include "naf_kernels.cuh"
 #include "naf_pack.cuh"
 #include "naf_text.cuh"
@@ -192,6 +193,16 @@ struct nafgpu_ctx {
     bool prepared = false, ran = false;
     bool win_counts = false;           // counts + status of the last run are on the host (windowed fetch)
     PinBuf win;                        // the current window of a job that is read in windows (nafgpu_job_fetch_window)
+    uint32_t want = 0;                 // the want bits of the prepared job
+    // device-resident export (nafgpu_job_export): the archives' counters and the export descriptors of the last run, built and
+    // uploaded once per run by the first export: [ExpRec x n_exp_rec | ExpSpan x n_exp_span[f] for ids, comments, sequence, quality]
+    bool exp_ready = false;
+    std::vector<nafgpu_counts> counts;
+    DevBuf exp_desc;
+    PinBuf exp_stage;
+    uint32_t n_exp_rec = 0, n_exp_span[4] = {0, 0, 0, 0};
+    uint64_t o_exp_span[4] = {0, 0, 0, 0}, exp_bytes[4] = {0, 0, 0, 0}, exp_records = 0, exp_residues = 0;
+    cudaEvent_t ev_exp_ready = nullptr, ev_exp_done = nullptr;
     cudaEvent_t ev[N_STAGES + 3];
     bool ev_ok = false;
 #if !defined(NAFGPU_EMULATE)
@@ -235,6 +246,7 @@ int enqueue_run(nafgpu_ctx* c, StageEvents* ev) {
     CUDA_TRY(c, cudaGetLastError());
     c->ran = true;
     c->win_counts = false;
+    c->exp_ready = false;
     return NAFGPU_OK;
 }
 
@@ -527,6 +539,76 @@ int archive_status(nafgpu_ctx* c, uint32_t a, std::string& msg) {
     return status_to_code(s & ~zc::E_UTF8, msg);
 }
 
+// Status words and the archives' counters of the last run on the host, once per run (a synchronise on the context's stream).
+int read_counts(nafgpu_ctx* c) {
+    if (c->win_counts) return NAFGPU_OK;
+    CUDA_TRY(c, wait_stream(c));
+    CUDA_TRY(c, cudaMemcpyAsync(c->misc_host.p, c->misc.p, c->misc_words * 4, cudaMemcpyDeviceToHost, c->st));
+    CUDA_TRY(c, cudaMemcpyAsync(c->result.p, c->arena.p, c->counts_size, cudaMemcpyDeviceToHost, c->st));
+    CUDA_TRY(c, cudaStreamSynchronize(c->st));
+    read_lz_stats(c);
+    c->win_counts = true;
+    return NAFGPU_OK;
+}
+
+// The counters of every archive and the export descriptors of the last run (include/nafgpu.h, nafgpu_job_export): built on the
+// host from the counters and uploaded in one copy on the context's stream.  They stay unchanged until the next run, which the
+// context's stream only starts once the exports that read them are done.
+int export_tables(nafgpu_ctx* c) {
+    if (c->exp_ready) return NAFGPU_OK;
+    { int rc = read_counts(c); if (rc) return rc; }
+    const uint32_t n = (uint32_t)c->arch.size();
+    c->counts.assign(n, nafgpu_counts());
+    std::vector<nk::ExpRec> recs;
+    std::vector<nk::ExpSpan> spans[4];
+    uint64_t records = 0, residues = 0, bytes[4] = {0, 0, 0, 0};
+    for (uint32_t a = 0; a < n; a++) {
+        const nk::NafDev& D = c->arch[a];
+        const ArchPlan& P = c->aplan[a];
+        const nk::NafCounts* C = (const nk::NafCounts*)((const uint8_t*)c->result.p + D.counts_off);
+        nafgpu_counts& k = c->counts[a];
+        memset(&k, 0, sizeof k);
+        k.n_records = P.n_records;
+        k.first_bad_record = nk::NO_RECORD;
+        std::string msg;
+        k.status = archive_status(c, a, msg);
+        if (k.status) continue;
+        k.n_ids = P.dec[0] ? std::min<uint64_t>(C->n_ids, P.n_records) : 0;
+        k.n_comments = P.dec[1] ? std::min<uint64_t>(C->n_comments, P.n_records) : 0;
+        k.n_lengths = P.dec[2] ? C->n_lengths : 0;
+        k.total_residues = P.dec[2] ? C->total_residues : 0;
+        k.id_bytes = P.dec[0] ? D.ids_size : 0;
+        k.comment_bytes = P.dec[1] ? D.com_size : 0;
+        k.first_bad_record = C->first_bad_record;
+        k.record_status = (C->first_bad_record != nk::NO_RECORD) ? NAFGPU_ERR_UTF8 : 0;
+        if (k.n_lengths)
+            recs.push_back({records, residues, D.rec_offsets_off, {P.dec[4] ? D.ascii_off : nk::NO_FIELD, P.dec[5] ? D.qual_off : nk::NO_FIELD}, 0});
+        const uint64_t field_bytes[4] = {k.id_bytes, k.comment_bytes, P.dec[4] ? k.total_residues : 0, P.dec[5] ? k.total_residues : 0};
+        const uint64_t field_off[4] = {D.ids_off, D.com_off, D.ascii_off, D.qual_off};
+        for (int f = 0; f < 4; f++) {
+            if (!field_bytes[f]) continue;
+            spans[f].push_back({bytes[f], field_off[f]});
+            bytes[f] += field_bytes[f];
+        }
+        records += k.n_lengths;
+        residues += k.total_residues;
+    }
+    uint64_t off = align_up(recs.size() * sizeof(nk::ExpRec), 16);
+    for (int f = 0; f < 4; f++) { c->o_exp_span[f] = off; off += align_up(spans[f].size() * sizeof(nk::ExpSpan), 16); }
+    if (!c->exp_desc.ensure(off + 64)) return fail(c, NAFGPU_ERR_NOMEM, "device allocation failed");
+    if (!c->exp_stage.ensure(off + 64)) return fail(c, NAFGPU_ERR_NOMEM, "pinned host allocation failed");
+    uint8_t* S = (uint8_t*)c->exp_stage.p;       // (free: the stream was synchronised above, after the last copy from it)
+    if (!recs.empty()) memcpy(S, recs.data(), recs.size() * sizeof(nk::ExpRec));
+    for (int f = 0; f < 4; f++) if (!spans[f].empty()) memcpy(S + c->o_exp_span[f], spans[f].data(), spans[f].size() * sizeof(nk::ExpSpan));
+    if (off) CUDA_TRY(c, cudaMemcpyAsync(c->exp_desc.p, S, off, cudaMemcpyHostToDevice, c->st));
+    c->n_exp_rec = (uint32_t)recs.size();
+    for (int f = 0; f < 4; f++) { c->n_exp_span[f] = (uint32_t)spans[f].size(); c->exp_bytes[f] = bytes[f]; }
+    c->exp_records = records;
+    c->exp_residues = residues;
+    c->exp_ready = true;
+    return NAFGPU_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -549,6 +631,7 @@ int nafgpu_ctx_create(int device, nafgpu_ctx** out) {
     if (cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming) != cudaSuccess) { delete c; return NAFGPU_ERR_CUDA; }
     if (cudaEventCreateWithFlags(&c->ev_block, cudaEventDisableTiming | cudaEventBlockingSync) != cudaSuccess) { c->ev_block = nullptr; cudaGetLastError(); }
     if (cudaEventCreateWithFlags(&c->ev_d2h, cudaEventDisableTiming) != cudaSuccess) { c->ev_d2h = nullptr; cudaGetLastError(); }
+    if (cudaEventCreateWithFlags(&c->ev_exp_ready, cudaEventDisableTiming) != cudaSuccess || cudaEventCreateWithFlags(&c->ev_exp_done, cudaEventDisableTiming) != cudaSuccess) { delete c; return NAFGPU_ERR_CUDA; }
     for (int i = 0; i < N_STAGES + 3; i++) if (cudaEventCreate(&c->ev[i]) != cudaSuccess) { delete c; return NAFGPU_ERR_CUDA; }
     c->ev_ok = true;
     c->coop_ctas = zk::lz_resolve_max_ctas(device);
@@ -562,9 +645,12 @@ void nafgpu_ctx_destroy(nafgpu_ctx* c) {
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->st);
     drop_graph(c);
-    DevBuf* d[] = {&c->comp, &c->arena, &c->lit, &c->desc, &c->bstate, &c->hufw, &c->fsstate, &c->lzidx, &c->scanagg, &c->debug, &c->tables, &c->table_al, &c->seq32, &c->seq64, &c->misc, &c->flush, &c->text, &c->fin_g, &c->pack_in, &c->pack_out};
+    DevBuf* d[] = {&c->comp, &c->arena, &c->lit, &c->desc, &c->bstate, &c->hufw, &c->fsstate, &c->lzidx, &c->scanagg, &c->debug, &c->tables, &c->table_al, &c->seq32, &c->seq64, &c->misc, &c->flush, &c->text, &c->fin_g, &c->pack_in, &c->pack_out, &c->exp_desc};
     for (DevBuf* b : d) b->release();
     c->stage.release(); c->result.release(); c->misc_host.release(); c->text_host.release(); c->text_stage.release(); c->pack_host.release(); c->win.release();
+    c->exp_stage.release();
+    if (c->ev_exp_ready) cudaEventDestroy(c->ev_exp_ready);
+    if (c->ev_exp_done) cudaEventDestroy(c->ev_exp_done);
     if (c->ev_ok) for (int i = 0; i < N_STAGES + 3; i++) cudaEventDestroy(c->ev[i]);
     if (c->ev_fork) cudaEventDestroy(c->ev_fork);
     if (c->ev_join) cudaEventDestroy(c->ev_join);
@@ -600,6 +686,7 @@ int nafgpu_job_prepare(nafgpu_ctx* c, const nafgpu_archive* archives, uint32_t n
     CUDA_TRY(c, cudaStreamSynchronize(c->st));
     c->prepared = false; c->ran = false;
     drop_graph(c);
+    c->want = want;
     c->plan.clear();
     c->arch.assign(n, nk::NafDev());
     c->aplan.assign(n, ArchPlan());
@@ -914,6 +1001,7 @@ int nafgpu_zstd_decompress(nafgpu_ctx* c, const uint8_t* frame, uint64_t frame_s
     CUDA_TRY(c, cudaStreamSynchronize(c->st));
     c->prepared = false; c->ran = false;
     drop_graph(c);
+    c->want = 0;
     c->plan.clear(); c->arch.clear(); c->aplan.clear();
     memset(&c->stats, 0, sizeof c->stats);
     c->counts_size = ALIGN;
@@ -1271,14 +1359,7 @@ int nafgpu_job_fetch_window(nafgpu_ctx* c, uint32_t archive, uint64_t first, uin
     if (!c->prepared || !c->ran) return fail(c, NAFGPU_ERR_ARGUMENT, "job has not been run");
     if (archive >= c->arch.size()) return fail(c, NAFGPU_ERR_ARGUMENT, "bad archive index");
     CUDA_TRY(c, cudaSetDevice(c->device));
-    if (!c->win_counts) {                // once per run: status words and the archives' counters
-        CUDA_TRY(c, wait_stream(c));
-        CUDA_TRY(c, cudaMemcpyAsync(c->misc_host.p, c->misc.p, c->misc_words * 4, cudaMemcpyDeviceToHost, c->st));
-        CUDA_TRY(c, cudaMemcpyAsync(c->result.p, c->arena.p, c->counts_size, cudaMemcpyDeviceToHost, c->st));
-        CUDA_TRY(c, cudaStreamSynchronize(c->st));
-        read_lz_stats(c);
-        c->win_counts = true;
-    }
+    { int rc = read_counts(c); if (rc) return rc; }
     const nk::NafDev& D = c->arch[archive];
     const ArchPlan& P = c->aplan[archive];
     const nk::NafCounts* C = (const nk::NafCounts*)((const uint8_t*)c->result.p + D.counts_off);
@@ -1363,6 +1444,70 @@ int nafgpu_job_device_result(nafgpu_ctx* c, uint32_t archive, const uint8_t** se
     if (!c->prepared || archive >= c->arch.size()) return fail(c, NAFGPU_ERR_ARGUMENT, "bad archive index");
     *sequence_dev = (const uint8_t*)c->arena.p + c->arch[archive].ascii_off;
     *capacity_bytes = c->arch[archive].seq_residues;
+    return NAFGPU_OK;
+}
+
+int nafgpu_job_counts(nafgpu_ctx* c, nafgpu_counts* out, uint32_t n) {
+    if (!c || (!out && n)) return NAFGPU_ERR_ARGUMENT;
+    if (!c->prepared || !c->ran) return fail(c, NAFGPU_ERR_ARGUMENT, "job has not been run");
+    if (n != c->arch.size()) return fail(c, NAFGPU_ERR_ARGUMENT, "count differs from the prepared job");
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    { int rc = export_tables(c); if (rc) return rc; }
+    if (n) memcpy(out, c->counts.data(), (size_t)n * sizeof(nafgpu_counts));
+    return NAFGPU_OK;
+}
+
+int nafgpu_job_export(nafgpu_ctx* c, const nafgpu_export* spec, void* stream) {
+    if (!c || !spec) return NAFGPU_ERR_ARGUMENT;
+    if (!c->prepared || !c->ran) return fail(c, NAFGPU_ERR_ARGUMENT, "job has not been run");
+    const int field = spec->field, layout = spec->layout;
+    if (layout != NAFGPU_EXPORT_FLAT && layout != NAFGPU_EXPORT_ROWS && layout != NAFGPU_EXPORT_OFFSETS) return fail(c, NAFGPU_ERR_ARGUMENT, "bad export layout");
+    int f = -1;                                         // index of the field among ids, comments, sequence, quality
+    if (layout != NAFGPU_EXPORT_OFFSETS) {
+        static const int fields[4] = {NAFGPU_SEC_ID, NAFGPU_SEC_COMMENT, NAFGPU_SEC_SEQUENCE, NAFGPU_SEC_QUALITY};
+        static const uint32_t want_bit[4] = {NAFGPU_WANT_ID, NAFGPU_WANT_COMMENT, NAFGPU_WANT_SEQUENCE, NAFGPU_WANT_QUALITY};
+        for (int k = 0; k < 4; k++) if (field == fields[k]) f = k;
+        if (f < 0) return fail(c, NAFGPU_ERR_ARGUMENT, "bad export field");
+        if (layout == NAFGPU_EXPORT_ROWS && f < 2) return fail(c, NAFGPU_ERR_ARGUMENT, "rows export of ids or comments: only sequence and quality have residues");
+        if (!(c->want & want_bit[f])) return fail(c, NAFGPU_ERR_ARGUMENT, "export of a field that was not decoded (want bits of the job)");
+    }
+    if (layout == NAFGPU_EXPORT_ROWS && !spec->rows && spec->n_rows) return fail(c, NAFGPU_ERR_ARGUMENT, "rows export without a row table");
+    if (layout == NAFGPU_EXPORT_ROWS && spec->row_length && spec->n_rows > UINT64_MAX / spec->row_length) return fail(c, NAFGPU_ERR_ARGUMENT, "rows export larger than 2^64 bytes");
+    if (layout == NAFGPU_EXPORT_OFFSETS && ((uintptr_t)spec->out & 7)) return fail(c, NAFGPU_ERR_ARGUMENT, "offsets export: out must be 8-byte aligned");
+    CUDA_TRY(c, cudaSetDevice(c->device));
+    { int rc = export_tables(c); if (rc) return rc; }
+    const uint64_t need = layout == NAFGPU_EXPORT_FLAT ? c->exp_bytes[f] : layout == NAFGPU_EXPORT_ROWS ? spec->n_rows * spec->row_length : 8 * (c->exp_records + 1);
+    if (spec->out_bytes < need || (!spec->out && need)) {
+        char b[128];
+        snprintf(b, sizeof b, "export needs %llu bytes of output, out_bytes is %llu", (unsigned long long)need, (unsigned long long)spec->out_bytes);
+        return fail(c, NAFGPU_ERR_ARGUMENT, b);
+    }
+    // ordering: the caller's stream waits for the run (and the descriptors' upload); the context's stream, where every later
+    // call on this context enqueues its work, waits for the export
+    cudaStream_t st = stream ? (cudaStream_t)stream : c->st;
+    if (st != c->st) {
+        CUDA_TRY(c, cudaEventRecord(c->ev_exp_ready, c->st));
+        CUDA_TRY(c, cudaStreamWaitEvent(st, c->ev_exp_ready, 0));
+    }
+    nk::ExpTable table;
+    memcpy(table.b, spec->table, 256);
+    bool identity = true;
+    for (int i = 0; i < 256; i++) identity = identity && spec->table[i] == (uint8_t)i;
+    const uint8_t* arena = (const uint8_t*)c->arena.p;
+    const uint8_t* desc = (const uint8_t*)c->exp_desc.p;
+    const nk::ExpRec* recs = (const nk::ExpRec*)desc;
+    if (layout == NAFGPU_EXPORT_FLAT)
+        nk::launch_export_flat(arena, (const nk::ExpSpan*)(desc + c->o_exp_span[f]), c->n_exp_span[f], need, table, identity, (uint8_t*)spec->out, st);
+    else if (layout == NAFGPU_EXPORT_ROWS)
+        nk::launch_export_rows(arena, recs, c->n_exp_rec, c->exp_records, f == 3 ? 1u : 0u, spec->rows, spec->n_rows, spec->row_length, table, identity,
+                               spec->pad, (uint8_t*)spec->out, st);
+    else
+        nk::launch_export_offsets(arena, recs, c->n_exp_rec, c->exp_records, c->exp_residues, (int64_t*)spec->out, st);
+    CUDA_TRY(c, cudaGetLastError());
+    if (st != c->st) {
+        CUDA_TRY(c, cudaEventRecord(c->ev_exp_done, st));
+        CUDA_TRY(c, cudaStreamWaitEvent(c->st, c->ev_exp_done, 0));
+    }
     return NAFGPU_OK;
 }
 

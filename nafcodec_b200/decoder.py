@@ -20,7 +20,7 @@ import numpy as np
 
 from . import _ffi
 from .data import Flag, Flags, FormatVersion, Header, Record, SequenceType
-from .errors import NafIoError, raise_for_status
+from .errors import NafArgumentError, NafIoError, raise_for_status
 
 _SEQTYPE_NAMES = {0: "dna", 1: "rna", 2: "protein", 3: "text"}
 
@@ -124,6 +124,26 @@ class Context:
     def fetch(self):
         res = self.fetch_raw()
         return [ArchiveResult._copy_from(self._arr[i].header, res[i]) for i in range(self._n)]
+
+    def counts(self) -> List["_ffi.Counts"]:
+        """Per-archive counters of the job that was run (nafgpu_job_counts: one small copy and a synchronise per run)."""
+        res = (_ffi.Counts * self._n)()
+        with self._lock:
+            self._check_export(self.lib.dll.nafgpu_job_counts(self._ctx, res, self._n))
+        return list(res)
+
+    def export(self, spec: "_ffi.Export", stream: int = 0):
+        """Enqueues one export of the job that was run into device memory (nafgpu_job_export) on `stream` (a cudaStream_t
+        handle; 0 = the context's own stream).  A refused export raises NafArgumentError."""
+        with self._lock:
+            self._check_export(self.lib.dll.nafgpu_job_export(self._ctx, C.byref(spec), stream or None))
+
+    def _check_export(self, rc):
+        if rc == _ffi.ERR_ARGUMENT:
+            e = NafArgumentError(self.lib.strerror(rc) + ": " + self.lib.dll.nafgpu_last_error(self._ctx).decode())
+            e.status = rc
+            raise e
+        raise_for_status(self.lib, rc, self._ctx)
 
     def stats(self) -> "_ffi.JobStats":
         s = _ffi.JobStats()

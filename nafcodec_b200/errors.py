@@ -20,6 +20,10 @@ class NafUnicodeError(NafError, UnicodeError):
     """Error::Utf8 / Io(InvalidData) from String::from_utf8 (reader.rs:108-109)."""
 
 
+class NafArgumentError(NafError, ValueError):
+    """A device export the library refused (NAFGPU_ERR_ARGUMENT): no run, a field that was not decoded, too small an output."""
+
+
 class NafDeviceError(NafError, RuntimeError):
     """CUDA failure, missing device or missing library: there is no CPU fallback."""
 

@@ -122,6 +122,45 @@ pub struct nafgpu_pack_result {
     pub first_invalid: u64,
 }
 
+/// `nafgpu_counts` (include/nafgpu.h): per-archive counters of the job that was run.
+#[repr(C)]
+#[derive(Clone, Copy, Default)]
+pub struct nafgpu_counts {
+    pub n_records: u64,
+    pub n_ids: u64,
+    pub n_comments: u64,
+    pub n_lengths: u64,
+    pub total_residues: u64,
+    pub id_bytes: u64,
+    pub comment_bytes: u64,
+    pub first_bad_record: u64,
+    pub record_status: i32,
+    pub status: i32,
+}
+
+pub const NAFGPU_SEC_ID: i32 = 0;
+pub const NAFGPU_SEC_COMMENT: i32 = 1;
+pub const NAFGPU_SEC_SEQUENCE: i32 = 4;
+pub const NAFGPU_SEC_QUALITY: i32 = 5;
+pub const NAFGPU_EXPORT_FLAT: i32 = 0;
+pub const NAFGPU_EXPORT_ROWS: i32 = 1;
+pub const NAFGPU_EXPORT_OFFSETS: i32 = 2;
+
+/// `nafgpu_export` (include/nafgpu.h): one export of the decoded job into device memory the caller owns.
+#[repr(C)]
+pub struct nafgpu_export {
+    pub field: i32,
+    pub layout: i32,
+    pub table: [u8; 256],
+    pub pad: u8,
+    pub _pad: [u8; 7],
+    pub out: *mut c_void,         // DEVICE memory
+    pub out_bytes: u64,
+    pub rows: *const i64,         // DEVICE, ROWS: n_rows (record, start) pairs
+    pub n_rows: u64,
+    pub row_length: u64,
+}
+
 extern "C" {
     pub fn nafgpu_ctx_create(device: c_int, out: *mut *mut nafgpu_ctx) -> c_int;
     pub fn nafgpu_ctx_destroy(ctx: *mut nafgpu_ctx);
@@ -172,4 +211,7 @@ extern "C" {
     pub fn nafgpu_pipeline_last_error(p: *const nafgpu_pipeline) -> *const c_char;
     pub fn nafgpu_pipeline_lanes(p: *const nafgpu_pipeline) -> u32;
     pub fn nafgpu_pack(ctx: *mut nafgpu_ctx, input: *const nafgpu_pack_input, out: *mut nafgpu_pack_result) -> c_int;
+    pub fn nafgpu_job_counts(ctx: *mut nafgpu_ctx, out: *mut nafgpu_counts, n: u32) -> c_int;
+    /// enqueued on `stream` (a cudaStream_t; null = the context's stream), ordered after the run and before the context's next call
+    pub fn nafgpu_job_export(ctx: *mut nafgpu_ctx, spec: *const nafgpu_export, stream: *mut c_void) -> c_int;
 }
