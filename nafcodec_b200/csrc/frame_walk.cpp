@@ -30,8 +30,10 @@ static int frame_header(const uint8_t* s, uint64_t n, uint64_t dst_size, uint64_
         uint64_t base = 1ull << (10 + (wd >> 3));
         window = base + (base >> 3) * (wd & 7);
     }
-    // match offsets travel through the kernels in 29 bits beside the symbolic repeat-offset encoding (zstd_format.h,
-    // OFF_SYMBOLIC): a frame that may use longer ones (zstd --long=30/31) is refused, not mis-decoded
+    // match offsets travel through the kernels as 31-bit values: bit 31 marks the symbolic repeat-offset encoding
+    // (zstd_format.h, OFF_SYMBOLIC; a decoded raw offset with bit 31 set flags the block, and the LZ rounds never redirect a
+    // match to a sum of 2^31 or more).  A window descriptor above 512 MiB (zstd --long=30/31) is refused, not mis-decoded;
+    // a single-segment frame's window is its content size, checked below.
     if (window > (1ull << 29)) FAIL(ERR_UNSUPPORTED, "zstd frame: window of %llu bytes exceeds the supported 512 MiB", (unsigned long long)window);
     static const int dict_sz[4] = {0, 1, 2, 4};
     uint32_t dict_id = 0;
@@ -44,6 +46,9 @@ static int frame_header(const uint8_t* s, uint64_t n, uint64_t dst_size, uint64_
     for (int i = 0; i < fcs_sz; i++) fcs |= (uint64_t)s[p++] << (8 * i);
     if (fcs_sz == 2) fcs += 256;
     if (single) window = fcs;
+    // (offsets of a single-segment frame are below its content size; up to 1 GiB they stay clear of bit 31 and of the
+    //  finisher's bound on chunk-relative distances, 0x7F000000)
+    if (single && window > (1ull << 30)) FAIL(ERR_UNSUPPORTED, "zstd frame: single-segment window of %llu bytes exceeds the supported 1 GiB", (unsigned long long)window);
     if (fcs_sz && fcs != dst_size) FAIL(ERR_INVALID, "zstd frame: content size %llu differs from the section size %llu",
                                         (unsigned long long)fcs, (unsigned long long)dst_size);
 

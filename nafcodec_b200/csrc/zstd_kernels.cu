@@ -607,7 +607,7 @@ __device__ __forceinline__ void seq_consume_batch(uint32_t* b_ov, const uint32_t
             if ((uint32_t)lane >= cnt) m = last;                     // (lane 31 carries the batch's total below)
         } else rep_warp_scan(m, lane, t.bad);
         RepSym off; off.src = m.s[0]; off.val = m.v[0];
-        if (off.src >= 0 && off.val > 0x1FFFFFFFu) t.bad = true;
+        if (off.src >= 0 ? off.val > 0x1FFFFFFFu : off.val > 0x7FFFFFFFu) t.bad = true;    // (raw offsets with bit 31 set: OF codes 31+, corrupt)
         if ((uint32_t)lane < cnt) b_ov[lane] = encode_off(off);
         rep_shfl(t.carry, m, 31);                        // (lanes past the batch hold the identity: lane 31 has the batch's total)
     }
@@ -659,6 +659,13 @@ constexpr uint32_t SEQ_BATCH = 32;
 #define SEQ_REPORT(slot, a, b, nseq) ((void)0)
 #endif
 
+// A block whose sequences are not decoded (its frame failed before, or its own stream is corrupt) still owns its records:
+// the LZ stages find the frame of sequence i through J.seq[i].block before they look at the frame's status, and a record
+// left as the previous job wrote it would send them to another frame's block, or past the end of the tables.
+__device__ __forceinline__ void seq_claim_records(const JobDev& J, const BlockDesc& B, uint32_t bi, uint32_t t, uint32_t nt) {
+    for (uint32_t j = t; j < B.n_seq; j += nt) J.seq[B.seq_base + j].block = bi;
+}
+
 __global__ void __launch_bounds__(64) k_decode_sequences(JobDev J) {
     NAF_DYN_SMEM(uint32_t, sbits);                       // staged bitstream: J.seq_stage_bytes (job maximum, capped)
     __shared__ __align__(8) SeqCell stab[3][FSE_SLOT_CELLS];
@@ -667,11 +674,11 @@ __global__ void __launch_bounds__(64) k_decode_sequences(JobDev J) {
     const uint32_t bi = J.tiny_blocks ? J.seq_big_list[blockIdx.x] : blockIdx.x;      // (with tiny_blocks: a list of the blocks that are not
     const BlockDesc& B = J.blocks[bi];                                                  //  k_decode_sequences_tiny's -- 2 x 10^6 CTAs that exit at once cost 2.9 ms)
     if (B.btype != BT_COMPRESSED || B.n_seq == 0) return;
-    if (J.frame_bad[B.frame]) return;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    if (J.frame_bad[B.frame]) { seq_claim_records(J, B, bi, tid, 64); return; }
     BlockState& S = J.bstate[bi];
     const uint8_t* src = J.comp + B.src_off;
-    if (S.seq_bits_off >= B.src_size) { if (tid == 0) flag_error(J, B.frame, zc::E_SEQ_STREAM); return; }
+    if (S.seq_bits_off >= B.src_size) { if (tid == 0) flag_error(J, B.frame, zc::E_SEQ_STREAM); seq_claim_records(J, B, bi, tid, 64); return; }
     const uint32_t nbytes = B.src_size - S.seq_bits_off;
     const uint8_t* g = src + S.seq_bits_off;
     const bool staged = nbytes + 48 <= J.seq_stage_bytes;
@@ -689,7 +696,7 @@ __global__ void __launch_bounds__(64) k_decode_sequences(JobDev J) {
         for (uint32_t c = tid; c < nchunks; c += 64) ((uint4*)sbits)[1 + c] = gbase[c];
     }
     const uint8_t last = g[nbytes - 1];
-    if (last == 0) { if (tid == 0) flag_error(J, B.frame, zc::E_SEQ_STREAM); return; }     // (uniform)
+    if (last == 0) { if (tid == 0) flag_error(J, B.frame, zc::E_SEQ_STREAM); seq_claim_records(J, B, bi, tid, 64); return; }     // (uniform)
     __syncthreads();
     if (staged && (uint32_t)tid < 16 + a) ((uint8_t*)sbits)[tid] = 0;
     if (tid == 0) s_left = 0;
@@ -781,13 +788,13 @@ __global__ void __launch_bounds__(SEQ_TINY_WARPS * 32) k_decode_sequences_tiny(J
     if (bi >= J.n_blocks) return;
     const BlockDesc& B = J.blocks[bi];
     if (!tiny_seq_block(B)) return;
-    if (J.frame_bad[B.frame]) return;
+    if (J.frame_bad[B.frame]) { seq_claim_records(J, B, bi, lane, 32); return; }
     BlockState& S = J.bstate[bi];
-    if (S.seq_bits_off >= B.src_size) { if (lane == 0) flag_error(J, B.frame, zc::E_SEQ_STREAM); return; }
+    if (S.seq_bits_off >= B.src_size) { if (lane == 0) flag_error(J, B.frame, zc::E_SEQ_STREAM); seq_claim_records(J, B, bi, lane, 32); return; }
     const uint32_t nbytes = B.src_size - S.seq_bits_off;
     const uint8_t* g = J.comp + B.src_off + S.seq_bits_off;
     // (more bytes than 32 sequences can consume: the stream cannot end exactly at bit 0)
-    if (nbytes > SEQ_TINY_BYTES || g[nbytes - 1] == 0) { if (lane == 0) flag_error(J, B.frame, zc::E_SEQ_STREAM); return; }
+    if (nbytes > SEQ_TINY_BYTES || g[nbytes - 1] == 0) { if (lane == 0) flag_error(J, B.frame, zc::E_SEQ_STREAM); seq_claim_records(J, B, bi, lane, 32); return; }
     uint32_t* sbits = sb_all[warp];
     const uint32_t a = (uint32_t)((uintptr_t)g & 15);
     const uint32_t nchunks = (a + nbytes + 15) >> 4;                       // <= 25
@@ -815,6 +822,7 @@ __global__ void __launch_bounds__(SEQ_TINY_WARPS * 32) k_decode_sequences_tiny(J
     __syncwarp();
     SeqTotals tot; tot.init();
     if (left == 0) seq_consume_batch(r_all[warp][1], r_all[warp][2], r_all[warp][0], n, lane, (uint4*)(J.seq + B.seq_base), bi, tot);
+    else seq_claim_records(J, B, bi, lane, 32);                             // (the block is flagged below)
     tot.bad = __any_sync(0xFFFFFFFFu, tot.bad);
     if (lane != 0) return;
     seq_finish_block(J, B, S, tot, left);
@@ -2389,7 +2397,9 @@ __device__ __forceinline__ int lz_try(const JobDev& J, uint32_t i, uint32_t roun
         if (blocker == 0xFFFFFFFFu) { verdict = 1; break; }
         const SeqRec& Q = J.seq[blocker];
         if (hop == LZ_HOPS || off < ml || Q.match_pos > s || e > Q.match_pos + Q.ml) { J.lz_blocker[i] = blocker; break; }      // cannot redirect: wait
-        off += resolve_offset(J, Q.off, Q.block);
+        const uint32_t add = resolve_offset(J, Q.off, Q.block);
+        if (add > 0x7FFFFFFFu - off) { J.lz_blocker[i] = blocker; break; }     // (the sum is stored in R.off: bit 31 would read as OFF_SYMBOLIC)
+        off += add;
     }
     if (off != off0) R.off = off;                                      // keep the shortcut for later rounds (and for others)
     return verdict;

@@ -92,7 +92,7 @@ class Context:
         with self._lock:
             rc = self.lib.dll.nafgpu_zstd_decompress(self._ctx, src, len(frame), regen_size, dst)
             raise_for_status(self.lib, rc, self._ctx)
-        return bytes(dst[:regen_size])
+        return C.string_at(dst, regen_size)          # (one copy: a slice of a ctypes array is a list of ints)
 
     # staged API (bench / profiling)
     def prepare(self, archives, want=_ffi.WANT_ALL):

@@ -126,8 +126,8 @@ def test_frame_content_checksum_is_verified(backend):
 
 
 def test_window_beyond_the_offset_encoding_is_refused(backend):
-    # offsets travel in 29 bits beside the symbolic repeat-offset encoding: a frame that declares a 1 GiB window
-    # (zstd --long=30) is refused on the host instead of being mis-decoded
+    # a frame that declares a 1 GiB window (zstd --long=30) is refused on the host instead of being mis-decoded
+    # (tests/test_zstd_sequences.py: offsets up to 2^29, single-segment frames)
     ctx = N.shared_context(0, library(backend))
     p = b"ACGT" * 1000
     frame = bytearray(O.zstd_compress(p, 3))
