@@ -170,34 +170,34 @@ static __global__ void __launch_bounds__(EXPORT_THREADS) k_export_offsets(const 
     }
 }
 
-// enough CTAs to fill the 148 SMs several times over; the kernels loop over whatever is left
-static uint32_t export_ctas(uint64_t items) {
+// enough CTAs to fill the `sms` multiprocessors several times over; the kernels loop over whatever is left
+static uint32_t export_ctas(uint64_t items, uint32_t sms) {
     const uint64_t ctas = (items + EXPORT_THREADS - 1) / EXPORT_THREADS;
-    return (uint32_t)(ctas < 148u * 16u ? (ctas ? ctas : 1) : 148u * 16u);
+    return (uint32_t)(ctas < sms * 16u ? (ctas ? ctas : 1) : sms * 16u);
 }
 
 // out[0, total) <- table[field bytes of spans[0, n_spans)] (16-byte aligned stores; out may have any alignment).
 static void launch_export_flat(const uint8_t* arena, const ExpSpan* spans, uint32_t n_spans, uint64_t total, const ExpTable& table,
-                        bool identity, uint8_t* out, cudaStream_t st) {
+                        bool identity, uint8_t* out, uint32_t sms, cudaStream_t st) {
     if (!total) return;
-    NAF_LAUNCH(k_export_flat, export_ctas(total / 16 + 2), EXPORT_THREADS, 0, st, arena, spans, n_spans, total, table, identity ? 1u : 0u, out);
+    NAF_LAUNCH(k_export_flat, export_ctas(total / 16 + 2, sms), EXPORT_THREADS, 0, st, arena, spans, n_spans, total, table, identity ? 1u : 0u, out);
 }
 
 // out[i * L + c] <- table[field byte `start + c` of record `record`] for (record, start) = rows[2i], rows[2i + 1]; pad past the
 // record's end, and the whole row for a record out of [0, n_records), a start outside [0, length) or a field not decoded.
 static void launch_export_rows(const uint8_t* arena, const ExpRec* recs, uint32_t n_recs, uint64_t n_records, uint32_t field,
                         const int64_t* rows, uint64_t n_rows, uint64_t row_length, const ExpTable& table, bool identity,
-                        uint8_t pad, uint8_t* out, cudaStream_t st) {
+                        uint8_t pad, uint8_t* out, uint32_t sms, cudaStream_t st) {
     const uint64_t total = n_rows * row_length;
     if (!total) return;
-    NAF_LAUNCH(k_export_rows, export_ctas(total / 16 + 2), EXPORT_THREADS, 0, st, arena, recs, n_recs, n_records, field, rows,
+    NAF_LAUNCH(k_export_rows, export_ctas(total / 16 + 2, sms), EXPORT_THREADS, 0, st, arena, recs, n_recs, n_records, field, rows,
                row_length, total, table, identity ? 1u : 0u, (uint32_t)pad, out);
 }
 
 // out[j] <- job-global exclusive offset of record j, j in [0, n_records]; out[n_records] = total_residues.
 static void launch_export_offsets(const uint8_t* arena, const ExpRec* recs, uint32_t n_recs, uint64_t n_records, uint64_t total_residues,
-                           int64_t* out, cudaStream_t st) {
-    NAF_LAUNCH(k_export_offsets, export_ctas(n_records + 1), EXPORT_THREADS, 0, st, arena, recs, n_recs, n_records, total_residues, out);
+                           int64_t* out, uint32_t sms, cudaStream_t st) {
+    NAF_LAUNCH(k_export_offsets, export_ctas(n_records + 1, sms), EXPORT_THREADS, 0, st, arena, recs, n_recs, n_records, total_residues, out);
 }
 
 }  // namespace nk

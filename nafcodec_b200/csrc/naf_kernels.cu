@@ -499,8 +499,8 @@ __global__ void __launch_bounds__(256) k_utf8_validate(uint8_t* arena, const Naf
 
 // --------------------------------------------------------------------------------------------------------------
 int launch_naf_stage(uint8_t* arena, const NafDev* archives, uint32_t n_archives, uint64_t max_records, uint64_t max_scan_bytes, void* scan_agg,
-                     uint32_t max_chunks, uint64_t max_text_bytes, bool any_mask, bool any_text_mask, uint32_t* status, cudaStream_t st,
-                     StageEvents* ev) {
+                     uint32_t max_chunks, uint64_t max_text_bytes, bool any_mask, bool any_text_mask, uint32_t* status, uint32_t sms,
+                     cudaStream_t st, StageEvents* ev) {
     StageEvents none;
     if (!ev) ev = &none;
     int launches = 0;
@@ -523,7 +523,7 @@ int launch_naf_stage(uint8_t* arena, const NafDev* archives, uint32_t n_archives
     ev->mark();
     if (max_text_bytes > 0) {
         uint32_t g = (uint32_t)((max_text_bytes / 16 + 255) / 256);
-        if (g > 148 * 8) g = 148 * 8;
+        if (g > sms * 8) g = sms * 8;
         if (g == 0) g = 1;
         NAF_LAUNCH(k_ascii_check, dim3(g, n_archives, 2), 256, 0, st, arena, archives); launches++;
     }

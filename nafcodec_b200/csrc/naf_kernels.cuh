@@ -47,10 +47,10 @@ struct NafDev {
 // Enqueues the NAF stage for n_archives archives on `stream`.  max_* are maxima over the archives (grid sizing).
 // max_scan_bytes: largest ids / comments / lengths / mask section of the job; scan_agg: n_archives x 4 x slices x NAF_AGG_BYTES of
 // scratch when that is more than one NAF_SLICE.  Returns the number of kernels launched; `ev` (optional) gets one mark per stage (NAF_STAGES).
-// any_mask: some archive decodes sequence + mask; any_text_mask: one of those is protein/text.
+// any_mask: some archive decodes sequence + mask; any_text_mask: one of those is protein/text.  sms: the device's multiprocessors.
 int launch_naf_stage(uint8_t* arena, const NafDev* archives_dev, uint32_t n_archives, uint64_t max_records, uint64_t max_scan_bytes, void* scan_agg,
-                     uint32_t max_chunks, uint64_t max_text_bytes, bool any_mask, bool any_text_mask, uint32_t* status, cudaStream_t stream,
-                     StageEvents* ev);
+                     uint32_t max_chunks, uint64_t max_text_bytes, bool any_mask, bool any_text_mask, uint32_t* status, uint32_t sms,
+                     cudaStream_t stream, StageEvents* ev);
 constexpr int NAF_STAGES = 5;
 
 }  // namespace nk

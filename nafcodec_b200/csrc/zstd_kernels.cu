@@ -21,6 +21,7 @@
 //                   k_lz_finish, k_lz_finish2  endless chains (text-like sections): byte-level pointer jumping inside 64 KB chunks on all SMs,
 //                                            then across chunks over the chunks' roots
 //                   k_frame_checksum         frames that carry a content checksum (XXH64)
+#include "frame_walk.h"          // (first: the emulator's cuda_compat.h defines __noinline__, which <string> uses)
 #include "zstd_kernels.cuh"
 
 #include <algorithm>
@@ -3135,69 +3136,125 @@ void lz_finish_ctas(int device, uint32_t* level1, uint32_t* level2) {
 #endif
 }
 
-int launch_zstd_stage(const JobDev& J, cudaStream_t st, cudaStream_t st2, cudaEvent_t fork, cudaEvent_t join, StageEvents* ev,
-                      cudaStream_t st3, cudaEvent_t fork3, cudaEvent_t join3, cudaEvent_t fork4, cudaEvent_t join4) {
+bool Streams::create() {
+    for (cudaStream_t* s : {&st, &st2, &st3}) if (cudaStreamCreateWithFlags(s, cudaStreamNonBlocking) != cudaSuccess) return false;
+    for (cudaEvent_t* e : {fork, fork + 1, fork + 2, join, join + 1, join + 2}) if (cudaEventCreateWithFlags(e, cudaEventDisableTiming) != cudaSuccess) return false;
+    return true;
+}
+
+void Streams::destroy() {
+    for (cudaEvent_t* e : {fork, fork + 1, fork + 2, join, join + 1, join + 2}) { if (*e) cudaEventDestroy(*e); *e = nullptr; }
+    for (cudaStream_t* s : {&st, &st2, &st3}) { if (*s) cudaStreamDestroy(*s); *s = 0; }
+}
+
+// A cooperative grid for `want` CTAs of work: at least 8, at most the co-resident `max` (a barrier over 27 CTAs returns sooner
+// than one over 592, and a cooperative grid costs microseconds to launch even when it has nothing to do).
+static uint32_t coop_grid(uint64_t want, uint32_t max) {
+    const uint32_t cap = max ? max : 1u;
+    return want < 8 ? std::min(8u, cap) : (uint32_t)std::min<uint64_t>(want, cap);
+}
+
+Launch choose_paths(JobDev& J, const fw::JobPlan& pl, const Overrides& ov, uint32_t sms, uint64_t arena_size) {
+    const uint64_t nseq = J.n_seq;
+    // thousands of tiny blocks (a FASTQ section flushed per record): warp-per-block kernels for them, and the two-warp CTAs of
+    // the others do not carry the shared memory of ... the others
+    J.tiny_blocks = ov.tiny_blocks ? *ov.tiny_blocks : (pl.n_tiny_seq_blocks >= 4096u ? 1u : 0u);
+    J.seq_stage_bytes = std::min<uint32_t>((((J.tiny_blocks ? pl.max_seq_section_big : pl.max_seq_section) + 15u) & ~15u) + 64u, 16u * 1024u);
+    // one CTA for the matches of a small job (k_lz_small holds up to 8192; beyond ~2000 the general rounds are faster)
+    const uint64_t small_max = ov.lz_small ? *ov.lz_small : 2048;
+    J.lz_small = (nseq <= small_max && J.n_frames <= 65535 && arena_size < (1ull << 32)) ? 1u : 0u;
+    J.lz_flow_on = ov.lz_flow ? *ov.lz_flow : (nseq > 8192 ? 1u : 0u);
+    J.flow_ctas = (uint32_t)std::min<uint64_t>((nseq + 255) / 256, sms * 8u);
+    J.lz_flow_early = ov.lz_flow_early ? *ov.lz_flow_early : ((nseq > 2048 && nseq <= 65536 && !ov.lz_small) ? 1u : 0u);
+    // the finisher's first level handles a 64 KB chunk in ~90 us on one SM, all SMs at once; its second level (barrier rounds over
+    // the unresolved bytes) costs about twice that again when the chains cross many chunks (cfg3: 13 M bytes)
+    const uint64_t waves = ((uint64_t)J.fin_total_chunks + J.fin_ctas - 1) / std::max<uint32_t>(J.fin_ctas, 1u);
+    J.fin_cost_us = ov.fin_cost_us ? *ov.fin_cost_us : (uint32_t)std::min<uint64_t>(300 + waves * 270, 0x7FFFFFFFu);   // (both levels: 3.6 ms for the 1907 chunks of a 250 Mbp frame)
+    J.huf_block_min = ov.huf_block_min ? *ov.huf_block_min : 0;
+
+    Launch L;
+    // a job with both kinds of Huffman streams (one archive: the big blocks of the sequence, the short ids / lengths / last
+    // block): the two decodes side by side -- for a single small archive this branch is the critical path (25 us each)
+    L.huf_side = J.n_huf_big && J.n_huf_items > J.n_huf_big;
+    // Two shapes of the same decode of the big streams.  Enough blocks to fill the device several times over (a batch, a
+    // chromosome): one CTA per BLOCK, its four streams in turn, tables built once (k_huf_decode_block: 1.31 ms against 1.63 ms
+    // on the 256-archive job).  A handful of blocks (one small archive): one CTA per STREAM, the four of a block as a
+    // thread-block cluster that shares the table construction through DSMEM -- four times the CTAs in flight, which is what
+    // latency wants (k_huf_decode_big).
+    L.huf_per_block = J.n_huf_big / 4 >= (J.huf_block_min ? J.huf_block_min : 296u);
+    L.huf_small_smem = huf_fixed_smem(HUF_T_SMALL) + ((J.max_huf_small + 15 + 16 + 16 + 15) & ~15u);
+    L.huf_big_smem = hb_smem_bytes(J.max_huf_stream);
+    // a job with both kinds of blocks (a FASTQ archive: 2 x 10^6 tiny blocks and the ~130 big blocks of the ids, each one chain of
+    // ~10^4 sequences, 2.9 ms): the general kernel beside the tiny blocks' (2.0 ms)
+    L.seq_side = J.tiny_blocks && J.n_seq_big;
+    // (jobs of 10^5+ tiny blocks -- FASTQ flushed per record -- have a handful of runs per block: no split, fewer CTAs)
+    L.lit_blocks = J.tiny_blocks ? J.n_lit_big : J.n_blocks;
+    L.lit_few = L.lit_blocks <= 64u;
+    L.lit_split = L.lit_few ? 4 * LZLIT_SPLIT : (L.lit_blocks > 16384u ? 1 : LZLIT_SPLIT);
+    L.lz_small_smem = lzs_smem_bytes((uint32_t)nseq);
+    // (small jobs: one entry per thread, as many CTAs as entries need -- latency; big jobs: LZ_U entries per thread)
+    L.first_ctas = (uint32_t)((nseq + LZ_CTA - 1) / LZ_CTA);
+    if (L.first_ctas > sms * 8u) L.first_ctas = std::max<uint32_t>(sms * 8u, (uint32_t)((nseq + LZ_CTA * LZ_U - 1) / (LZ_CTA * LZ_U)));
+    if (L.first_ctas > sms * 64u) L.first_ctas = sms * 64u;
+    // a small job takes no more CTAs than its matches can use: a single archive pays one barrier per dependency round
+    L.resolve_ctas = coop_grid((nseq + LZ_CTA * 2 - 1) / (LZ_CTA * 2), J.coop_ctas);
+    L.finish_ctas = J.fin_total_chunks < J.fin_ctas ? J.fin_total_chunks : J.fin_ctas;
+    L.finish = L.finish_ctas && nseq > LZ_MIN_PENDING;       // (k_lz_resolve never hands over fewer than LZ_MIN_PENDING matches)
+    L.finish2_ctas = coop_grid(J.fin_total_chunks * 2u, J.fin2_ctas);
+    return L;
+}
+
+int launch_zstd_stage(const JobDev& J, const Launch& L, const Streams& S, StageEvents* ev) {
     StageEvents none;
     if (!ev) ev = &none;
-    int launches = 0;
-    if (J.n_blocks == 0) { for (int i = 0; i < ZSTD_STAGES; i++) ev->mark(); return 0; }
+    int launches = 0, stage = 0;
+    // the one place that marks stage ends: a stage a job skips gets an empty interval, so that there are always ZSTD_STAGES
+    const auto end_stage = [&](int s) { for (; stage < s; stage++) ev->mark(); };
+    if (J.n_blocks == 0) { end_stage(ZSTD_STAGES); return 0; }
     // Two independent branches: (A) FSE tables -> sequences -> frame scan on `st`; (B) Huffman weights -> Huffman decode into
-    // the literal staging buffer on `st2` (when given).  They join before k_lz_literals.
-    cudaStream_t sb = st2 ? st2 : st;
-    (void)sb;                                          // (the emulator's launch macro ignores the stream)
-    if (st2) { cudaEventRecord(fork, st); cudaStreamWaitEvent(st2, fork, 0); }
+    // the literal staging buffer on `st2` (not in a profiled run).  They join before k_lz_literals.
+    const cudaStream_t st = S.st, st2 = ev != &none ? (cudaStream_t)0 : S.st2, st3 = S.st3;
+    const cudaStream_t sb = st2 ? st2 : st;
+    (void)sb; (void)st3;                               // (the emulator's launch macro ignores the stream)
+    if (st2) { cudaEventRecord(S.fork[0], st); cudaStreamWaitEvent(st2, S.fork[0], 0); }
     if (J.n_huf_items) {
         NAF_LAUNCH(k_build_tables<1>, J.n_blocks, 32, 0, sb, J); launches++;
-        // a job with both kinds of streams (one archive: the big blocks of the sequence, the short ids / lengths / last block):
-        // the two decodes side by side -- for a single small archive this branch is the critical path (25 us each)
-        const bool side = st2 && st3 && J.n_huf_big && J.n_huf_items > J.n_huf_big;
-        (void)side;
+        const bool side = st2 && st3 && L.huf_side;
         if (side) {
-            cudaEventRecord(fork3, sb); cudaStreamWaitEvent(st3, fork3, 0);
-            const uint32_t smem = huf_fixed_smem(HUF_T_SMALL) + ((J.max_huf_small + 15 + 16 + 16 + 15) & ~15u);
-            NAF_LAUNCH((k_huf_decode<HUF_T_SMALL>), J.n_huf_items - J.n_huf_big, HUF_T_SMALL, smem, st3, J, J.huf_items + J.n_huf_big); launches++;
-            cudaEventRecord(join3, st3);
+            cudaEventRecord(S.fork[1], sb); cudaStreamWaitEvent(st3, S.fork[1], 0);
+            NAF_LAUNCH((k_huf_decode<HUF_T_SMALL>), J.n_huf_items - J.n_huf_big, HUF_T_SMALL, L.huf_small_smem, st3, J, J.huf_items + J.n_huf_big); launches++;
+            cudaEventRecord(S.join[1], st3);
         }
         if (J.n_huf_big) {   // items [0, n_huf_big): the streams of 4-stream blocks, four consecutive items (= one cluster) per block
-            const uint32_t smem = hb_smem_bytes(J.max_huf_stream);
             if (!st2) ev->kernel_begin();
-            // Two shapes of the same decode.  Enough blocks to fill the device several times over (a batch, a chromosome): one CTA
-            // per BLOCK, its four streams in turn, tables built once (k_huf_decode_block: 1.31 ms against 1.63 ms on the
-            // 256-archive job).  A handful of blocks (one small archive): one CTA per STREAM, the four of a block as a
-            // thread-block cluster that shares the table construction through DSMEM -- four times the CTAs in flight, which
-            // is what latency wants (k_huf_decode_big).
-            const bool per_block = J.n_huf_big / 4 >= (J.huf_block_min ? J.huf_block_min : 296u);
-            if (per_block) {
-                NAF_SET_MAX_SMEM(k_huf_decode_block, smem);
-                NAF_LAUNCH(k_huf_decode_block, J.n_huf_big / 4, HB_T, smem, sb, J); launches++;
+            if (L.huf_per_block) {
+                NAF_SET_MAX_SMEM(k_huf_decode_block, L.huf_big_smem);
+                NAF_LAUNCH(k_huf_decode_block, J.n_huf_big / 4, HB_T, L.huf_big_smem, sb, J); launches++;
             } else {
-                NAF_SET_MAX_SMEM(k_huf_decode_big, smem);
-                NAF_LAUNCH(k_huf_decode_big, J.n_huf_big, HB_T, smem, sb, J); launches++;
+                NAF_SET_MAX_SMEM(k_huf_decode_big, L.huf_big_smem);
+                NAF_LAUNCH(k_huf_decode_big, J.n_huf_big, HB_T, L.huf_big_smem, sb, J); launches++;
             }
             if (!st2) ev->kernel_end();
         }
-        if (side) cudaStreamWaitEvent(sb, join3, 0);
+        if (side) cudaStreamWaitEvent(sb, S.join[1], 0);
         else if (J.n_huf_items > J.n_huf_big) {
-            const uint32_t smem = huf_fixed_smem(HUF_T_SMALL) + ((J.max_huf_small + 15 + 16 + 16 + 15) & ~15u);
-            NAF_LAUNCH((k_huf_decode<HUF_T_SMALL>), J.n_huf_items - J.n_huf_big, HUF_T_SMALL, smem, sb, J, J.huf_items + J.n_huf_big); launches++;
+            NAF_LAUNCH((k_huf_decode<HUF_T_SMALL>), J.n_huf_items - J.n_huf_big, HUF_T_SMALL, L.huf_small_smem, sb, J, J.huf_items + J.n_huf_big); launches++;
         }
     }
-    if (st2) cudaEventRecord(join, st2);
-    else ev->mark();                                  // serial (profiled) order: the Huffman branch first
-    NAF_LAUNCH(k_build_tables<0>, J.n_blocks + 1, 96, 0, st, J); launches++; ev->mark();
-    // a job with both kinds of blocks (a FASTQ archive: 2 x 10^6 tiny blocks and the ~130 big blocks of the ids, each one chain of
-    // ~10^4 sequences, 2.9 ms): the general kernel on the third stream, beside the tiny blocks' (2.0 ms)
-    const bool seq_side = st2 && st3 && J.tiny_blocks && J.n_seq_big;
-    (void)seq_side;
+    if (st2) cudaEventRecord(S.join[0], st2);
+    end_stage(1);                                      // (serial: the Huffman branch first)
+    NAF_LAUNCH(k_build_tables<0>, J.n_blocks + 1, 96, 0, st, J); launches++;
+    end_stage(2);
+    const bool seq_side = st2 && st3 && L.seq_side;
     if (seq_side) {
-        cudaEventRecord(fork4, st); cudaStreamWaitEvent(st3, fork4, 0);
+        cudaEventRecord(S.fork[2], st); cudaStreamWaitEvent(st3, S.fork[2], 0);
         NAF_LAUNCH(k_decode_sequences, J.n_seq_big, 64, J.seq_stage_bytes, st3, J); launches++;
-        cudaEventRecord(join4, st3);
+        cudaEventRecord(S.join[2], st3);
     }
     if (J.tiny_blocks) { NAF_LAUNCH(k_decode_sequences_tiny, (J.n_blocks + SEQ_TINY_WARPS - 1) / SEQ_TINY_WARPS, SEQ_TINY_WARPS * 32, 0, st, J); launches++; }
-    if (seq_side) cudaStreamWaitEvent(st, join4, 0);
+    if (seq_side) cudaStreamWaitEvent(st, S.join[2], 0);
     else if (!J.tiny_blocks || J.n_seq_big) { NAF_LAUNCH(k_decode_sequences, J.tiny_blocks ? J.n_seq_big : J.n_blocks, 64, J.seq_stage_bytes, st, J); launches++; }
-    ev->mark();
+    end_stage(3);
     NAF_LAUNCH(k_frame_scan, J.n_frames, FSCAN_T, 0, st, J); launches++;
     if (J.n_fs_tiles) {
         NAF_LAUNCH(k_fs_reduce, J.n_fs_tiles, FSCAN_T, 0, st, J);
@@ -3205,55 +3262,35 @@ int launch_zstd_stage(const JobDev& J, cudaStream_t st, cudaStream_t st2, cudaEv
         NAF_LAUNCH(k_fs_apply, J.n_fs_tiles, FSCAN_T, 0, st, J);
         launches += 3;
     }
-    ev->mark();
-    if (st2) { cudaStreamWaitEvent(st, join, 0); ev->mark(); }
-    // (jobs of 10^5+ tiny blocks -- FASTQ flushed per record -- have a handful of runs per block: no split, fewer CTAs)
+    end_stage(4);
+    if (st2) cudaStreamWaitEvent(st, S.join[0], 0);
     if (J.tiny_blocks) { NAF_LAUNCH(k_lz_literals_tiny, (J.n_blocks + 7) / 8, 256, 0, st, J); launches++; }
-    const uint32_t lit_blocks = J.tiny_blocks ? J.n_lit_big : J.n_blocks;
-    if (lit_blocks == 0) {}
-    else if (lit_blocks <= 64u) { NAF_LAUNCH(k_lz_literals<4>, dim3(lit_blocks, 4 * LZLIT_SPLIT), 256, 0, st, J); launches++; }
-    else { NAF_LAUNCH(k_lz_literals<1>, dim3(lit_blocks, lit_blocks > 16384u ? 1 : LZLIT_SPLIT), 256, 0, st, J); launches++; }
-    ev->mark();
+    if (L.lit_blocks && L.lit_few) { NAF_LAUNCH(k_lz_literals<4>, dim3(L.lit_blocks, L.lit_split), 256, 0, st, J); launches++; }
+    else if (L.lit_blocks) { NAF_LAUNCH(k_lz_literals<1>, dim3(L.lit_blocks, L.lit_split), 256, 0, st, J); launches++; }
+    end_stage(5);
     if (J.n_seq > 0) {
-        // (small jobs: one entry per thread, as many CTAs as entries need -- latency; big jobs: LZ_U entries per thread)
         if (J.lz_small) {
-            const uint32_t smem = lzs_smem_bytes((uint32_t)J.n_seq);
-            NAF_SET_MAX_SMEM(k_lz_small, smem);
-            NAF_LAUNCH(k_lz_small, 1, LZS_T, smem, st, J); launches++;
-            ev->mark(); ev->mark();
+            NAF_SET_MAX_SMEM(k_lz_small, L.lz_small_smem);
+            NAF_LAUNCH(k_lz_small, 1, LZS_T, L.lz_small_smem, st, J); launches++;
+            end_stage(7);
         } else {
-        uint32_t grid = (uint32_t)((J.n_seq + LZ_CTA - 1) / LZ_CTA);
-        if (grid > 148u * 8u) grid = std::max<uint32_t>(148u * 8u, (uint32_t)((J.n_seq + LZ_CTA * LZ_U - 1) / (LZ_CTA * LZ_U)));
-        if (grid > 148u * 64u) grid = 148u * 64u;
-        NAF_LAUNCH(k_lz_index, (uint32_t)((J.n_seq + 255) / 256), 256, 0, st, J); launches++;
-        if (J.lz_flow_early) { NAF_LAUNCH(k_lz_flow, J.flow_ctas ? J.flow_ctas : 1u, LZF_T, 0, st, J, 1); launches++; }
-        NAF_LAUNCH(k_lz_first, grid, LZ_CTA, 0, st, J); launches++;
-        ev->mark();
-        // co-resident CTAs for the grid barrier (queried by the API); a small job takes no more than its matches can use: a
-        // barrier over 27 CTAs returns sooner than one over 592, and a single archive pays one per dependency round
-        uint32_t cg = J.coop_ctas ? J.coop_ctas : 1u;
-        { const uint64_t want = (J.n_seq + LZ_CTA * 2 - 1) / (LZ_CTA * 2); if (want < cg) cg = want < 8 ? 8u : (uint32_t)want; if (cg > (J.coop_ctas ? J.coop_ctas : 1u)) cg = J.coop_ctas ? J.coop_ctas : 1u; }
-        (void)cg;
-        JobDev Jc = J;
-        NAF_LAUNCH_COOP(k_lz_resolve, cg, LZ_CTA, st, Jc); launches++;
-        if (J.lz_flow_on) { NAF_LAUNCH(k_lz_flow, J.flow_ctas ? J.flow_ctas : 1u, LZF_T, 0, st, J, 0); launches++; }
-        ev->mark();
+            NAF_LAUNCH(k_lz_index, (uint32_t)((J.n_seq + 255) / 256), 256, 0, st, J); launches++;
+            if (J.lz_flow_early) { NAF_LAUNCH(k_lz_flow, J.flow_ctas, LZF_T, 0, st, J, 1); launches++; }
+            NAF_LAUNCH(k_lz_first, L.first_ctas, LZ_CTA, 0, st, J); launches++;
+            end_stage(6);
+            JobDev Jc = J;
+            NAF_LAUNCH_COOP(k_lz_resolve, L.resolve_ctas, LZ_CTA, st, Jc); launches++;
+            if (J.lz_flow_on) { NAF_LAUNCH(k_lz_flow, J.flow_ctas, LZF_T, 0, st, J, 0); launches++; }
+            end_stage(7);
         }
         JobDev Jc = J;
-        const uint32_t fin_grid = J.fin_total_chunks < J.fin_ctas ? J.fin_total_chunks : J.fin_ctas;
-        if (fin_grid && J.n_seq > LZ_MIN_PENDING) {       // (k_lz_resolve never hands over fewer than LZ_MIN_PENDING matches)
+        if (L.finish) {
             NAF_SET_MAX_SMEM(k_lz_finish, FIN_SMEM);
-            NAF_LAUNCH(k_lz_finish, fin_grid, FIN_T, FIN_SMEM, st, J); launches++;
-            // (a small job: no more CTAs than its chunks can use -- a cooperative grid of 592 CTAs costs microseconds to launch
-            //  even when it has nothing to do, which is the normal case)
-            uint32_t cg2 = J.fin2_ctas ? J.fin2_ctas : 1u;
-            if (J.fin_total_chunks * 2u < cg2) cg2 = J.fin_total_chunks * 2u < 8u ? 8u : J.fin_total_chunks * 2u;
-            if (cg2 > (J.fin2_ctas ? J.fin2_ctas : 1u)) cg2 = J.fin2_ctas ? J.fin2_ctas : 1u;
-            (void)cg2;
-            NAF_LAUNCH_COOP(k_lz_finish2, cg2, FIN2_T, st, Jc); launches++;
+            NAF_LAUNCH(k_lz_finish, L.finish_ctas, FIN_T, FIN_SMEM, st, J); launches++;
+            NAF_LAUNCH_COOP(k_lz_finish2, L.finish2_ctas, FIN2_T, st, Jc); launches++;
         }
-        ev->mark();
-    } else { ev->mark(); ev->mark(); ev->mark(); }
+    }
+    end_stage(ZSTD_STAGES);
     if (J.n_checksums) { NAF_LAUNCH(k_frame_checksum, J.n_frames, 32, 0, st, J); launches++; }      // (profiled runs count it with the next stage)
     return launches;
 }
