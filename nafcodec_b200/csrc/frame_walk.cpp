@@ -188,7 +188,10 @@ int walk_frame_part(const uint8_t* frame, uint64_t src_off, uint64_t src_size, u
                     if (pay_size < 6) FAIL(ERR_INVALID, "zstd literals: missing jump table");
                     uint32_t z1 = c[pay] | (c[pay + 1] << 8), z2 = c[pay + 2] | (c[pay + 3] << 8), z3 = c[pay + 4] | (c[pay + 5] << 8);
                     uint32_t seg = (regen + 3) / 4;
-                    if (6ull + z1 + z2 + z3 >= pay_size || 3 * seg >= regen) FAIL(ERR_INVALID, "zstd literals: bad jump table");
+                    if (6ull + z1 + z2 + z3 >= pay_size) FAIL(ERR_INVALID, "zstd literals: bad jump table");
+                    // libzstd's MIN_LITERALS_FOR_4_STREAMS.  From 6 on, 3 * seg <= regen: the fourth stream regenerates
+                    // regen - 3 * seg >= 0 symbols (0 at 6 and 9: a stream of one byte, the end marker alone)
+                    if (regen < 6) FAIL(ERR_INVALID, "zstd literals: fewer than 6 literals in 4-stream mode");
                     so[0] = pay + 6; so[1] = so[0] + z1; so[2] = so[1] + z2; so[3] = so[2] + z3;
                     ss[0] = z1; ss[1] = z2; ss[2] = z3; ss[3] = pay_size - 6 - z1 - z2 - z3;
                     for (int k = 0; k < 4; k++) { dof[k] = seg * k; dn[k] = k < 3 ? seg : regen - 3 * seg; }

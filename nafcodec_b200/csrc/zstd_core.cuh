@@ -291,16 +291,18 @@ ZHD int huf_read_weights(const uint8_t* src, uint32_t src_len, uint8_t* weights,
             if (bb.P < 0) { weights[n++] = cells[s1].sym; break; }
         }
     }
-    uint32_t tot = 0;
+    uint32_t tot = 0, ones = 0;
     for (int i = 0; i < n; i++) {
         if (weights[i] > HUF_MAX_BITS) return 0;
         if (weights[i]) tot += 1u << (weights[i] - 1);
+        ones += weights[i] == 1;
     }
     if (tot == 0) return 0;
     int max_bits = highbit32(tot) + 1;
     if (max_bits > HUF_MAX_BITS) return 0;
     uint32_t left = (1u << max_bits) - tot;
     if (left & (left - 1)) return 0;           // must be a power of two
+    if (ones + (left == 1u) < 2) return 0;     // at least two codes of max_bits (libzstd's HUF_readStats)
     weights[n++] = (uint8_t)(highbit32(left) + 1);
     *max_bits_out = max_bits;
     return n;

@@ -290,16 +290,20 @@ __global__ void __launch_bounds__(PART == 0 ? 96 : 32) k_build_tables(JobDev J) 
             good = n > 0;
         }
         __syncwarp();
-        // validation: weights <= 11, the sum of 2^(w-1) is short of a power of two by a power of two (the implied last weight)
-        uint32_t tot = 0, bad = 0;
-        for (int i = l1; i < n; i += 32) { const uint32_t x = w[i]; if (x > (uint32_t)zc::HUF_MAX_BITS) bad = 1; else if (x) tot += 1u << (x - 1); }
+        // validation: weights <= 11, the sum of 2^(w-1) is short of a power of two by a power of two (the implied last weight),
+        // and at least two symbols of weight 1, the implied one included (libzstd's HUF_readStats: the longest codes come in
+        // pairs; a tree without them, e.g. weights 2, 2, has no code of Max_Number_of_Bits)
+        uint32_t tot = 0, bad = 0, ones = 0;
+        for (int i = l1; i < n; i += 32) { const uint32_t x = w[i]; if (x > (uint32_t)zc::HUF_MAX_BITS) bad = 1; else if (x) tot += 1u << (x - 1); ones += x == 1; }
 #pragma unroll
-        for (int d = 16; d > 0; d >>= 1) { tot += __shfl_xor_sync(0xFFFFFFFFu, tot, d); bad |= __shfl_xor_sync(0xFFFFFFFFu, bad, d); }
+        for (int d = 16; d > 0; d >>= 1) {
+            tot += __shfl_xor_sync(0xFFFFFFFFu, tot, d); bad |= __shfl_xor_sync(0xFFFFFFFFu, bad, d); ones += __shfl_xor_sync(0xFFFFFFFFu, ones, d);
+        }
         int ns = 0, mb = 0;
         if (good && !bad && tot != 0) {
             mb = zc::highbit32(tot) + 1;
             const uint32_t left = (1u << mb) - tot;
-            if (mb <= zc::HUF_MAX_BITS && (left & (left - 1)) == 0) {
+            if (mb <= zc::HUF_MAX_BITS && (left & (left - 1)) == 0 && ones + (left == 1u) >= 2) {
                 if (l1 == 0) w[n] = (uint8_t)(zc::highbit32(left) + 1);
                 ns = n + 1;
             }

@@ -242,29 +242,6 @@ class _Back:
         return (self.v << -self.p) & ((1 << n) - 1)
 
 
-def _huffman_depth(c):
-    """Largest code length of a Huffman tree description (RFC 8878 4.2.1) at c[0]."""
-    hb = c[0]
-    if hb >= 128:
-        n = hb - 127
-        w = [(c[1 + i // 2] >> (0 if i % 2 else 4)) & 15 for i in range(n)]
-    else:
-        al, norm, used = _read_ncount(c, 1, 15)
-        t = _fse_table(al, norm)
-        rd = _Back(bytes(c[1 + used:1 + hb]))
-        s1, s2 = rd.read(al), rd.read(al)
-        w = []
-        while True:
-            sym, nb, base = t[s1]; w.append(sym); s1 = base + rd.read(nb)
-            if rd.p < 0:
-                w.append(t[s2][0]); break
-            sym, nb, base = t[s2]; w.append(sym); s2 = base + rd.read(nb)
-            if rd.p < 0:
-                w.append(t[s1][0]); break
-    total = sum(1 << (x - 1) for x in w if x)
-    return total.bit_length()           # the implied last weight rounds total up to 2^depth
-
-
 class Block:
     """One block of a frame as `frame_codes` reads it: type, size; for compressed blocks the literals section (type, streams,
     sizes, Huffman depth when a tree is described) and the sequences (codes, values, resolved offsets)."""
@@ -333,7 +310,9 @@ def _read_block(c, b, reps, prev):
         regen, csize = v & ((1 << bits) - 1), v >> bits
         b.lit_streams = 1 if sf == 0 else 4
         if lt == 2:
-            b.huf_depth = _huffman_depth(c[hsz:hsz + csize])
+            from _zhuf import read_tree                  # (tests/_zhuf.py reads Huffman sections; it builds on this module)
+            w, _ = read_tree(c[hsz:hsz + csize])
+            b.huf_depth = sum(1 << (x - 1) for x in w if x).bit_length() - 1
     b.lit_regen = regen
     q = hsz + csize
     n = c[q]
