@@ -234,6 +234,7 @@ const char* nafgpu_pipeline_last_error(const nafgpu_pipeline* p);
 uint32_t nafgpu_pipeline_lanes(const nafgpu_pipeline* p);
 int nafgpu_pipeline_lane_stats(nafgpu_pipeline* p, uint32_t lane, nafgpu_job_stats* out);   /* sizes of the lane's last batch */
 
+
 /* ---- encode side (SURVEY 8f rank 4) -----------------------------------------------------------------------------------
  * What the reference's writers compute per record before the bytes reach the zstd compressors, for all records of an
  * archive at once:
@@ -311,6 +312,26 @@ typedef struct nafgpu_export {
  * NAFGPU_ERR_ARGUMENT: no run, a field that was not requested (want bits), ROWS of ids / comments, out_bytes too small,
  * rows NULL with n_rows > 0.  An empty job, or an archive without records, exports zero bytes (OFFSETS: the one entry 0). */
 int nafgpu_job_export(nafgpu_ctx* ctx, const nafgpu_export* spec, void* stream);
+
+/* ---- pipeline device tickets ------------------------------------------------------------------------------------------
+ * The pipeline's lanes, but the decoded sub-batch stays in the lane's device arena, for consumers on the GPU (the
+ * nafgpu_job_export surface above, per ticket).  Host and device tickets may be interleaved on one pipeline; at most `lanes`
+ * tickets of either kind are decoded-but-unreleased at a time.
+ *   submit_device  as nafgpu_pipeline_submit; the lane runs prepare + run + nafgpu_job_counts and copies no result back
+ *   wait_counts    blocks until the ticket is decoded; `out` gets n per-archive counters, as nafgpu_job_counts.  `archives` and
+ *                  the bytes they point to are borrowed until it returns (the counters' read synchronises the lane's stream,
+ *                  so the sub-batch's H2D has completed).  A corrupt archive only sets its own out[i].status (it contributes
+ *                  no records); a CUDA, memory or argument failure of the sub-batch is the return value
+ *   export         nafgpu_job_export on the ticket's lane: same spec, same stream semantics, same errors.  Exports of one
+ *                  ticket may come from several threads (they take turns on a per-lane mutex)
+ *   release        (nafgpu_pipeline_release, for both kinds) hands the lane back.  The lane's next prepare is enqueued on its
+ *                  context's stream, which waits for every export already enqueued from the ticket, so releasing right after
+ *                  an export on another stream is safe
+ * NAFGPU_ERR_ARGUMENT with a message in nafgpu_pipeline_last_error: nafgpu_pipeline_wait on a device ticket, wait_counts on a
+ * host ticket, an export from a ticket that was not waited for, whose decode failed, or that was released. */
+int64_t nafgpu_pipeline_submit_device(nafgpu_pipeline* p, const nafgpu_archive* archives, uint32_t n, uint32_t want);
+int nafgpu_pipeline_wait_counts(nafgpu_pipeline* p, int64_t ticket, nafgpu_counts* out, uint32_t n);
+int nafgpu_pipeline_export(nafgpu_pipeline* p, int64_t ticket, const nafgpu_export* spec, void* stream);
 
 #ifdef __cplusplus
 }

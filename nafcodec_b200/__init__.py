@@ -7,7 +7,7 @@ The compute runs in hand-written sm_100a kernels behind the C ABI of include/naf
 from .data import Flag, Flags, FormatVersion, Header, Record, SequenceType
 from .decoder import (ArchiveResult, Context, Decoder, DecoderBuilder, Pipeline, decode_batch, parse_archive, shared_context,
                       to_fasta, to_fastq, to_text)
-from .device import TABLES, DeviceRecords, decode_to_device
+from .device import TABLES, DeviceRecords, DeviceStream, decode_to_device, stream_to_device
 from .encoder import Encoder, pack_sequences
 from .errors import NafArgumentError, NafDeviceError, NafError, NafIoError, NafParseError, NafUnicodeError
 
@@ -25,4 +25,4 @@ def open(file, mode="r", **options):
 
 __all__ = ["Decoder", "DecoderBuilder", "Record", "Header", "Flag", "Flags", "SequenceType", "FormatVersion", "Encoder", "open",
            "pack_sequences", "Context", "Pipeline", "ArchiveResult", "decode_batch", "to_text", "to_fasta", "to_fastq", "parse_archive", "shared_context",
-           "decode_to_device", "DeviceRecords", "TABLES", "NafError", "NafArgumentError", "NafIoError", "NafParseError", "NafUnicodeError", "NafDeviceError"]
+           "decode_to_device", "DeviceRecords", "stream_to_device", "DeviceStream", "TABLES", "NafError", "NafArgumentError", "NafIoError", "NafParseError", "NafUnicodeError", "NafDeviceError"]

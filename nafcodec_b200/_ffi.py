@@ -89,7 +89,7 @@ SYMBOLS = ["nafgpu_parse_archive", "nafgpu_variable_u64", "nafgpu_strerror", "na
            "nafgpu_job_get_stats", "nafgpu_job_time", "nafgpu_job_run_profiled", "nafgpu_stage_name",
            "nafgpu_job_device_result", "nafgpu_zstd_decompress", "nafgpu_job_format", "nafgpu_format_batch", "nafgpu_pack", "nafgpu_pipeline_create", "nafgpu_pipeline_destroy", "nafgpu_pipeline_submit",
            "nafgpu_pipeline_wait", "nafgpu_pipeline_release", "nafgpu_pipeline_last_error", "nafgpu_pipeline_lanes", "nafgpu_pipeline_lane_stats",
-           "nafgpu_job_counts", "nafgpu_job_export"]
+           "nafgpu_job_counts", "nafgpu_job_export", "nafgpu_pipeline_submit_device", "nafgpu_pipeline_wait_counts", "nafgpu_pipeline_export"]
 
 
 class Library:
@@ -146,6 +146,10 @@ class Library:
         L.nafgpu_job_device_result.argtypes = [C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64)]
         L.nafgpu_job_counts.argtypes = [C.c_void_p, C.POINTER(Counts), C.c_uint32]
         L.nafgpu_job_export.argtypes = [C.c_void_p, C.POINTER(Export), C.c_void_p]
+        L.nafgpu_pipeline_submit_device.argtypes = [C.c_void_p, C.POINTER(Archive), C.c_uint32, C.c_uint32]
+        L.nafgpu_pipeline_submit_device.restype = C.c_int64
+        L.nafgpu_pipeline_wait_counts.argtypes = [C.c_void_p, C.c_int64, C.POINTER(Counts), C.c_uint32]
+        L.nafgpu_pipeline_export.argtypes = [C.c_void_p, C.c_int64, C.POINTER(Export), C.c_void_p]
 
     def strerror(self, code):
         return self.dll.nafgpu_strerror(code).decode()

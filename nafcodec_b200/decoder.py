@@ -558,10 +558,10 @@ class Pipeline:
             msg = self.lib.dll.nafgpu_pipeline_last_error(self._p).decode()
             raise_for_status(self.lib, rc, None, msg)
 
-    def _submit(self, part, want):
+    def _submit(self, part, want, submit=None):
         cnt = len(part)
         arr = (_ffi.Archive * cnt)(*part)
-        t = self.lib.dll.nafgpu_pipeline_submit(self._p, arr, cnt, want)
+        t = (submit or self.lib.dll.nafgpu_pipeline_submit)(self._p, arr, cnt, want)
         if t < 0:
             self._raise(int(t))
         return t, arr, cnt
@@ -641,6 +641,31 @@ class Pipeline:
         if err is not None:
             raise err
         return done
+
+    # -- device tickets (nafgpu_pipeline_submit_device / _wait_counts / _export): the sub-batch stays in the lane's arena -------
+    def submit_device(self, archives, want: int = _ffi.WANT_ALL):
+        """Submits a device ticket; returns (ticket, archive array).  The array and the archives' bytes are borrowed until
+        wait_counts returns."""
+        return self._submit(archives, want, self.lib.dll.nafgpu_pipeline_submit_device)[:2]
+
+    def wait_counts(self, ticket: int, n: int) -> List["_ffi.Counts"]:
+        """Blocks until the device ticket is decoded: n per-archive counters (a corrupt archive only sets its own status)."""
+        res = (_ffi.Counts * n)()
+        self._raise(self.lib.dll.nafgpu_pipeline_wait_counts(self._p, ticket, res, n))
+        return list(res)
+
+    def export(self, ticket: int, spec: "_ffi.Export", stream: int = 0):
+        """nafgpu_job_export on the ticket's lane (as Context.export); a refused export raises NafArgumentError."""
+        rc = self.lib.dll.nafgpu_pipeline_export(self._p, ticket, C.byref(spec), stream or None)
+        if rc == _ffi.ERR_ARGUMENT:
+            e = NafArgumentError(self.lib.strerror(rc) + ": " + self.lib.dll.nafgpu_pipeline_last_error(self._p).decode())
+            e.status = rc
+            raise e
+        self._raise(rc)
+
+    def release(self, ticket: int):
+        if self._p:                     # (after close the tickets went with the pipeline)
+            self._raise(self.lib.dll.nafgpu_pipeline_release(self._p, ticket))
 
     def stats(self):
         out = []

@@ -12,17 +12,26 @@ numbered across the job: archive 0's records first, then archive 1's; an archive
 The job stays in HBM while `recs` lives, so any number of exports can be taken from one decode.  `recs` owns a context for
 that time; closing or collecting it returns the context to a small per-device pool, so batch after batch allocates device
 memory once.
+
+`stream_to_device` does the same for a collection of any size: it cuts the input into sub-batches and decodes them on the
+lanes of a pipeline (nafgpu_pipeline_submit_device), so that the header walk and H2D of one sub-batch overlap the kernels of
+another, and yields one `DeviceRecords` per sub-batch, backed by its pipeline ticket instead of a pooled context.
+
+    for recs in stream_to_device(files, batch_bytes=256 << 20, lanes=2):
+        x, rows = recs.windows(1024, table="dna5")
+        recs.close()                                # hands the lane back
 """
 import ctypes as C
 import threading
 import weakref
+from collections import deque
 from typing import List, Optional
 
 import numpy as np
 
 from . import _ffi
-from .decoder import Context, _read_all, _want_bits, parse_archive
-from .errors import NafUnicodeError, raise_for_status
+from .decoder import Context, Pipeline, _read_all, _want_bits, parse_archive
+from .errors import NafError, NafUnicodeError, raise_for_status
 
 
 def _presets():
@@ -105,14 +114,26 @@ def _resolve_device(device, lib):
     return dev, 0
 
 
-class DeviceRecords:
-    """A decoded job kept in device memory; every method returns torch tensors on `device` (see the module docstring)."""
+class _Ticket:
+    """A device ticket of a pipeline, as what backs a DeviceRecords: its exports run on the ticket's lane."""
 
-    def __init__(self, ctx: Context, archives, want: int, device, counts):
+    def __init__(self, pipe: Pipeline, ticket: int):
+        self.pipe, self.ticket = pipe, ticket
+
+    def export(self, spec, stream=0):
+        self.pipe.export(self.ticket, spec, stream)
+
+
+class DeviceRecords:
+    """A decoded job kept in device memory; every method returns torch tensors on `device` (see the module docstring).
+    `first_archive` is the input index of the job's archive 0 (nonzero for the sub-batches of stream_to_device)."""
+
+    def __init__(self, ctx, archives, want: int, device, counts, release=None, first_archive: int = 0):
         self.device = device
-        self._ctx = ctx
+        self._ctx = ctx                 # what holds the decoded job: a pooled Context, or a pipeline ticket (_Ticket)
         self._want = want
-        self._finalizer = weakref.finalize(self, _give, (ctx.lib.path, ctx.device), ctx)
+        self.first_archive = first_archive
+        self._finalizer = weakref.finalize(self, *(release or (_give, (ctx.lib.path, ctx.device), ctx)))
         self._counts = counts
         self.status = [c.status for c in counts]
         self.first_bad_record = [None if c.first_bad_record == _ffi.NO_RECORD else int(c.first_bad_record) for c in counts]
@@ -128,7 +149,8 @@ class DeviceRecords:
 
     # -- life time -----------------------------------------------------------------------------------------------------------
     def close(self):
-        """Returns the context (and with it the decoded job) to the pool; tensors already exported stay valid."""
+        """Returns the context to the pool, or the ticket to its pipeline, and with it the decoded job; tensors already exported
+        stay valid."""
         self._finalizer()
 
     def __enter__(self):
@@ -266,14 +288,196 @@ def decode_to_device(files, *, id: bool = False, comment: bool = False, sequence
     recs = DeviceRecords(ctx, archives, want, dev, counts)
     if strict:
         n = len(counts)
-        for i, c in enumerate(counts):
-            if c.status:
-                recs.close()
-                raise_for_status(lib, c.status, None, f"archive {i} of {n}" if n > 1 else "")
-        for i, c in enumerate(counts):
-            if c.record_status:
-                recs.close()
-                e = NafUnicodeError(f"failed to decode UTF-8 data [archive {i}, record {c.first_bad_record}]")
-                e.status, e.archive, e.record = c.record_status, i, int(c.first_bad_record)
-                raise e
+        try:
+            _raise_for_counts(lib, counts, 0, lambda i: f"archive {i} of {n}" if n > 1 else "")
+        except BaseException:
+            recs.close()
+            raise
     return recs
+
+
+# ---- streaming a collection through the pipeline's device tickets ------------------------------------------------------------
+_MAX_SUB_BATCH = 65535            # archives of one job (nafgpu_decode_batch)
+
+
+def _sub_batches(files, batch_bytes, lib):
+    """(first input index, [archive], exception) for contiguous runs of `files`, read one archive ahead of the sub-batch being
+    cut.  A sub-batch ends where the next archive would take it past batch_bytes of compressed input, or at 65535 archives; an
+    input that cannot be read or parsed ends the runs with (its index, [], the exception)."""
+    part, first, size = [], 0, 0
+    for i, f in enumerate(files):
+        try:
+            data = _read_all(f)
+            a = parse_archive(data, lib)
+        except Exception as e:
+            if part:
+                yield first, part, None
+            yield i, [], e
+            return
+        if part and (size + len(data) > batch_bytes or len(part) == _MAX_SUB_BATCH):
+            yield first, part, None
+            part, first, size = [], i, 0
+        part.append(a)
+        size += len(data)
+    if part:
+        yield first, part, None
+
+
+def _shutdown(pipe, inflight, yielded):
+    """Ends a stream: every ticket in flight is waited for and released, every yielded DeviceRecords still open is closed, and
+    the pipeline (its lane threads and contexts) is destroyed."""
+    try:
+        for _, part, ticket, _ in inflight:
+            if part is None:
+                continue
+            try:
+                pipe.wait_counts(ticket, len(part))
+            except Exception:
+                pass                    # (a failed sub-batch is released all the same)
+            pipe.release(ticket)
+        inflight.clear()
+        for ref in yielded:
+            r = ref()
+            if r is not None:
+                r.close()
+        yielded.clear()
+    finally:
+        pipe.close()
+
+
+class DeviceStream:
+    """The iterator stream_to_device returns (see there).  close() ends it early; so do an exception and garbage collection."""
+
+    def __init__(self, files, batch_bytes, lanes, device, want, strict, lib):
+        self.lanes = lanes
+        self._lib, self._want, self._strict = lib, want, strict
+        self._device, index = _resolve_device(device, lib)
+        self._pieces = _sub_batches(files, batch_bytes, lib)
+        self._pending = None            # a sub-batch read but not submitted (all lanes were held)
+        self._exhausted = False
+        self._pipe = Pipeline(index, lanes, lib)
+        self._inflight = deque()        # (first, [archive], ticket, archive array) submitted; (first, None, None, exception)
+        self._yielded = []              # weak references to the DeviceRecords yielded (open until closed or collected)
+        self._finalizer = weakref.finalize(self, _shutdown, self._pipe, self._inflight, self._yielded)
+
+    def __iter__(self):
+        return self
+
+    def close(self):
+        self._finalizer()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+        return False
+
+    def _open(self):
+        self._yielded[:] = [r for r in self._yielded if r() is not None and r()._finalizer.alive]
+        return len(self._yielded) + sum(1 for e in self._inflight if e[1] is not None)
+
+    def _fill(self):
+        """Submits sub-batches while fewer than `lanes` tickets are in flight or yielded and open."""
+        while not self._exhausted:
+            if self._pending is None:
+                if self._inflight and self._open() >= self.lanes:
+                    return              # (with nothing in flight, one sub-batch is read to tell the input's end from held lanes)
+                self._pending = next(self._pieces, None)
+                if self._pending is None:
+                    self._exhausted = True
+                    return
+            first, part, err = self._pending
+            if err is not None:
+                self._inflight.append((first, None, None, err))
+                self._pending = None
+                continue
+            if self._open() >= self.lanes:
+                return
+            ticket, arr = self._pipe.submit_device(part, self._want)
+            self._inflight.append((first, part, ticket, arr))
+            self._pending = None
+
+    def __next__(self) -> DeviceRecords:
+        if not self._finalizer.alive:
+            raise StopIteration
+        try:
+            self._fill()
+            if not self._inflight:
+                if self._exhausted:
+                    raise StopIteration
+                raise _AllLanesHeld(f"{self.lanes} DeviceRecords of this stream are open: close a DeviceRecords before asking for "
+                                    f"more than lanes={self.lanes}")
+            first, part, ticket, arr = self._inflight.popleft()
+            if part is None:
+                raise _at_input(arr, first)
+            try:
+                counts = self._pipe.wait_counts(ticket, len(part))
+            except BaseException:
+                self._pipe.release(ticket)
+                raise
+            recs = DeviceRecords(_Ticket(self._pipe, ticket), part, self._want, self._device, counts,
+                                 release=(self._pipe.release, ticket), first_archive=first)
+            self._yielded.append(weakref.ref(recs))
+            if self._strict:
+                _raise_for_counts(self._lib, counts, first, lambda i: f"archive {first + i} of the input")
+            return recs
+        except _AllLanesHeld:
+            raise                       # the stream goes on once a DeviceRecords is closed
+        except BaseException:
+            self.close()
+            raise
+
+
+class _AllLanesHeld(RuntimeError):
+    pass
+
+
+def _at_input(e, index):
+    """The exception reading or parsing input `index` raised, naming the index."""
+    if isinstance(e, NafError):
+        named = type(e)(f"{e} [archive {index} of the input]")
+        named.status = e.status
+        named.__cause__ = e
+        return named
+    e.add_note(f"reading archive {index} of the input")
+    return e
+
+
+def _raise_for_counts(lib, counts, first, label):
+    """strict=True: the first failed archive raises as Context.decode does (its message ends with label(i)), then the first
+    text that is not UTF-8 (NafUnicodeError with .archive = first + i and .record)."""
+    for i, c in enumerate(counts):
+        if c.status:
+            raise_for_status(lib, c.status, None, label(i))
+    for i, c in enumerate(counts):
+        if c.record_status:
+            e = NafUnicodeError(f"failed to decode UTF-8 data [archive {first + i}, record {c.first_bad_record}]")
+            e.status, e.archive, e.record = c.record_status, first + i, int(c.first_bad_record)
+            raise e
+
+
+def stream_to_device(files, *, batch_bytes: int = 256 << 20, lanes: int = 2, device="cuda:0", id: bool = False,
+                     comment: bool = False, sequence: bool = True, quality: bool = True, mask: bool = True, strict: bool = True,
+                     _library=None) -> DeviceStream:
+    """Decodes a collection of archives into device memory in sub-batches, yielding one DeviceRecords per sub-batch in input
+    order.  `files` is any iterable of archives (bytes, paths or file objects), read lazily.  A sub-batch is a contiguous run
+    of the input that ends where the next archive would take it past `batch_bytes` of compressed input, or at 65535 archives;
+    an archive larger than batch_bytes is a sub-batch of its own.  `recs.first_archive` is the input index of the sub-batch's
+    first archive, so input archive recs.first_archive + a holds records [recs.archive_records[a], recs.archive_records[a + 1]).
+
+    The sub-batches are decoded on `lanes` lanes of a pipeline.  At most `lanes` of them are in flight or yielded and not yet
+    closed: close each DeviceRecords when done with it (that hands its lane back; tensors already exported stay valid).  Asking
+    for the next one while `lanes` are open raises RuntimeError and the stream goes on once one is closed.  When the stream
+    ends (exhausted, an exception, close() or garbage collection) every ticket in flight is released, every DeviceRecords it
+    yielded is closed and the pipeline's threads are gone.
+
+    strict=True raises as decode_to_device does at the sub-batch that holds a corrupt archive or text that is not UTF-8, after
+    the sub-batches before it have been yielded, naming the input index; with strict=False statuses are carried as there.
+    An input that cannot be read or is not a NAF archive raises at its sub-batch either way."""
+    lib = _library or _ffi.default_library()
+    if int(batch_bytes) <= 0:
+        raise ValueError("batch_bytes must be positive")
+    if not 1 <= int(lanes) <= 64:
+        raise ValueError("lanes must be in [1, 64]")
+    return DeviceStream(files, int(batch_bytes), int(lanes), device, _want_bits(id, comment, sequence, quality, mask), strict, lib)

@@ -214,4 +214,10 @@ extern "C" {
     pub fn nafgpu_job_counts(ctx: *mut nafgpu_ctx, out: *mut nafgpu_counts, n: u32) -> c_int;
     /// enqueued on `stream` (a cudaStream_t; null = the context's stream), ordered after the run and before the context's next call
     pub fn nafgpu_job_export(ctx: *mut nafgpu_ctx, spec: *const nafgpu_export, stream: *mut c_void) -> c_int;
+    /// a device ticket: the lane decodes and reads the counters, the sub-batch stays in its arena until release
+    pub fn nafgpu_pipeline_submit_device(p: *mut nafgpu_pipeline, archives: *const nafgpu_archive, n: u32, want: u32) -> i64;
+    /// the archives are borrowed until this returns; per-archive failures are in out[i].status
+    pub fn nafgpu_pipeline_wait_counts(p: *mut nafgpu_pipeline, ticket: i64, out: *mut nafgpu_counts, n: u32) -> c_int;
+    /// nafgpu_job_export on the ticket's lane (after wait_counts, before release)
+    pub fn nafgpu_pipeline_export(p: *mut nafgpu_pipeline, ticket: i64, spec: *const nafgpu_export, stream: *mut c_void) -> c_int;
 }
