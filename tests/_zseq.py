@@ -154,6 +154,7 @@ _PREDEF = {  # RFC 8878 3.1.1.3.2.2: (accuracy log, distribution)
     "ml": (6, [1, 4, 3, 2, 2, 2, 2, 2, 2] + [1] * 37 + [-1] * 7),
 }
 _MAX_SYM = {"ll": 35, "of": 31, "ml": 52}
+_MAX_AL = {"ll": 9, "of": 8, "ml": 9}
 MODE_NAMES = ("predefined", "rle", "fse", "repeat")
 
 
@@ -325,6 +326,7 @@ def _read_block(c, b, reps, prev):
     else:
         n = c[q + 1] + (c[q + 2] << 8) + 0x7F00; q += 3
     b.modes = c[q]; q += 1
+    assert b.modes & 3 == 0, "reserved mode bits set"
     tables = {}
     for kind, shift in (("ll", 6), ("of", 4), ("ml", 2)):
         mode = (b.modes >> shift) & 3
@@ -333,16 +335,20 @@ def _read_block(c, b, reps, prev):
             al, norm = _PREDEF[kind]
             tables[kind] = (al, _fse_table(al, norm))
         elif mode == 1:
+            assert c[q] <= _MAX_SYM[kind], f"RLE {kind} symbol {c[q]}"
             tables[kind] = (0, [(c[q], 0, 0)]); q += 1
         elif mode == 2:
             al, norm, used = _read_ncount(c, q, _MAX_SYM[kind]); q += used
+            assert al <= _MAX_AL[kind] and q <= len(c), f"{kind} accuracy log {al}, or description past the block"
             tables[kind] = (al, _fse_table(al, norm))
             b.al[kind] = al
         else:
+            assert prev[kind] is not None, "repeat mode without an earlier table"
             tables[kind] = prev[kind]
         prev[kind] = tables[kind]
     (all_, tll), (aof, tof), (aml, tml) = tables["ll"], tables["of"], tables["ml"]
     b.seq_bytes = len(c) - q
+    assert b.seq_bytes and c[-1] != 0, "sequence bitstream empty or without end marker"
     rd = _Back(bytes(c[q:]))
     sll, sof, sml = rd.read(all_), rd.read(aof), rd.read(aml)
     for i in range(n):
