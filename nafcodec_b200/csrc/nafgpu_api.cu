@@ -187,7 +187,7 @@ struct nafgpu_ctx {
     zk::Streams streams;
     cudaEvent_t ev_block = nullptr, ev_d2h = nullptr;
     std::string err;
-    DevBuf comp, arena, lit, desc, bstate, hufw, fsstate, lzidx, scanagg, debug, tables, table_al, seq32, seq64, misc, flush, text, fin_g, pack_in, pack_out;
+    DevBuf comp, arena, lit, desc, bstate, hufw, hufb, fsstate, lzidx, scanagg, debug, tables, table_al, seq32, seq64, misc, flush, text, fin_g, pack_in, pack_out;
     size_t o_frames = 0, o_naf = 0, o_huf = 0, o_chunks = 0, o_gbase = 0, o_tiles = 0, o_big = 0, o_bigseq = 0, o_biglit = 0;   // layout of `desc` (blocks at 0): one H2D copy for all descriptors
     PinBuf stage, result, misc_host, text_host, text_stage, pack_host;
     fw::JobPlan plan;                  // frames, Huffman items and totals of the job (block descriptors live in the tasks)
@@ -731,6 +731,7 @@ int stage_descriptors(nafgpu_ctx* c, uint32_t n, size_t nb, const std::vector<Co
               c->desc.ensure(stage_bytes + 64) && c->fin_g.ensure((size_t)g_base[nf] * 4 + 256 + (size_t)S.total_chunks * 8192) &&
               c->bstate.ensure(nb * sizeof(zf::BlockState) + 64) && c->fsstate.ensure(tiles.size() * sizeof(zf::FsTileState) + 64) && c->lzidx.ensure(((size_t)S.total_chunks * 16 + nf + 16) * 4) &&
               c->scanagg.ensure((size_t)n * 4 * ((c->max_scan + nk::NAF_SLICE - 1) / nk::NAF_SLICE + 1) * nk::NAF_AGG_BYTES + 64) && c->hufw.ensure((size_t)pl.n_huf_slots * 258 + 64) &&
+              c->hufb.ensure((size_t)pl.n_huf_big * 1024 + 64) &&
               c->tables.ensure((size_t)pl.n_slots * zf::FSE_SLOT_CELLS * sizeof(zc::SeqCell)) && c->table_al.ensure(pl.n_slots + 64) &&
               c->seq32.ensure(nseq * 5 * 4 + 64) && c->seq64.ensure(nseq * sizeof(zf::SeqRec) + 64) && c->misc.ensure(c->misc_words * 4);
     if (!ok) return fail(c, NAFGPU_ERR_NOMEM, "device allocation failed");
@@ -821,7 +822,7 @@ int bind_job(nafgpu_ctx* c, size_t nb, const Staged& S, const zk::Overrides& ov)
     J.fin_g = (uint32_t*)c->fin_g.p; J.fin_ext = (uint32_t*)c->fin_g.p + S.g_entries + 64;
     J.fin_g_base = (const uint64_t*)(desc + c->o_gbase);
     J.huf_weights = (uint8_t*)c->hufw.p; J.huf_meta = (uint8_t*)c->hufw.p + (size_t)pl.n_huf_slots * 256;
-    J.huf_items = (const zf::HufItem*)(desc + c->o_huf); J.n_huf_items = (uint32_t)nh; J.n_huf_big = pl.n_huf_big; J.max_huf_stream = pl.max_huf_stream; J.max_huf_small = pl.max_huf_small;
+    J.huf_items = (const zf::HufItem*)(desc + c->o_huf); J.huf_bounds = (uint32_t*)c->hufb.p; J.n_huf_items = (uint32_t)nh; J.n_huf_big = pl.n_huf_big; J.max_huf_stream = pl.max_huf_stream; J.max_huf_small = pl.max_huf_small;
     J.debug = nullptr; J.debug_seq = nullptr;
     if (ov.debug_huf && nh) {
         if (!c->debug.ensure(nh * 64 + 64)) return fail(c, NAFGPU_ERR_NOMEM, "debug buffer");
@@ -989,7 +990,7 @@ void nafgpu_ctx_destroy(nafgpu_ctx* c) {
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->streams.st);
     drop_graph(c);
-    DevBuf* d[] = {&c->comp, &c->arena, &c->lit, &c->desc, &c->bstate, &c->hufw, &c->fsstate, &c->lzidx, &c->scanagg, &c->debug, &c->tables, &c->table_al, &c->seq32, &c->seq64, &c->misc, &c->flush, &c->text, &c->fin_g, &c->pack_in, &c->pack_out, &c->exp_desc};
+    DevBuf* d[] = {&c->comp, &c->arena, &c->lit, &c->desc, &c->bstate, &c->hufw, &c->hufb, &c->fsstate, &c->lzidx, &c->scanagg, &c->debug, &c->tables, &c->table_al, &c->seq32, &c->seq64, &c->misc, &c->flush, &c->text, &c->fin_g, &c->pack_in, &c->pack_out, &c->exp_desc};
     for (DevBuf* b : d) b->release();
     c->stage.release(); c->result.release(); c->misc_host.release(); c->text_host.release(); c->text_stage.release(); c->pack_host.release(); c->win.release();
     c->exp_stage.release();

@@ -10,6 +10,7 @@
 //                   k_frame_scan (+ k_fs_reduce / k_fs_prefix / k_fs_apply for frames of 10^4+ blocks)
 //                                            per frame: block output offsets (prefix sum) + repeat-offset carry across blocks
 //   Huffman branch  k_build_tables<1>        per block: Huffman tree description -> 256 weights, once per tree
+//                   k_huf_scout              per big block: the exact start and output offset of every range of its four streams
 //                   k_huf_decode_block       per big block: intra-stream parallel decode of its four streams into the literal staging buffer
 //                   k_huf_decode_big         the same per stream, four CTAs of a block as a cluster (DSMEM): a job of a few blocks
 //                   k_huf_decode<128>        short streams
@@ -68,6 +69,7 @@ __device__ __forceinline__ saddr_t to_saddr(const void* p) { return (saddr_t)__c
 __device__ __forceinline__ uint32_t lds32(saddr_t a) { uint32_t v; asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
 __device__ __forceinline__ uint2 lds64(saddr_t a) { uint2 v; asm volatile("ld.shared.v2.u32 {%0, %1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(a)); return v; }
 __device__ __forceinline__ uint32_t lds16(saddr_t a) { uint16_t v; asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(a)); return v; }
+__device__ __forceinline__ uint32_t lds8(saddr_t a) { uint32_t v; asm volatile("ld.shared.u8 %0, [%1];" : "=r"(v) : "r"(a)); return v; }
 __device__ __forceinline__ void sts8(saddr_t a, uint32_t v) { asm volatile("st.shared.u8 [%0], %1;" :: "r"(a), "r"(v)); }
 __device__ __forceinline__ void sts32(saddr_t a, uint32_t v) { asm volatile("st.shared.u32 [%0], %1;" :: "r"(a), "r"(v)); }
 #else
@@ -76,6 +78,7 @@ static inline saddr_t to_saddr(const void* p) { return (saddr_t)p; }
 static inline uint32_t lds32(saddr_t a) { return *(const uint32_t*)a; }
 static inline uint2 lds64(saddr_t a) { return *(const uint2*)a; }
 static inline uint32_t lds16(saddr_t a) { return *(const uint16_t*)a; }
+static inline uint32_t lds8(saddr_t a) { return *(const uint8_t*)a; }
 static inline void sts8(saddr_t a, uint32_t v) { *(uint8_t*)a = (uint8_t)v; }
 static inline void sts32(saddr_t a, uint32_t v) { *(uint32_t*)a = v; }
 #endif
@@ -1151,10 +1154,12 @@ __device__ __forceinline__ uint64_t map_compose(uint64_t g, uint64_t f) {
 }
 constexpr uint64_t MAP_IDENTITY = 0xFEDCBA9876543210ull;
 
-// Entries [lo, hi) of the two tables over 12-bit windows, from the finished base table: decode the window while whole
+// Entries [lo, hi) of the tables over 12-bit windows, from the finished base table: decode the window while whole
 // codewords fit (no barrier inside; the caller separates it from the base-table build and from the first use).
+//   tc (optional): count table, entry = bits of all whole codewords | their number << 4 (both <= 12)
 template <int HUF_T, bool MULTI>
-__device__ __forceinline__ void huf_build_wide(const uint16_t* table, int maxbits, uint16_t* bm, uint32_t* t3, uint32_t lo, uint32_t hi) {
+__device__ __forceinline__ void huf_build_wide(const uint16_t* table, int maxbits, uint16_t* bm, uint32_t* t3, uint32_t lo, uint32_t hi,
+                                               uint8_t* tc = nullptr) {
     const int sh1 = HUF_W - maxbits;
     for (uint32_t i = lo + threadIdx.x; i < hi; i += HUF_T) {
         uint32_t used = 0, n = 0, syms = 0, used3 = 0, mask = 0;
@@ -1169,6 +1174,7 @@ __device__ __forceinline__ void huf_build_wide(const uint16_t* table, int maxbit
         }
         if (bm) bm[i] = (uint16_t)mask;
         if (MULTI) t3[i] = syms | (used3 << 24) | (n << 28);
+        if (tc) tc[i] = (uint8_t)(used | ((uint32_t)__popc(mask) << 4));
     }
 }
 
@@ -1779,17 +1785,18 @@ __global__ void HB_CLUSTER_ATTR __launch_bounds__(HB_T, 3) k_huf_decode_big(JobD
     }
 }
 
-// The counting legs of k_huf_decode_block: like track_advance, but the steady state reads the 3-symbol table (bits used and
-// symbol count are in its top byte) and the exact stop at `lim` walks single symbols with the base table.
-__device__ __forceinline__ void track_advance3(saddr_t comp, saddr_t t3, saddr_t t1, int maxbits, int xtop, int& q, int& cnt, int lim) {
+// The counting legs of k_huf_scout: like track_advance, but the steady state reads the count table (bits and number of all
+// whole codewords of the next 12 bits: one byte, no bit tricks) and the exact stop at `lim` walks single symbols with the
+// base table.
+__device__ __forceinline__ void track_count(saddr_t comp, saddr_t tc, saddr_t t1, int maxbits, int xtop, int& q, int& cnt, int lim) {
     int rem = lim - q;
     if (rem <= 0) return;
     Win w;
     win_init(w, comp, xtop - q);
     while (rem > HUF_W) {
-        const uint32_t e = lds32(t3 + win_peek_x4(w));
-        const int used = (int)(e >> 24) & 15;
-        cnt += (int)(e >> 28);
+        const uint32_t e = lds8(tc + win_peek(w));
+        const int used = (int)(e & 15u);
+        cnt += (int)(e >> 4);
         rem -= used;
         win_consume(w, used);
     }
@@ -1803,25 +1810,282 @@ __device__ __forceinline__ void track_advance3(saddr_t comp, saddr_t t3, saddr_t
     q = lim - rem;
 }
 
-// k_huf_decode_block: the same decode, ONE CTA PER BLOCK working through the block's four streams one after the other.  The
-// tables (base table, 3-symbol table) are built once per block by the CTA itself -- no cluster, no exchange -- and stay in
-// shared memory for all four streams; the counting legs read the 3-symbol table too (bits used, symbols), so the boundary-mask
-// table is gone, and with it the two XU-pipe instructions per lookup that decoded it; the exact stop at a checkpoint walks
-// single symbols with the base table.  The next stream's bytes are fetched (bulk asynchronous copy) while the current
-// stream's output is flushed.  Measured against the cluster version on the 256-archive job: see profiles/r2_summary.md.
+// k_huf_scout: where every range of k_huf_decode_block starts, for the block's four streams at once (one CTA per block, one
+// thread per COARSE range of HS_F consecutive fine ranges; the fine ranges are k_huf_decode_block's 256 ranges of S bits).
+// The speculation of the cluster kernel's phase 1 -- all max_bits candidates at the top of a range, tracks merging at
+// checkpoints 12, 108 and 320 bits in -- is paid once per coarse range instead of once per fine range; from the end of the
+// first fine range on, the (nearly always single) surviving track is followed to the next fine boundary, and so on.  Every
+// leg between checkpoints is dealt out as work items over the whole CTA (all four streams), as in k_huf_decode_big.
+// Leg tables, one slot per fine range: [slot][range][landing offset at the top] = landing offset at the end | symbols << 4;
+// slot 0 holds the first fine range composed (indexed by the offset where the first stop landed), slots 1..3 serve the legs
+// inside the first fine range until it is composed, then the further fine ranges.  The coarse maps are composed along each
+// stream (64 entries: two warps), the true candidate of every coarse range resolves the chain of its fine ranges, and a
+// scan of the symbol counts gives their output offsets.  Output: J.huf_bounds, 256 words per stream (fine range order):
+// output offset << 4 | start offset (bits below the top of the range).
+// The four compressed streams are staged side by side (bulk asynchronous copies): the counting reads them about 1.3 times.
+// Shared memory: 36.3 KB + 4 stream images (cfg2: 101 KB, 2 CTAs per SM); ptxas (sm_100a): 55 registers, no spills.
+constexpr int HS_C = 64;                                    // coarse ranges per stream
+constexpr int HS_T = 4 * HS_C;                              // threads: the coarse ranges of the block's four streams
+constexpr int HS_F = HB_T / HS_C;                           // fine ranges per coarse range
+constexpr int HS_NLEG = HB_NLEG + HS_F - 1;                 // legs after the first stop
+static_assert(HS_T == HB_T && HS_F > HB_NLEG, "k_huf_scout: one scan shape with k_huf_decode_block; slots 1..3 for the first fine range's legs");
+constexpr uint32_t HS_LEG_BYTES = HS_F * HS_T * MAXC * 2u, HS_Q_BYTES = HS_T * MAXC * 2u;
+constexpr uint32_t HS_FIXED = 4096u + 768u + 4096u + HS_LEG_BYTES + HS_Q_BYTES;   // t1 | weights, wcnt, misc | count table | leg tables | queue
+__host__ __device__ constexpr uint32_t hs_image_bytes(uint32_t max_stream) { return (max_stream + 15u + 16u + 16u + 15u) & ~15u; }
+__host__ __device__ constexpr uint32_t hs_smem_bytes(uint32_t max_stream) { return HS_FIXED + 4u * hs_image_bytes(max_stream); }
+
+// checkpoint j of a coarse range (bits below the top of the stream): the first stop's limit, two more inside the first fine
+// range, then the fine boundaries; never past the end of the stream
+__device__ __forceinline__ int hs_checkpoint(int ctop, int S, int P0, int j) {
+    const int ck = j == 0 ? HB_CK0 : j == 1 ? HB_CK1 : HB_CK2;
+    const int rel = j < HB_NLEG ? (S < ck ? S : ck) : (j - HB_NLEG + 1) * S;
+    return ctop + rel < P0 ? ctop + rel : P0;
+}
+
+__global__ void __launch_bounds__(HS_T, 2) k_huf_scout(JobDev J) {
+    NAF_DYN_SMEM(unsigned char, smem);
+    uint16_t* t1 = (uint16_t*)smem;
+    uint8_t* weights = smem + 4096;
+    uint16_t* wcnt = (uint16_t*)(smem + 4096 + 256);
+    uint32_t* misc = (uint32_t*)(smem + 4096 + 512);                    // [0..15] scan buffers, [16..23] warp start candidates,
+                                                                        // [24..39] per stream: XTOP, P0, S; [56..57] mbarrier
+    uint64_t* wmap = (uint64_t*)(smem + 4096 + 256);                    // [8] composed map of each warp (reuses wcnt after the table build)
+    uint8_t* tc = smem + 4864;
+    uint16_t* legtab = (uint16_t*)(smem + 4864 + 4096);
+    uint16_t* qitems = (uint16_t*)(smem + 4864 + 4096 + HS_LEG_BYTES);  // range | offset << 8
+    uint8_t* images = smem + HS_FIXED;
+    const uint32_t stride = hs_image_bytes(J.max_huf_stream);
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int s = tid / HS_C, c = tid % HS_C;                            // stream, coarse range
+
+    const uint32_t item0 = blockIdx.x * 4u;
+    const BlockDesc& B = J.blocks[J.huf_items[item0].block];
+    const HufItem it = J.huf_items[item0 + s];
+    const uint8_t* g = J.comp + B.src_off + it.src_off;
+    const uint32_t a = (uint32_t)((uintptr_t)g & 15);
+    const uint32_t bytes = ((a + it.src_size + 15u) >> 4) << 4;
+    uint8_t* img = images + s * stride;                                 // 16 zero bytes, then the 16 B-aligned image of global memory
+#if defined(__CUDA_ARCH__)
+    const uint32_t mbar = (uint32_t)__cvta_generic_to_shared(&misc[56]);
+    if (tid == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(mbar), "r"(4));
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    if (c == 0) {
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(mbar), "r"(bytes) : "memory");
+        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                     :: "r"((uint32_t)__cvta_generic_to_shared(img + 16)), "l"(g - a), "r"(bytes), "r"(mbar) : "memory");
+    }
+#else
+    for (uint32_t k = c; k < (bytes >> 4); k += HS_C) ((uint4*)(img + 16))[k] = ((const uint4*)(g - a))[k];
+#endif
+    for (int i = tid; i < 64; i += HS_T) ((uint32_t*)weights)[i] = ((const uint32_t*)(J.huf_weights + (size_t)B.huf_slot * 256))[i];
+    const int nsym = (int)J.huf_meta[(size_t)B.huf_slot * 2] + 1, maxbits = (int)J.huf_meta[(size_t)B.huf_slot * 2 + 1];
+    __syncthreads();
+    if (maxbits != 0) {                                                 // (a bad tree was flagged by k_build_tables)
+        huf_build_t1<HS_T>(weights, nsym, maxbits, t1, wcnt);
+        huf_build_wide<HS_T, false>(t1, maxbits, nullptr, nullptr, 0u, 1u << HUF_W, tc);
+    }
+    // a tree whose codes all have the same length never lets tracks merge -- and does not need to: the codeword boundaries
+    // are the multiples of that length
+    const bool fixed_len = !__syncthreads_or(tid < 128 && (tid & 15) >= 2 && (tid & 15) <= zc::HUF_MAX_BITS && wcnt[tid] != 0);
+    // (one thread reads the flag: another stream's kernel may set it at any moment, and the decision must be the CTA's)
+    const bool skip = __syncthreads_or(maxbits == 0 || (tid == 0 && J.frame_bad[B.frame] != 0));
+#if defined(__CUDA_ARCH__)
+    {   // the bulk copies have landed (also before an early exit: the shared memory must not be handed on under them)
+        uint32_t done;
+        do {
+            asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
+                         : "=r"(done) : "r"(mbar), "r"(0) : "memory");
+        } while (!done);
+    }
+#endif
+    if (skip) return;
+    if ((uint32_t)c < 16 + a) img[c] = 0;                                // bits below the stream start read as zero
+    const uint8_t last = img[16 + a + it.src_size - 1];
+    if (__syncthreads_or(last == 0)) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); return; }
+
+    // q = distance (in bits) from the top of the stream; smem bit position x = XTOP - q
+    const int P0 = 8 * (int)(it.src_size - 1) + zc::highbit32(last);
+    const int XTOP = (int)(16 + a) * 8 + P0;
+    int S = (P0 + HB_T - 1) / HB_T;                                     // fine ranges: exactly k_huf_decode_block's
+    if (S < 2 * MAXC) S = 2 * MAXC;
+    if (c == 0) { misc[24 + 4 * s] = (uint32_t)XTOP; misc[25 + 4 * s] = (uint32_t)P0; misc[26 + 4 * s] = (uint32_t)S; }
+    const int ctop = c * HS_F * S;
+    const bool active = ctop < P0;
+    const saddr_t s_images = to_saddr(images), s_tc = to_saddr(tc), s_t1 = to_saddr(t1);
+    const saddr_t s_comp = s_images + s * stride;
+
+    // (1) first stop: every candidate lands on its first codeword boundary at or past checkpoint 0
+    uint64_t first = ~0ull, fcnt = 0;                                   // candidate -> landing offset / symbols so far (4 bits each)
+    uint32_t live = 0;                                                  // landing offsets in use at the current checkpoint
+    if (active) {
+        const int l0 = hs_checkpoint(ctop, S, P0, 0);
+        first = 0;
+        if (fixed_len) {
+            int q = ctop + (maxbits - ctop % maxbits) % maxbits, n = 0;
+            track_count(s_comp, s_tc, s_t1, maxbits, XTOP, q, n, l0);
+            first = (uint64_t)(uint32_t)(q - l0) * 0x1111111111111111ull;
+            fcnt = (uint64_t)(uint32_t)n * 0x1111111111111111ull;
+            live = 1u << (q - l0);
+        } else {
+            for (int k = 0; k < maxbits; k++) {
+                int q = ctop + k, n = 0;
+                track_count(s_comp, s_tc, s_t1, maxbits, XTOP, q, n, l0);
+                const uint32_t o = (uint32_t)(q - l0);
+                first |= (uint64_t)o << (4 * k);
+                fcnt |= (uint64_t)n << (4 * k);
+                live |= 1u << o;
+            }
+        }
+        if (maxbits < 16) first |= ~0ull << (4 * maxbits);              // candidates that cannot occur: dead (15)
+    }
+    // (2) legs between checkpoints: the live tracks of ALL coarse ranges are work items dealt out evenly over the CTA
+    auto slot_of = [](int leg) { return leg <= HB_NLEG ? leg : leg - HB_NLEG; };
+    auto tab = [&](int slot, int range, uint32_t o) { return to_saddr(legtab) + 2u * (((uint32_t)slot * HS_T + (uint32_t)range) * MAXC + o); };
+    uint32_t leg_done = 0, live1 = 0;
+    uint64_t land1 = 0;                                                 // first-stop landing -> landing at the end of fine range 0
+    for (int leg = 1; leg <= HS_NLEG; leg++) {
+        if (leg == HB_NLEG + 1) {                                       // the first fine range is complete: compose it into slot 0
+            if (active) {
+                uint32_t starts = 0;
+                for (int k = 0; k < maxbits; k++) starts |= 1u << ((uint32_t)(first >> (4 * k)) & 15u);
+                for (uint32_t m = starts; m; m &= m - 1) {
+                    const uint32_t o0 = (uint32_t)(__ffs((int)m) - 1);
+                    uint32_t o = o0, n = 0;
+                    for (int l = 1; l <= HB_NLEG; l++)
+                        if (leg_done & (1u << l)) { const uint32_t e = lds16(tab(l, tid, o)); o = e & 15u; n += e >> 4; }
+                    legtab[(uint32_t)tid * MAXC + o0] = (uint16_t)(o | (n << 4));
+                    land1 |= (uint64_t)o << (4 * o0);
+                }
+            }
+            live1 = live;
+        }
+        const int slot = slot_of(leg);
+        const uint32_t mine = (active && hs_checkpoint(ctop, S, P0, leg - 1) < hs_checkpoint(ctop, S, P0, leg)) ? live : 0u;
+        if (mine) leg_done |= 1u << leg;
+        uint32_t qtotal;
+        uint32_t idx = hb_scan((uint32_t)__popc(mine), misc + 8 * (leg & 1), &qtotal);
+        for (uint32_t m = mine; m; m &= m - 1) qitems[idx++] = (uint16_t)((uint32_t)tid | ((uint32_t)(__ffs((int)m) - 1) << 8));
+        __syncthreads();
+        for (uint32_t i = tid; i < qtotal; i += HS_T) {
+            const uint32_t item = qitems[i];
+            const int owner = (int)(item & 0xFFu), o = (int)(item >> 8);
+            const int os = owner / HS_C;
+            const int oxtop = (int)misc[24 + 4 * os], op0 = (int)misc[25 + 4 * os], oS = (int)misc[26 + 4 * os];
+            const int octop = (owner % HS_C) * HS_F * oS;
+            const int lim = hs_checkpoint(octop, oS, op0, leg);
+            int q = hs_checkpoint(octop, oS, op0, leg - 1) + o, n = 0;
+            track_count(s_images + os * stride, s_tc, s_t1, maxbits, oxtop, q, n, lim);
+            legtab[((uint32_t)slot * HS_T + (uint32_t)owner) * MAXC + (uint32_t)o] = (uint16_t)((uint32_t)(q - lim) | ((uint32_t)n << 4));
+        }
+        __syncthreads();
+        if (mine) {
+            uint32_t nl = 0;
+            for (uint32_t m = mine; m; m &= m - 1) nl |= 1u << (lds16(tab(slot, tid, (uint32_t)(__ffs((int)m) - 1))) & 15u);
+            live = nl;
+        }
+    }
+    // (3) the map candidate -> candidate of the next coarse range
+    uint64_t fmap = MAP_IDENTITY;
+    if (active) {
+        uint64_t exit_of = 0;                                           // landing at the end of fine range 0 -> at the end of the coarse range
+        for (uint32_t m = live1; m; m &= m - 1) {
+            const uint32_t o1 = (uint32_t)(__ffs((int)m) - 1);
+            uint32_t o = o1;
+#pragma unroll
+            for (int j = 1; j < HS_F; j++) if (leg_done & (1u << (HB_NLEG + j))) o = lds16(tab(j, tid, o)) & 15u;
+            exit_of |= (uint64_t)o << (4 * o1);
+        }
+        fmap = 0;
+        for (int k = 0; k < maxbits; k++) {
+            const uint32_t o1 = (uint32_t)(land1 >> (4 * ((uint32_t)(first >> (4 * k)) & 15u))) & 15u;
+            fmap |= ((exit_of >> (4 * o1)) & 15ull) << (4 * k);
+        }
+        if (maxbits < 16) fmap |= ~0ull << (4 * maxbits);
+    }
+    // ---- compose the maps along each stream: inclusive scan in the warp, then the stream's two warp totals ----------------
+    uint64_t inc_map = fmap;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint64_t o = __shfl_up_sync(0xFFFFFFFFu, inc_map, d);
+        const bool need = lane >= d && !map_is_const(inc_map, maxbits);
+        if (__any_sync(0xFFFFFFFFu, need)) { if (need) inc_map = map_compose(inc_map, o); }
+    }
+    uint64_t exc_map = __shfl_up_sync(0xFFFFFFFFu, inc_map, 1);
+    if (lane == 0) exc_map = MAP_IDENTITY;
+    if (lane == 31) wmap[warp] = inc_map;
+    __syncthreads();
+    constexpr int WPS = HS_C / 32;                                      // warps per stream
+    if (tid < 4) {
+        uint32_t k = 0;
+        for (int w = tid * WPS; w < (tid + 1) * WPS; w++) { misc[16 + w] = k; k = (uint32_t)(wmap[w] >> (4 * k)) & 15u; }
+    }
+    __syncthreads();
+    const uint32_t ktrue = (uint32_t)(exc_map >> (4 * misc[16 + warp])) & 15u;     // this coarse range's true candidate
+    // ---- the chain of the true track through the fine ranges: start offsets and symbols ------------------------------------
+    uint32_t start[HS_F], cnt[HS_F];
+#pragma unroll
+    for (int j = 0; j < HS_F; j++) { start[j] = 0; cnt[j] = 0; }
+    bool bad_end = false;
+    if (active) {
+        const bool at_end = ctop + HS_F * S >= P0;                      // the stream ends in this coarse range: the true track must land on P0
+        if (ktrue < (uint32_t)maxbits) {
+            const uint32_t o0 = (uint32_t)(first >> (4 * ktrue)) & 15u;
+            const uint32_t e0 = lds16(tab(0, tid, o0));
+            start[0] = ktrue;
+            cnt[0] = ((uint32_t)(fcnt >> (4 * ktrue)) & 15u) + (e0 >> 4);
+            uint32_t o = e0 & 15u;
+#pragma unroll
+            for (int j = 1; j < HS_F; j++) {
+                start[j] = o;
+                if (leg_done & (1u << (HB_NLEG + j))) { const uint32_t e = lds16(tab(j, tid, o)); o = e & 15u; cnt[j] = e >> 4; }
+            }
+            bad_end = at_end && o != 0;
+        } else {
+            bad_end = at_end;
+        }
+    }
+    uint32_t mine = 0;
+#pragma unroll
+    for (int j = 0; j < HS_F; j++) mine += cnt[j];
+    // ---- output offsets: exclusive scan of the symbols over each stream ------------------------------------------------
+    uint32_t inc = mine;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) { const uint32_t t = __shfl_up_sync(0xFFFFFFFFu, inc, d); if (lane >= d) inc += t; }
+    if (lane == 31) misc[warp] = inc;
+    __syncthreads();
+    uint32_t before = 0, total = 0;
+#pragma unroll
+    for (int w = 0; w < WPS; w++) { const uint32_t x = misc[s * WPS + w]; total += x; if (s * WPS + w < warp) before += x; }
+    if (__syncthreads_or(bad_end || total != it.n_sym)) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); return; }
+    uint32_t off = before + inc - mine;
+    uint32_t* dst = J.huf_bounds + (size_t)(item0 + s) * HB_T + (uint32_t)c * HS_F;
+#pragma unroll
+    for (int j = 0; j < HS_F; j += 4) {
+        uint32_t v[4];
+#pragma unroll
+        for (int u = 0; u < 4; u++) { v[u] = (off << 4) | start[j + u]; off += cnt[j + u]; }
+        *(uint4*)(dst + j) = make_uint4(v[0], v[1], v[2], v[3]);
+    }
+}
+
+// k_huf_decode_block: the write pass, ONE CTA PER BLOCK working through the block's four streams one after the other, every
+// thread from the exact start and output offset k_huf_scout found for its range.  The tables (base table, 3-symbol table) are
+// built once per block by the CTA itself -- no cluster, no exchange -- and stay in shared memory for all four streams.  The
+// next stream's bytes are fetched (bulk asynchronous copy) while the current stream's output is flushed.
 __global__ void __launch_bounds__(HB_T, 3) k_huf_decode_block(JobDev J) {
     NAF_DYN_SMEM(unsigned char, smem);
     uint16_t* t1 = (uint16_t*)smem;
     uint8_t* weights = smem + 4096;
     uint16_t* wcnt = (uint16_t*)(smem + 4096 + 256);
-    uint32_t* misc = (uint32_t*)(smem + 4096 + 512);                    // [0..15] two scan buffers, [16..23] warp start candidates, [56..57] mbarrier
-    uint64_t* wmap = (uint64_t*)(smem + 4096 + 256);                    // [HB_NW] composed map of each warp (reuses wcnt after the table build)
+    uint32_t* misc = (uint32_t*)(smem + 4096 + 512);                    // [56..57] mbarrier
     uint32_t* t3 = (uint32_t*)(smem + 4864);
     uint8_t* sout = smem + 4864 + 16384;
-    uint16_t* legtab = (uint16_t*)sout;                                 // [leg][range][offset] = landing offset | symbols << 4
-    uint16_t* qitems = (uint16_t*)(sout + HB_LEG_BYTES);                // range | offset << 8
     uint32_t* scomp = (uint32_t*)(smem + HB_FIXED);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x;
+    (void)misc;
 
     const uint32_t item0 = blockIdx.x * 4u;                              // the block's four streams are four consecutive items
     const BlockDesc& B = J.blocks[J.huf_items[item0].block];
@@ -1859,13 +2123,12 @@ __global__ void __launch_bounds__(HB_T, 3) k_huf_decode_block(JobDev J) {
         huf_build_t1<HB_T>(weights, nsym, maxbits, t1, wcnt);
         huf_build_wide<HB_T, true>(t1, maxbits, nullptr, t3, 0u, 1u << HUF_W);
     }
-    // a tree whose codes all have the same length (e.g. 16 equiprobable byte values) never lets tracks merge -- and does not
-    // need to: the codeword boundaries are the multiples of that length
-    const bool fixed_len = !__syncthreads_or(tid < 128 && (tid & 15) >= 2 && (tid & 15) <= zc::HUF_MAX_BITS && wcnt[tid] != 0);
-    // (one thread reads the flag: another stream's kernel may set it at any moment, and the decision must be the CTA's)
+    // (one thread reads the flag: k_huf_scout flags every stream it refuses, and another stream's kernel may set it at any
+    // moment -- the decision must be the CTA's)
     const bool skip = __syncthreads_or(maxbits == 0 || (tid == 0 && J.frame_bad[B.frame] != 0));
     for (uint32_t sidx = 0; sidx < 4u; sidx++) {
     const HufItem it = J.huf_items[item0 + sidx];
+    const uint32_t bound = skip ? 0u : J.huf_bounds[(size_t)(item0 + sidx) * HB_T + tid];     // output offset << 4 | start offset
     const uint8_t* g = J.comp + B.src_off + it.src_off;
     const uint32_t a = (uint32_t)((uintptr_t)g & 15);
 #if defined(__CUDA_ARCH__)
@@ -1881,135 +2144,22 @@ __global__ void __launch_bounds__(HB_T, 3) k_huf_decode_block(JobDev J) {
     if ((uint32_t)tid < 16 + a) ((uint8_t*)scomp)[tid] = 0;              // bits below the stream start read as zero
     __syncthreads();
 
-    // ---- phase 1: transition map of every range -------------------------------------------------------------------------
-    // q = distance (in bits) from the top of the stream; smem bit position x = XTOP - q.
-    const int Z = (int)(16 + a) * 8;
+    // q = distance (in bits) from the top of the stream; smem bit position x = XTOP - q.  (k_huf_scout refused a zero last byte.)
     const uint8_t last = ((const uint8_t*)scomp)[16 + a + it.src_size - 1];
-    if (last == 0) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); break; }
     const int P0 = 8 * (int)(it.src_size - 1) + zc::highbit32(last);
-    const int XTOP = Z + P0;
+    const int XTOP = (int)(16 + a) * 8 + P0;
     int S = (P0 + HB_T - 1) / HB_T;
     if (S < 2 * MAXC) S = 2 * MAXC;
-    const int ck[HB_NLEG + 1] = {S < HB_CK0 ? S : HB_CK0, S < HB_CK1 ? S : HB_CK1, S < HB_CK2 ? S : HB_CK2, S};
     const int q0 = tid * S;
     const int qe = (q0 + S < P0) ? q0 + S : P0;
-    const bool active = q0 < P0;
-    const saddr_t s_comp = to_saddr(scomp), s_t3 = to_saddr(t3), s_t1 = to_saddr(t1);
-    auto cp_at = [&](int rq0, int rqe, int j) { const int x = rq0 + ck[j]; return x < rqe ? x : rqe; };      // checkpoint j of a range
-
-    // (1) first stop: every candidate lands on its first codeword boundary at or past checkpoint 0 (one lookup each, out of one
-    //     64-bit window); candidates of the same codeword chain land together.
-    uint64_t first = ~0ull, fcnt = 0;                                   // candidate -> landing offset / symbols so far (4 bits each)
-    uint32_t live = 0;                                                  // landing offsets in use at the current checkpoint
-    if (active) {
-        const int l0 = cp_at(q0, qe, 0);
-        first = 0;
-        if (fixed_len) {
-            int q = q0 + (maxbits - q0 % maxbits) % maxbits, c = 0;     // the one candidate that is a boundary; the others follow it
-            track_advance3(s_comp, s_t3, s_t1, maxbits, XTOP, q, c, l0);
-            first = (uint64_t)(uint32_t)(q - l0) * 0x1111111111111111ull;
-            fcnt = (uint64_t)(uint32_t)c * 0x1111111111111111ull;
-            live = 1u << (q - l0);
-        } else {
-            for (int k = 0; k < maxbits; k++) {
-                int q = q0 + k, c = 0;
-                track_advance3(s_comp, s_t3, s_t1, maxbits, XTOP, q, c, l0);
-                const uint32_t o = (uint32_t)(q - l0);
-                first |= (uint64_t)o << (4 * k);
-                fcnt |= (uint64_t)c << (4 * k);
-                live |= 1u << o;
-            }
-        }
-        if (maxbits < 16) first |= ~0ull << (4 * maxbits);              // candidates that cannot occur: dead (15)
-    }
-    // (2) legs between checkpoints: the live tracks of ALL ranges are work items dealt out evenly over the CTA
-    uint32_t leg_done = 0;
-    for (int leg = 0; leg < HB_NLEG; leg++) {
-        if (ck[leg + 1] == ck[leg]) continue;                           // (uniform) short ranges: nothing between these checkpoints
-        leg_done |= 1u << leg;
-        const uint32_t n_mine = (uint32_t)__popc(live);
-        uint32_t qtotal;
-        uint32_t idx = hb_scan(n_mine, misc + 8 * (leg & 1), &qtotal);
-        for (uint32_t m = live; m; m &= m - 1) qitems[idx++] = (uint16_t)((uint32_t)tid | ((uint32_t)(__ffs((int)m) - 1) << 8));
-        __syncthreads();
-        for (uint32_t i = tid; i < qtotal; i += HB_T) {
-            const uint32_t item = qitems[i];
-            const int owner = (int)(item & 0xFFu), o = (int)(item >> 8);
-            const int oq0 = owner * S, oqe = (oq0 + S < P0) ? oq0 + S : P0;
-            const int lim = cp_at(oq0, oqe, leg + 1);
-            int q = cp_at(oq0, oqe, leg) + o, c = 0;
-            track_advance3(s_comp, s_t3, s_t1, maxbits, XTOP, q, c, lim);
-            legtab[(leg * HB_T + owner) * MAXC + o] = (uint16_t)((uint32_t)(q - lim) | ((uint32_t)c << 4));
-        }
-        __syncthreads();
-        uint32_t nl = 0;
-        for (uint32_t m = live; m; m &= m - 1) nl |= 1u << (legtab[(leg * HB_T + tid) * MAXC + (__ffs((int)m) - 1)] & 15u);
-        live = nl;
-    }
-    // (3) the map candidate -> candidate of the next range: exit offset of every landing offset in use after the first stop
-    uint64_t fmap = MAP_IDENTITY;
-    if (active) {
-        uint64_t exit_of = 0;
-        uint32_t starts = 0;
-        for (int k = 0; k < maxbits; k++) starts |= 1u << ((uint32_t)(first >> (4 * k)) & 15u);
-        for (uint32_t m = starts; m; m &= m - 1) {
-            const int o0 = __ffs((int)m) - 1;
-            uint32_t o = (uint32_t)o0;
-#pragma unroll
-            for (int leg = 0; leg < HB_NLEG; leg++) if (leg_done & (1u << leg)) o = legtab[(leg * HB_T + tid) * MAXC + o] & 15u;
-            exit_of |= (uint64_t)o << (4 * o0);
-        }
-        fmap = 0;
-        for (int k = 0; k < maxbits; k++) fmap |= ((exit_of >> (4 * ((uint32_t)(first >> (4 * k)) & 15u))) & 15ull) << (4 * k);
-        if (maxbits < 16) fmap |= ~0ull << (4 * maxbits);
-    }
-    // ---- compose the maps along the stream: inclusive scan in the warp, then warp totals serially ------------------------------
-    // inc_map(lane) = f_lane o ... o f_(lane - 2^d + 1); a constant map absorbs everything before it, and after the first
-    // step nearly every lane holds one: the gather runs only when some lane of the warp still needs it.
-    uint64_t inc_map = fmap;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        const uint64_t o = __shfl_up_sync(0xFFFFFFFFu, inc_map, d);
-        const bool need = lane >= d && !map_is_const(inc_map, maxbits);
-        if (__any_sync(0xFFFFFFFFu, need)) { if (need) inc_map = map_compose(inc_map, o); }
-    }
-    uint64_t exc_map = __shfl_up_sync(0xFFFFFFFFu, inc_map, 1);
-    if (lane == 0) exc_map = MAP_IDENTITY;
-    if (lane == 31) wmap[warp] = inc_map;
-    __syncthreads();
-    if (tid == 0) {
-        uint32_t k = 0;
-        for (int w = 0; w < HB_NW; w++) { misc[16 + w] = k; k = (uint32_t)(wmap[w] >> (4 * k)) & 15u; }
-    }
-    __syncthreads();
-    const uint32_t kw = misc[16 + warp];
-    const uint32_t ktrue = (uint32_t)(exc_map >> (4 * kw)) & 15u;      // this thread's true candidate
-    // symbols of the true track, and where it lands
-    uint32_t mycnt = 0;
-    int myland = -1;
-    if (active && ktrue < (uint32_t)maxbits) {
-        uint32_t o = (uint32_t)(first >> (4 * ktrue)) & 15u;
-        mycnt = (uint32_t)(fcnt >> (4 * ktrue)) & 15u;
-#pragma unroll
-        for (int leg = 0; leg < HB_NLEG; leg++) {
-            if (leg_done & (1u << leg)) { const uint32_t e = legtab[(leg * HB_T + tid) * MAXC + o]; o = e & 15u; mycnt += e >> 4; }
-        }
-        myland = qe + (int)o;
-    }
-    // the stream must end exactly on its first bit: the last active range's true track lands on P0
-    const bool bad_end = active && qe == P0 && myland != P0;
-    // ---- count, scan, write ------------------------------------------------------------------------------------------
-    const int any_bad = __syncthreads_or(bad_end);                      // (also: every read of the leg tables is done before phase 2 overwrites them)
-    uint32_t total;
-    const uint32_t off = hb_scan(mycnt, misc, &total);
-    if (any_bad || total != it.n_sym) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); break; }
     uint8_t* dst = J.lit + B.lit_base + it.dst_off;
     const uint32_t a2 = (uint32_t)((uintptr_t)dst & 15);
-    if (mycnt) {
+    if (q0 < P0) {
         // write pass: from the true start to the first boundary at or past the end of the range.  Bytes go out as aligned 4-byte
         // words assembled in a register pair; the ragged head and tail (words shared with the neighbouring ranges) as bytes.
-        saddr_t out = to_saddr(sout) + a2 + off;
-        int q = q0 + (int)ktrue;
+        const saddr_t s_comp = to_saddr(scomp), s_t3 = to_saddr(t3), s_t1 = to_saddr(t1);
+        saddr_t out = to_saddr(sout) + a2 + (bound >> 4);
+        int q = q0 + (int)(bound & 15u);
         int rem = qe - q;
         Win w;
         win_init(w, s_comp, XTOP - q);
@@ -2055,7 +2205,7 @@ __global__ void __launch_bounds__(HB_T, 3) k_huf_decode_block(JobDev J) {
         if (last_full >= first_full && (last_full << 4) < endb && !(a2 && last_full == 0))
             for (uint32_t k = (last_full << 4) + tid; k < endb; k += HB_T) dal[k] = sout[k];
     }
-    __syncthreads();                                                    // the output image becomes the next stream's scratch
+    __syncthreads();                                                    // the output image is overwritten by the next stream
     }
 }
 
@@ -3181,13 +3331,14 @@ Launch choose_paths(JobDev& J, const fw::JobPlan& pl, const Overrides& ov, uint3
     // block): the two decodes side by side -- for a single small archive this branch is the critical path (25 us each)
     L.huf_side = J.n_huf_big && J.n_huf_items > J.n_huf_big;
     // Two shapes of the same decode of the big streams.  Enough blocks to fill the device several times over (a batch, a
-    // chromosome): one CTA per BLOCK, its four streams in turn, tables built once (k_huf_decode_block: 1.31 ms against 1.63 ms
-    // on the 256-archive job).  A handful of blocks (one small archive): one CTA per STREAM, the four of a block as a
-    // thread-block cluster that shares the table construction through DSMEM -- four times the CTAs in flight, which is what
-    // latency wants (k_huf_decode_big).
+    // chromosome): one CTA per BLOCK, its four streams in turn, tables built once, the range starts found beforehand by
+    // k_huf_scout (the pair: 1.17 ms on the 256-archive job; 1.63 ms for the cluster kernel).  A handful of blocks (one small
+    // archive): one CTA per STREAM, the four of a block as a thread-block cluster that shares the table construction through
+    // DSMEM -- four times the CTAs in flight and no second launch, which is what latency wants (k_huf_decode_big).
     L.huf_per_block = J.n_huf_big / 4 >= (J.huf_block_min ? J.huf_block_min : 296u);
     L.huf_small_smem = huf_fixed_smem(HUF_T_SMALL) + ((J.max_huf_small + 15 + 16 + 16 + 15) & ~15u);
     L.huf_big_smem = hb_smem_bytes(J.max_huf_stream);
+    L.huf_scout_smem = hs_smem_bytes(J.max_huf_stream);
     // a job with both kinds of blocks (a FASTQ archive: 2 x 10^6 tiny blocks and the ~130 big blocks of the ids, each one chain of
     // ~10^4 sequences, 2.9 ms): the general kernel beside the tiny blocks' (2.0 ms)
     L.seq_side = J.tiny_blocks && J.n_seq_big;
@@ -3232,6 +3383,9 @@ int launch_zstd_stage(const JobDev& J, const Launch& L, const Streams& S, StageE
         if (J.n_huf_big) {   // items [0, n_huf_big): the streams of 4-stream blocks, four consecutive items (= one cluster) per block
             if (!st2) ev->kernel_begin();
             if (L.huf_per_block) {
+                // (the scout and its write pass are one decode of the big streams: counted as one launch, like the cluster kernel)
+                NAF_SET_MAX_SMEM(k_huf_scout, L.huf_scout_smem);
+                NAF_LAUNCH(k_huf_scout, J.n_huf_big / 4, HS_T, L.huf_scout_smem, sb, J);
                 NAF_SET_MAX_SMEM(k_huf_decode_block, L.huf_big_smem);
                 NAF_LAUNCH(k_huf_decode_block, J.n_huf_big / 4, HB_T, L.huf_big_smem, sb, J); launches++;
             } else {

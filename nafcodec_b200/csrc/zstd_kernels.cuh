@@ -62,6 +62,7 @@ struct JobDev {
     uint32_t* fin_unresolved;         // unresolved bytes after level 1
     uint32_t* fin_count;              // [3] rotating per-round counters of level 2
     const zf::HufItem* huf_items;     // one per Huffman bitstream
+    uint32_t* huf_bounds;             // [n_huf_big x 256] k_huf_scout -> k_huf_decode_block: output offset << 4 | start offset of every range
     uint32_t huf_block_min;           // host: launch configuration: jobs with at least this many big blocks use k_huf_decode_block (0: default)
     uint32_t n_huf_items, n_huf_big;  // items [0, n_huf_big): streams of 4-stream blocks, four per block (k_huf_decode_big, one cluster per block); the rest: k_huf_decode<128>
     uint32_t max_huf_stream, max_huf_small;   // largest stream (bytes) in each class
@@ -122,7 +123,7 @@ struct Overrides {
 struct Launch {
     bool huf_side = false;            // small Huffman streams beside the big ones (given a third stream)
     bool huf_per_block = false;       // big streams: k_huf_decode_block (one CTA per block) rather than k_huf_decode_big
-    uint32_t huf_small_smem = 0, huf_big_smem = 0;
+    uint32_t huf_small_smem = 0, huf_big_smem = 0, huf_scout_smem = 0;
     bool seq_side = false;            // k_decode_sequences beside the tiny blocks' kernel (given a third stream)
     uint32_t lit_blocks = 0, lit_split = 0;   // k_lz_literals grid (blocks x split); lit_few: the <4> shape
     bool lit_few = false;
