@@ -39,7 +39,7 @@ struct StageEvents {
     int n = 0, cap = 0;
     cudaStream_t st = 0;
     void mark() { if (ev && n < cap) cudaEventRecord(ev[n++], st); }
-    // one extra interval around the dominant kernel alone (k_huf_decode<512>), for the roofline figure
+    // one extra interval around the dominant kernel alone (k_huf_decode_block, with its scout k_huf_scout), for the roofline figure
     cudaEvent_t kb = nullptr, ke = nullptr;
     bool k_used = false;
     void kernel_begin() { if (ev && kb) cudaEventRecord(kb, st); }

@@ -823,12 +823,11 @@ int bind_job(nafgpu_ctx* c, size_t nb, const Staged& S, const zk::Overrides& ov)
     J.fin_g_base = (const uint64_t*)(desc + c->o_gbase);
     J.huf_weights = (uint8_t*)c->hufw.p; J.huf_meta = (uint8_t*)c->hufw.p + (size_t)pl.n_huf_slots * 256;
     J.huf_items = (const zf::HufItem*)(desc + c->o_huf); J.huf_bounds = (uint32_t*)c->hufb.p; J.n_huf_items = (uint32_t)nh; J.n_huf_big = pl.n_huf_big; J.max_huf_stream = pl.max_huf_stream; J.max_huf_small = pl.max_huf_small;
-    J.debug = nullptr; J.debug_seq = nullptr;
-    if (ov.debug_huf && nh) {
-        if (!c->debug.ensure(nh * 64 + 64)) return fail(c, NAFGPU_ERR_NOMEM, "debug buffer");
-        cudaMemsetAsync(c->debug.p, 0, nh * 64 + 64, c->streams.st);
-        J.debug = (unsigned long long*)c->debug.p;
-        J.debug_seq = J.debug + nh * 8;
+    J.debug_seq = nullptr;
+    if (ov.debug_huf) {
+        if (!c->debug.ensure(64)) return fail(c, NAFGPU_ERR_NOMEM, "debug buffer");
+        cudaMemsetAsync(c->debug.p, 0, 64, c->streams.st);
+        J.debug_seq = (unsigned long long*)c->debug.p;
     }
     J.fs_tiles = (const zf::FsTile*)(desc + c->o_tiles); J.fs_big = (const zf::FsBigFrame*)(desc + c->o_big);
     J.fs_state = (zf::FsTileState*)c->fsstate.p; J.n_fs_tiles = S.n_tiles; J.n_fs_big = S.n_bigs; J.fs_big_frame = S.fs_big;
@@ -1103,24 +1102,12 @@ int nafgpu_job_fetch(nafgpu_ctx* c, nafgpu_result* out, uint32_t n) {
     CUDA_TRY(c, cudaSetDevice(c->device));
     { int rc_d2h = d2h_results(c); if (rc_d2h) return rc_d2h; }
     CUDA_TRY(c, cudaGetLastError());
-    if (c->J.debug) {
-        size_t nh = c->J.n_huf_items;
-        std::vector<unsigned long long> d(nh * 8 + 8);
-        cudaMemcpy(d.data(), c->J.debug, nh * 64 + 64, cudaMemcpyDeviceToHost);
-        const unsigned long long* q = d.data() + nh * 8;
-        double ph[6] = {0, 0, 0, 0, 0, 0}, iters = 0, maxit = 0;
-        size_t cnt = 0;
-        for (size_t i = 0; i < c->J.n_huf_big; i++) {
-            if (!d[i * 8 + 6]) continue;
-            for (int k = 0; k < 6; k++) ph[k] += (double)(d[i * 8 + k + 1] - d[i * 8 + k]);
-            iters += (double)d[i * 8 + 7]; if ((double)d[i * 8 + 7] > maxit) maxit = (double)d[i * 8 + 7];
-            cnt++;
-        }
+    if (c->J.debug_seq) {
+        unsigned long long q[8];
+        cudaMemcpy(q, c->J.debug_seq, sizeof(q), cudaMemcpyDeviceToHost);
         if (q[4]) fprintf(stderr, "[seq debug] %llu sequences: producer %.0f cycles work + %.0f waiting, consumer %.0f work + %.0f waiting (per sequence)\n", q[4],
                           (double)q[0] / q[4], (double)q[1] / q[4], (double)q[2] / q[4], (double)q[3] / q[4]);
         if (q[7]) fprintf(stderr, "[lz small debug] cycles: probe %llu, copy %llu, all rounds %llu\n", q[5], q[6], q[7]);
-        if (cnt) fprintf(stderr, "[huf debug] big CTAs %zu: cycles stage+weights %.0f, table %.0f, sync %.0f (iters avg %.2f max %.0f), scan %.0f, write %.0f, flush %.0f\n",
-                         cnt, ph[0] / cnt, ph[1] / cnt, ph[2] / cnt, iters / cnt, maxit, ph[3] / cnt, ph[4] / cnt, ph[5] / cnt);
     }
     read_lz_stats(c);
     const uint8_t* R = (const uint8_t*)c->result.p;

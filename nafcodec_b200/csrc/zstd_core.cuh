@@ -39,7 +39,7 @@ ZHD int highbit32(uint32_t v) {
 #if defined(__CUDA_ARCH__)
     return 31 - __clz((int)v);
 #else
-    return 31 - __builtin_clz(v);
+    return v ? 31 - __builtin_clz(v) : -1;          // (the device's value for 0; __builtin_clz(0) is undefined)
 #endif
 }
 

@@ -13,7 +13,7 @@
 //                   k_huf_scout              per big block: the exact start and output offset of every range of its four streams
 //                   k_huf_decode_block       per big block: intra-stream parallel decode of its four streams into the literal staging buffer
 //                   k_huf_decode_big         the same per stream, four CTAs of a block as a cluster (DSMEM): a job of a few blocks
-//                   k_huf_decode<128>        short streams
+//                   k_huf_decode_small       short streams
 //   LZ stage        k_lz_literals (+ _tiny)  per block: raw / RLE blocks, literal runs -> their output positions
 //                   k_lz_small               a job of at most 2048 matches: the whole match stage in one CTA
 //                   k_lz_index, k_lz_first   per match: position index; round 1 of the dependency-resolving match execution (+ redirect through copies)
@@ -986,10 +986,10 @@ __global__ void __launch_bounds__(FSCAN_T) k_fs_apply(JobDev J) {
 }
 
 // --------------------------------------------------------------------------------------------------------------
-// k_huf_decode: one CTA per Huffman bitstream, intra-stream parallel.
+// k_huf_decode_small: one CTA per short Huffman bitstream, intra-stream parallel.
 //
 // A zstd Huffman stream is one serial bitstream of up to 32 Ki symbols, read backwards; with one thread per stream a
-// 5 Mbp genome keeps ~80 lanes busy.  Here the stream is cut into HUF_T equal bit ranges, one per thread.  A thread
+// 5 Mbp genome keeps ~80 lanes busy.  Here the stream is cut into HUF_T_SMALL equal bit ranges, one per thread.  A thread
 // does not know where the first codeword of its range starts, but it must be one of the `max_bits` positions at the
 // top of the range.  So it follows ALL candidates ("tracks") through its range: tracks that reach the same bit
 // position merge (prefix codes usually resynchronise within a few symbols, so one track survives; near-fixed-length
@@ -999,18 +999,23 @@ __global__ void __launch_bounds__(FSCAN_T) k_fs_apply(JobDev J) {
 // thread 0 starts on the stream's first codeword.  Then: block-scan the symbol counts, decode once more from the true
 // start into a shared-memory image of the output, flush with 16-byte stores.
 //
-// Shared memory: decode table 4 KB | weights | scratch | compressed stream (16 B-aligned image of global memory,
-// preceded by >= 16 zero bytes so reads below bit 0 see zeros) | output image (same 16 B phase as the destination).
-constexpr int HUF_T_BIG = 512;                    // threads per stream for 4-stream blocks (up to 32 Ki symbols)
+// Shared memory: the common prefix (HufSmem) | output image (same 16 B phase as the destination) | compressed stream
+// (16 B-aligned image of global memory, preceded by >= 16 zero bytes so reads below bit 0 see zeros).
 constexpr int HUF_T_SMALL = 128;                  // four warps for short streams (1-stream blocks, tiny flushed blocks)
 constexpr int HUF_SEG = 96;                       // tracks are compared for merging every HUF_SEG bits
 constexpr int MAXC = zc::HUF_MAX_BITS;            // candidates per range
-// output image (phase 2) / boundary masks 8 KB + track queue 32 B per thread (phase 1)
-__host__ __device__ constexpr uint32_t huf_sout_bytes(int T) { return (T == HUF_T_BIG ? 32768u : 8192u + 32u * (uint32_t)T) + 64u; }
-// t1 4096 | weights 256 | wcnt 256 | misc 256 | [big only: t3 16384] | output image / boundary masks | (dynamic) compressed stream image
-// the boundary-mask table (8 KB, phase 1 only) shares its space with the output image (phase 2 and flush only)
-__host__ __device__ constexpr uint32_t huf_multi_bytes(int T) { return T == HUF_T_BIG ? 16384u : 0u; }
-__host__ __device__ constexpr uint32_t huf_fixed_smem(int T) { return 4096u + 768u + huf_multi_bytes(T) + huf_sout_bytes(T); }
+
+// The common prefix of the shared memory of every Huffman kernel; each kernel's own space follows it.
+struct HufSmem {
+    uint16_t t1[2048];                            // base table: index = next max_bits bits -> symbol << 8 | length
+    uint8_t weights[256];
+    uint16_t wcnt[128];                           // [8 symbol groups][16 weights]; after the table build: composed map of each warp
+    uint32_t misc[64];                            // scan buffers, warp start candidates; [56..57] the mbarrier of the bulk copies
+};
+static_assert(sizeof(HufSmem) == 4864, "HufSmem: t1 4096 | weights 256 | wcnt 256 | misc 256");
+// k_huf_decode_small: output image (phase 2) / boundary masks 8 KB + track queue 32 B per thread (phase 1)
+constexpr uint32_t HUF_SMALL_SOUT = 8192u + 32u * HUF_T_SMALL + 64u;
+constexpr uint32_t HUF_SMALL_FIXED = sizeof(HufSmem) + HUF_SMALL_SOUT;
 
 constexpr int HUF_W = 12;                          // index width of the multi-symbol tables
 
@@ -1087,28 +1092,14 @@ __device__ __forceinline__ void track_advance(saddr_t comp, saddr_t bm, int xtop
     q = lim - rem;
 }
 
-// Write pass: decodes from q to the first boundary >= lim, storing symbols at out.. (shared address). Returns the count.
-//   t3: index = next 12 bits, entry = sym1 | sym2 << 8 | sym3 << 16 | total length << 24 | n << 28
-//   t1: index = next max_bits bits, entry = symbol << 8 | length
-template <bool MULTI>
-__device__ __forceinline__ int track_write(saddr_t comp, saddr_t t3, saddr_t t1, int maxbits, int xtop, int q, int lim, saddr_t out) {
+// Write pass of k_huf_decode_small: decodes from q to the first boundary >= lim, storing symbols at out.. (shared address).
+// Returns the count.  t1: index = next max_bits bits, entry = symbol << 8 | length
+__device__ __forceinline__ int track_write(saddr_t comp, saddr_t t1, int maxbits, int xtop, int q, int lim, saddr_t out) {
     int rem = lim - q;
     if (rem <= 0) return 0;
     Win w;
     win_init(w, comp, xtop - q);
     int cnt = 0;
-    if (MULTI) {
-        while (rem > HUF_W) {
-            const uint32_t e = lds32(t3 + win_peek_x4(w));
-            const int n = (int)(e >> 28), len = (int)(e >> 24) & 15;
-            sts8(out + cnt, e);
-            if (n > 1) sts8(out + cnt + 1, e >> 8);
-            if (n > 2) sts8(out + cnt + 2, e >> 16);
-            cnt += n;
-            rem -= len;
-            win_consume(w, len);
-        }
-    }
     const int sh1 = HUF_W - maxbits;
     while (rem > 0) {
         const uint32_t e = lds16(t1 + 2 * (win_peek(w) >> sh1));
@@ -1156,6 +1147,8 @@ constexpr uint64_t MAP_IDENTITY = 0xFEDCBA9876543210ull;
 
 // Entries [lo, hi) of the tables over 12-bit windows, from the finished base table: decode the window while whole
 // codewords fit (no barrier inside; the caller separates it from the base-table build and from the first use).
+//   bm (optional): boundary masks, bit j set <=> j+1 bits is a cumulative length of whole codewords
+//   t3 (MULTI): 3-symbol write table, entry = sym1 | sym2 << 8 | sym3 << 16 | total length << 24 | n << 28
 //   tc (optional): count table, entry = bits of all whole codewords | their number << 4 (both <= 12)
 template <int HUF_T, bool MULTI>
 __device__ __forceinline__ void huf_build_wide(const uint16_t* table, int maxbits, uint16_t* bm, uint32_t* t3, uint32_t lo, uint32_t hi,
@@ -1178,9 +1171,8 @@ __device__ __forceinline__ void huf_build_wide(const uint16_t* table, int maxbit
     }
 }
 
-// Builds the three decode tables of one Huffman tree in shared memory (all HUF_T threads of the CTA must call):
-//   table: base table, index = next max_bits bits -> symbol << 8 | length (RFC 8878 4.2.1: ascending weight, then symbol)
-//   bm   : boundary masks of 12-bit windows;  t3 (WITH_T3): 3-symbol write table of 12-bit windows
+// Builds the base table of one Huffman tree in shared memory (all HUF_T threads of the CTA must call):
+//   table: index = next max_bits bits -> symbol << 8 | length (RFC 8878 4.2.1: ascending weight, then symbol)
 template <int HUF_T>
 __device__ __forceinline__ void huf_build_t1(const uint8_t* weights, int nsym, int maxbits, uint16_t* table, uint16_t* wcnt) {
     const int tid = threadIdx.x, lane = tid & 31;
@@ -1229,64 +1221,76 @@ __device__ __forceinline__ void huf_build_t1(const uint8_t* weights, int nsym, i
     __syncthreads();
 }
 
-template <int HUF_T, bool WITH_T3>
-__device__ __forceinline__ void huf_build_tables(const uint8_t* weights, int nsym, int maxbits, uint16_t* table, uint16_t* bm, uint32_t* t3,
-                                                 uint16_t* wcnt) {
-    huf_build_t1<HUF_T>(weights, nsym, maxbits, table, wcnt);
-    huf_build_wide<HUF_T, WITH_T3>(table, maxbits, bm, t3, 0u, 1u << HUF_W);
-    __syncthreads();
+// The tree of a block: its 256 weights to shared memory (NT threads), and its symbol count and max_bits (0: a bad tree, already
+// flagged by k_build_tables)
+struct HufTree { int nsym, maxbits; };
+template <int NT>
+__device__ __forceinline__ HufTree huf_tree(const JobDev& J, const BlockDesc& B, uint8_t* weights) {
+    for (int i = threadIdx.x; i < 64; i += NT) ((uint32_t*)weights)[i] = ((const uint32_t*)(J.huf_weights + (size_t)B.huf_slot * 256))[i];
+    return {(int)J.huf_meta[(size_t)B.huf_slot * 2] + 1, (int)J.huf_meta[(size_t)B.huf_slot * 2 + 1]};
 }
 
-template <int HUF_T>
-__global__ void __launch_bounds__(HUF_T, HUF_T == 512 ? 3 : 4) k_huf_decode(JobDev J, const HufItem* items) {
+// Geometry of a staged stream.  `img`: 16 zero bytes, then the 16 B-aligned image of global memory (the stream at 16 + a).
+// q = distance (in bits) from the top of the stream; smem bit position x = XTOP - q.  The stream is cut into `nranges` ranges
+// of S bits; k_huf_scout finds the starts of k_huf_decode_block's ranges, so the two must take S from here.
+struct HufShape { uint32_t last; int P0, XTOP, S; };
+__device__ __forceinline__ HufShape huf_stream_shape(const uint8_t* img, uint32_t a, uint32_t src_size, int nranges) {
+    const uint32_t last = img[16 + a + src_size - 1];                   // (0: the caller refuses the stream before using the rest)
+    const int P0 = 8 * (int)(src_size - 1) + zc::highbit32(last);
+    int S = (P0 + nranges - 1) / nranges;
+    if (S < 2 * MAXC) S = 2 * MAXC;
+    return {last, P0, (int)(16 + a) * 8 + P0, S};
+}
+
+// Flush of the output image by NT threads: sout[a2 + k] -> dst[k] for k < n, where a2 = dst & 15; aligned 16 B chunks in the
+// middle, bytes at the ragged ends
+template <int NT>
+__device__ __forceinline__ void flush_image(uint8_t* dst, const uint8_t* sout, uint32_t a2, uint32_t n) {
+    const int tid = threadIdx.x;
+    const uint32_t endb = a2 + n;
+    uint8_t* dal = dst - a2;
+    const uint32_t first_full = a2 ? 1u : 0u, last_full = endb >> 4;     // chunks [first_full, last_full) are complete
+    for (uint32_t c = first_full + tid; c < last_full; c += NT) ((uint4*)dal)[c] = ((const uint4*)sout)[c];
+    if (a2) { uint32_t hend = endb < 16 ? endb : 16; for (uint32_t k = a2 + tid; k < hend; k += NT) dal[k] = sout[k]; }
+    if (last_full >= first_full && (last_full << 4) < endb && !(a2 && last_full == 0))
+        for (uint32_t k = (last_full << 4) + tid; k < endb; k += NT) dal[k] = sout[k];
+}
+
+__global__ void __launch_bounds__(HUF_T_SMALL, 4) k_huf_decode_small(JobDev J, const HufItem* items) {
     NAF_DYN_SMEM(unsigned char, smem);
-    constexpr uint32_t HUF_FIXED_SMEM = huf_fixed_smem(HUF_T);
-    constexpr int NWARPS = HUF_T / 32;
-    uint16_t* table = (uint16_t*)smem;
-    uint8_t* weights = smem + 4096;
-    uint16_t* wcnt = (uint16_t*)(smem + 4096 + 256);                    // [8 symbol groups][16 weights]
-    uint32_t* misc = (uint32_t*)(smem + 4096 + 512);                    // [0..32] count scan, [34..49] warp start candidates
-    uint64_t* wmap = (uint64_t*)(smem + 4096 + 256);                    // [NWARPS] composed map of each warp; reuses wcnt after the table build
-    constexpr bool MULTI = HUF_T == HUF_T_BIG;
-    uint32_t* t3 = (uint32_t*)(smem + 4096 + 768);                      // MULTI only: 3-symbol write table
-    uint8_t* sout = smem + 4096 + 768 + huf_multi_bytes(HUF_T);         // output image (phase 2, flush)
+    constexpr int NWARPS = HUF_T_SMALL / 32;
+    HufSmem& sm = *(HufSmem*)smem;
+    uint16_t* table = sm.t1;
+    uint16_t* wcnt = sm.wcnt;
+    uint32_t* misc = sm.misc;                                           // [0..32] count scan, [34..49] warp start candidates
+    uint64_t* wmap = (uint64_t*)sm.wcnt;                                // [NWARPS] composed map of each warp
+    uint8_t* sout = smem + sizeof(HufSmem);                             // output image (phase 2, flush)
     uint16_t* bm = (uint16_t*)sout;                                     // boundary masks of 12-bit windows (phase 1): same space
-    uint32_t* scomp = (uint32_t*)(smem + HUF_FIXED_SMEM);
+    uint32_t* scomp = (uint32_t*)(smem + HUF_SMALL_FIXED);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
 
     const HufItem it = items[blockIdx.x];
     const BlockDesc& B = J.blocks[it.block];
     if (J.frame_bad[B.frame]) return;
-#if defined(__CUDA_ARCH__)
-#define HUF_TICK(k) do { if (J.debug && tid == 0) J.debug[(size_t)blockIdx.x * 8 + (k)] = clock64(); } while (0)
-#else
-#define HUF_TICK(k) ((void)0)
-#endif
-    HUF_TICK(0);
     // ---- stage the compressed stream (coalesced 16 B loads of the aligned image) and the weights -------------------
     const uint8_t* g = J.comp + B.src_off + it.src_off;
     const uint32_t a = (uint32_t)((uintptr_t)g & 15);
     const uint4* gbase = (const uint4*)(g - a);
     const uint32_t nchunks = (a + it.src_size + 15) >> 4;
-    for (uint32_t c = tid; c < nchunks; c += HUF_T) ((uint4*)scomp)[1 + c] = gbase[c];
-    for (int i = tid; i < 64; i += HUF_T) ((uint32_t*)weights)[i] = ((const uint32_t*)(J.huf_weights + (size_t)B.huf_slot * 256))[i];
-    const int nsym = (int)J.huf_meta[(size_t)B.huf_slot * 2] + 1, maxbits = (int)J.huf_meta[(size_t)B.huf_slot * 2 + 1];
+    for (uint32_t c = tid; c < nchunks; c += HUF_T_SMALL) ((uint4*)scomp)[1 + c] = gbase[c];
+    const HufTree tree = huf_tree<HUF_T_SMALL>(J, B, sm.weights);
+    const int maxbits = tree.maxbits;
     if (maxbits == 0) return;                                           // bad tree: already flagged by k_build_tables
     __syncthreads();
-    HUF_TICK(1);
     if ((uint32_t)tid < 16 + a) ((uint8_t*)scomp)[tid] = 0;              // bits below the stream start read as zero
-    huf_build_tables<HUF_T, MULTI>(weights, nsym, maxbits, table, bm, t3, wcnt);
-    HUF_TICK(2);
+    huf_build_t1<HUF_T_SMALL>(sm.weights, tree.nsym, maxbits, table, wcnt);
+    huf_build_wide<HUF_T_SMALL, false>(table, maxbits, bm, nullptr, 0u, 1u << HUF_W);
+    __syncthreads();
 
     // ---- phase 1: transition map of every range -------------------------------------------------------------------------
-    // q = distance (in bits) from the top of the stream; smem bit position x = XTOP - q.
-    const int Z = (int)(16 + a) * 8;                                    // smem bit position of stream bit 0
-    const uint8_t last = ((const uint8_t*)scomp)[16 + a + it.src_size - 1];
-    if (last == 0) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); return; }
-    const int P0 = 8 * (int)(it.src_size - 1) + zc::highbit32(last);
-    const int XTOP = Z + P0;
-    int S = (P0 + HUF_T - 1) / HUF_T;
-    if (S < 2 * MAXC) S = 2 * MAXC;
+    const HufShape shape = huf_stream_shape((const uint8_t*)scomp, a, it.src_size, HUF_T_SMALL);
+    if (shape.last == 0) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); return; }
+    const int P0 = shape.P0, XTOP = shape.XTOP, S = shape.S;
     const int q0 = tid * S;                                             // top of this thread's range
     const int qe = (q0 + S < P0) ? q0 + S : P0;                         // end of the range (exclusive)
     const bool active = q0 < P0;
@@ -1330,7 +1334,7 @@ __global__ void __launch_bounds__(HUF_T, HUF_T == 512 ? 3 : 4) k_huf_decode(JobD
     //     become work items in a shared-memory queue and are spread evenly over the CTA: following tracks thread-by-
     //     thread leaves lanes with fewer survivors idle (45 % thread efficiency measured); the queue keeps every lane on
     //     one track of equal length.  Two legs: to 96 bits past the first stop (twins merge), then to the range end.
-    constexpr int HUF_QCAP = 4 * HUF_T;
+    constexpr int HUF_QCAP = 4 * HUF_T_SMALL;
     uint32_t* q_owner = (uint32_t*)(sout + 8192);                        // [HUF_QCAP] owner thread | track << 16 (after the boundary masks)
     uint32_t* q_pc = q_owner + HUF_QCAP;                                 // [HUF_QCAP] position | symbols << 16
     for (int leg = 0; leg < 2; leg++) {
@@ -1357,7 +1361,7 @@ __global__ void __launch_bounds__(HUF_T, HUF_T == 512 ? 3 : 4) k_huf_decode(JobD
             for (int k = 0; k < MAXC; k++) if (l4 & (1u << k)) { q_owner[idx] = (uint32_t)tid | ((uint32_t)k << 16); q_pc[idx] = pc[k]; idx++; }
         }
         __syncthreads();
-        for (uint32_t i = tid; i < qtotal; i += HUF_T) {
+        for (uint32_t i = tid; i < qtotal; i += HUF_T_SMALL) {
             const int ot = (int)(q_owner[i] & 0xFFFFu);
             const int oq0 = ot * S, oqe = (oq0 + S < P0) ? oq0 + S : P0;
             const int mid = oq0 + HUF_W + HUF_SEG;
@@ -1407,7 +1411,6 @@ __global__ void __launch_bounds__(HUF_T, HUF_T == 512 ? 3 : 4) k_huf_decode(JobD
             fmap |= (uint64_t)land << (4 * k);
         }
     }
-    HUF_TICK(3);
     // ---- compose the maps along the stream: inclusive scan in the warp, then warp totals serially ------------------------
     uint64_t inc_map = fmap;
 #pragma unroll
@@ -1454,21 +1457,9 @@ __global__ void __launch_bounds__(HUF_T, HUF_T == 512 ? 3 : 4) k_huf_decode(JobD
     // the stage does not depend on the FSE branch, so the two run on different streams)
     uint8_t* dst = J.lit + B.lit_base + it.dst_off;
     const uint32_t a2 = (uint32_t)((uintptr_t)dst & 15);
-    HUF_TICK(4);
-    if (mycnt) track_write<MULTI>(s_comp, to_saddr(t3), to_saddr(table), maxbits, XTOP, q0 + (int)ktrue, qe, to_saddr(sout) + a2 + off);
+    if (mycnt) track_write(s_comp, to_saddr(table), maxbits, XTOP, q0 + (int)ktrue, qe, to_saddr(sout) + a2 + off);
     __syncthreads();
-    HUF_TICK(5);
-    {
-        // ---- flush: sout[a2 + k] -> dst[k]; aligned 16 B chunks in the middle, bytes at the ragged ends ----------------
-        const uint32_t n = it.n_sym, endb = a2 + n;
-        uint8_t* dal = dst - a2;
-        const uint32_t first_full = a2 ? 1u : 0u, last_full = endb >> 4;     // chunks [first_full, last_full) are complete
-        for (uint32_t c = first_full + tid; c < last_full; c += HUF_T) ((uint4*)dal)[c] = ((const uint4*)sout)[c];
-        if (a2) { uint32_t hend = endb < 16 ? endb : 16; for (uint32_t k = a2 + tid; k < hend; k += HUF_T) dal[k] = sout[k]; }
-        if (last_full >= first_full && (last_full << 4) < endb && !(a2 && last_full == 0))
-            for (uint32_t k = (last_full << 4) + tid; k < endb; k += HUF_T) dal[k] = sout[k];
-    }
-    HUF_TICK(6);
+    flush_image<HUF_T_SMALL>(dst, sout, a2, it.n_sym);
 }
 
 // --------------------------------------------------------------------------------------------------------------
@@ -1509,7 +1500,8 @@ constexpr int HB_CK0 = 12, HB_CK1 = 108, HB_CK2 = 320;      // checkpoints (bits
 constexpr uint32_t HB_SOUT = 32768u + 64u;                  // output image (phase 2); phase 1: boundary masks | leg tables | work queue
 constexpr uint32_t HB_BM_BYTES = 8192u, HB_LEG_BYTES = HB_NLEG * HB_T * MAXC * 2u, HB_Q_BYTES = HB_T * MAXC * 2u;
 static_assert(HB_BM_BYTES + HB_LEG_BYTES + HB_Q_BYTES <= HB_SOUT, "phase-1 scratch must fit the output image");
-constexpr uint32_t HB_FIXED = 4096u + 768u + 16384u + HB_SOUT;      // t1 | weights, wcnt, misc | t3 | output image
+// shared memory of k_huf_decode_big and k_huf_decode_block: HufSmem | t3 | output image | compressed stream image
+constexpr uint32_t HB_T3_AT = sizeof(HufSmem), HB_SOUT_AT = HB_T3_AT + 4u * (1u << HUF_W), HB_FIXED = HB_SOUT_AT + HB_SOUT;
 __host__ __device__ constexpr uint32_t hb_smem_bytes(uint32_t max_stream) { return HB_FIXED + ((max_stream + 15u + 16u + 16u + 15u) & ~15u); }
 
 // Exclusive prefix sum of one small value per thread over the CTA (HB_T threads); *total gets the sum.  One barrier; `buf`
@@ -1534,45 +1526,160 @@ __device__ __forceinline__ bool map_is_const(uint64_t m, int maxbits) {        /
     return ((m ^ rep) & lowmask) == 0;
 }
 
+// Staging of the compressed streams: bulk asynchronous copies (cp.async.bulk global -> shared) that complete on an mbarrier.
+// The emulator has no asynchronous copy: stage_stream copies synchronously, and the mbarrier calls do nothing.
+__device__ __forceinline__ void mbar_init(saddr_t mbar, uint32_t count) {     // one thread, before anyone arrives
+#if defined(__CUDA_ARCH__)
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(mbar), "r"(count));
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+#endif
+}
+// One thread: `bytes` (a multiple of 16) from src (16 B aligned) to dst, in one copy
+__device__ __forceinline__ void stage_stream(void* dst, const uint8_t* src, uint32_t bytes, saddr_t mbar) {
+#if defined(__CUDA_ARCH__)
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(mbar), "r"(bytes) : "memory");
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 :: "r"(to_saddr(dst)), "l"(src), "r"(bytes), "r"(mbar) : "memory");
+#else
+    for (uint32_t c = 0; c < (bytes >> 4); c++) ((uint4*)dst)[c] = ((const uint4*)src)[c];
+#endif
+}
+// Waits for phase `parity` of the mbarrier.  Every thread waits, also before an early exit: the shared memory must not be handed
+// to another CTA under a copy.
+__device__ __forceinline__ void mbar_wait(saddr_t mbar, uint32_t parity) {
+#if defined(__CUDA_ARCH__)
+    uint32_t done;
+    do {
+        asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
+                     : "=r"(done) : "r"(mbar), "r"(parity) : "memory");
+    } while (!done);
+#endif
+}
+
+// A tree whose codes all have the same length (e.g. 16 equiprobable byte values) never lets tracks merge -- and does not need
+// to: the codeword boundaries are the multiples of that length.  One barrier: the whole CTA calls.
+__device__ __forceinline__ bool huf_fixed_length(const uint16_t* wcnt) {
+    const int tid = threadIdx.x;
+    return !__syncthreads_or(tid < 128 && (tid & 15) >= 2 && (tid & 15) <= zc::HUF_MAX_BITS && wcnt[tid] != 0);
+}
+
+// First stop of phase 1: every candidate start q0 + k (k < max_bits) lands on its first codeword boundary at or past l0, so
+// candidates of the same codeword chain land together.  `count(q, c, lim)` follows one track.  Out: first / fcnt = candidate ->
+// landing offset (q - l0) / symbols so far (4 bits each; candidates that cannot occur: dead, 15); live |= landing offsets.
+template <class Count>
+__device__ __forceinline__ void hb_first_stop(int q0, int l0, int maxbits, bool fixed_len, Count count, uint64_t& first, uint64_t& fcnt,
+                                              uint32_t& live) {
+    first = 0;
+    if (fixed_len) {
+        int q = q0 + (maxbits - q0 % maxbits) % maxbits, c = 0;         // the one candidate that is a boundary; the others follow it
+        count(q, c, l0);
+        first = (uint64_t)(uint32_t)(q - l0) * 0x1111111111111111ull;
+        fcnt = (uint64_t)(uint32_t)c * 0x1111111111111111ull;
+        live = 1u << (q - l0);
+    } else {
+        for (int k = 0; k < maxbits; k++) {
+            int q = q0 + k, c = 0;
+            count(q, c, l0);
+            const uint32_t o = (uint32_t)(q - l0);
+            first |= (uint64_t)o << (4 * k);
+            fcnt |= (uint64_t)c << (4 * k);
+            live |= 1u << o;
+        }
+    }
+    if (maxbits < 16) first |= ~0ull << (4 * maxbits);
+}
+
+// Composes the transition maps along each stream of WPS consecutive warps: inclusive scan in the warp, then the stream's warp
+// totals serially; returns this thread's true candidate.  inc_map(lane) = f_lane o ... o f_(lane - 2^d + 1); a constant map
+// absorbs everything before it, and after the first step nearly every lane holds one: the gather runs only when some lane of
+// the warp still needs it.  wmap, kw: one entry per warp.  Two barriers: all HB_T threads call.
+template <int WPS>
+__device__ __forceinline__ uint32_t hb_compose(uint64_t fmap, int maxbits, uint64_t* wmap, uint32_t* kw) {
+    static_assert(HB_NW % WPS == 0, "hb_compose: whole streams");
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    uint64_t inc_map = fmap;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+        const uint64_t o = __shfl_up_sync(0xFFFFFFFFu, inc_map, d);
+        const bool need = lane >= d && !map_is_const(inc_map, maxbits);
+        if (__any_sync(0xFFFFFFFFu, need)) { if (need) inc_map = map_compose(inc_map, o); }
+    }
+    uint64_t exc_map = __shfl_up_sync(0xFFFFFFFFu, inc_map, 1);
+    if (lane == 0) exc_map = MAP_IDENTITY;
+    if (lane == 31) wmap[warp] = inc_map;
+    __syncthreads();
+    if (tid < HB_NW / WPS) {
+        uint32_t k = 0;
+        for (int w = tid * WPS; w < (tid + 1) * WPS; w++) { kw[w] = k; k = (uint32_t)(wmap[w] >> (4 * k)) & 15u; }
+    }
+    __syncthreads();
+    return (uint32_t)(exc_map >> (4 * kw[warp])) & 15u;
+}
+
+// Write pass of one range: from q (bits below the top of the stream) to the first boundary at or past qe, the symbols to `out`
+// on (shared address).  Bytes go out as aligned 4-byte words assembled in a register pair; the ragged head and tail (words
+// shared with the neighbouring ranges) as bytes.
+__device__ __forceinline__ void hb_write_range(saddr_t comp, saddr_t t3, saddr_t t1, int maxbits, int xtop, int q, int qe, saddr_t out) {
+    int rem = qe - q;
+    Win w;
+    win_init(w, comp, xtop - q);
+    const int sh1 = HUF_W - maxbits;
+    while ((out & 3u) && rem > 0) {                                     // head: single symbols up to a word boundary
+        const uint32_t e = lds16(t1 + 2 * (win_peek(w) >> sh1));
+        sts8(out, e >> 8); out++;
+        rem -= (int)(e & 0xFFu);
+        win_consume(w, (int)(e & 0xFFu));
+    }
+    uint32_t acc_lo = 0, acc_hi = 0;
+    int pc = 0;                                                         // bytes waiting in acc
+    while (rem > HUF_W) {
+        const uint32_t e = lds32(t3 + win_peek_x4(w));
+        const int n = (int)(e >> 28), len = (int)(e >> 24) & 15;
+        const uint32_t sy = e & 0xFFFFFFu;
+        acc_lo |= sy << (8 * pc);
+        acc_hi |= __funnelshift_l(sy, 0u, 8 * pc);                      // the bits that fall off the top of acc_lo
+        pc += n;
+        if (pc >= 4) { sts32(out, acc_lo); out += 4; acc_lo = acc_hi; acc_hi = 0; pc -= 4; }
+        rem -= len;
+        win_consume(w, len);
+    }
+    while (rem > 0) {                                                   // the last symbols, one at a time
+        const uint32_t e = lds16(t1 + 2 * (win_peek(w) >> sh1));
+        acc_lo |= (e >> 8) << (8 * pc);
+        pc++;
+        if (pc == 4) { sts32(out, acc_lo); out += 4; acc_lo = 0; pc = 0; }
+        rem -= (int)(e & 0xFFu);
+        win_consume(w, (int)(e & 0xFFu));
+    }
+    for (int k = 0; k < pc; k++) sts8(out + k, acc_lo >> (8 * k));
+}
+
 __global__ void HB_CLUSTER_ATTR __launch_bounds__(HB_T, 3) k_huf_decode_big(JobDev J) {
     NAF_DYN_SMEM(unsigned char, smem);
-    uint16_t* t1 = (uint16_t*)smem;
-    uint8_t* weights = smem + 4096;
-    uint16_t* wcnt = (uint16_t*)(smem + 4096 + 256);
-    uint32_t* misc = (uint32_t*)(smem + 4096 + 512);                    // [0..15] two scan buffers, [16..23] warp start candidates, [56..57] mbarrier
-    uint64_t* wmap = (uint64_t*)(smem + 4096 + 256);                    // [HB_NW] composed map of each warp (reuses wcnt after the table build)
-    uint32_t* t3 = (uint32_t*)(smem + 4864);
-    uint8_t* sout = smem + 4864 + 16384;
+    HufSmem& sm = *(HufSmem*)smem;
+    uint16_t* t1 = sm.t1;
+    uint32_t* misc = sm.misc;                                           // [0..15] two scan buffers, [16..23] warp start candidates, [56..57] mbarrier
+    uint32_t* t3 = (uint32_t*)(smem + HB_T3_AT);
+    uint8_t* sout = smem + HB_SOUT_AT;
     uint16_t* bm = (uint16_t*)sout;
     uint16_t* legtab = (uint16_t*)(sout + HB_BM_BYTES);                 // [leg][range][offset] = landing offset | symbols << 4
     uint16_t* qitems = (uint16_t*)(sout + HB_BM_BYTES + HB_LEG_BYTES);  // range | offset << 8
     uint32_t* scomp = (uint32_t*)(smem + HB_FIXED);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x;
 
     const HufItem it = J.huf_items[blockIdx.x];
     const BlockDesc& B = J.blocks[it.block];
     // ---- stage the stream: the 16 B-aligned image of global memory, behind 16 bytes that stay zero --------------------------
     const uint8_t* g = J.comp + B.src_off + it.src_off;
     const uint32_t a = (uint32_t)((uintptr_t)g & 15);
-    const uint32_t image_bytes = ((a + it.src_size + 15u) >> 4) << 4;
-#if defined(__CUDA_ARCH__)
-    const uint32_t mbar = (uint32_t)__cvta_generic_to_shared(&misc[56]);
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(mbar), "r"(1));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(mbar), "r"(image_bytes) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     :: "r"((uint32_t)__cvta_generic_to_shared(scomp + 4)), "l"(g - a), "r"(image_bytes), "r"(mbar) : "memory");
-    }
-#else
-    for (uint32_t c = tid; c < (image_bytes >> 4); c += HB_T) ((uint4*)scomp)[1 + c] = ((const uint4*)(g - a))[c];
-#endif
-    for (int i = tid; i < 64; i += HB_T) ((uint32_t*)weights)[i] = ((const uint32_t*)(J.huf_weights + (size_t)B.huf_slot * 256))[i];
-    const int nsym = (int)J.huf_meta[(size_t)B.huf_slot * 2] + 1, maxbits = (int)J.huf_meta[(size_t)B.huf_slot * 2 + 1];
+    const saddr_t mbar = to_saddr(&misc[56]);
+    if (tid == 0) { mbar_init(mbar, 1); stage_stream(scomp + 4, g - a, ((a + it.src_size + 15u) >> 4) << 4, mbar); }
+    const HufTree tree = huf_tree<HB_T>(J, B, sm.weights);
+    const int maxbits = tree.maxbits;
     __syncthreads();
     // a bad tree (flagged by k_build_tables) is the same for the whole cluster: nobody builds, nobody waits for a peer
     if (maxbits != 0) {
-        huf_build_t1<HB_T>(weights, nsym, maxbits, t1, wcnt);
+        huf_build_t1<HB_T>(sm.weights, tree.nsym, maxbits, t1, sm.wcnt);
 #if defined(__CUDA_ARCH__)
         namespace cg = cooperative_groups;
         cg::cluster_group cluster = cg::this_cluster();
@@ -1593,31 +1700,16 @@ __global__ void HB_CLUSTER_ATTR __launch_bounds__(HB_T, 3) k_huf_decode_big(JobD
         __syncthreads();
 #endif
     }
-#if defined(__CUDA_ARCH__)
-    {   // the bulk copy has landed (also before an early exit: the shared memory must not be handed to another CTA under it)
-        uint32_t done;
-        do {
-            asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                         : "=r"(done) : "r"(mbar), "r"(0) : "memory");
-        } while (!done);
-    }
-#endif
+    mbar_wait(mbar, 0);
     // (one thread reads the flag: another stream's kernel may set it at any moment, and the decision must be the CTA's)
     if (__syncthreads_or(maxbits == 0 || (tid == 0 && J.frame_bad[B.frame] != 0))) return;
     if ((uint32_t)tid < 16 + a) ((uint8_t*)scomp)[tid] = 0;              // bits below the stream start read as zero
-    // a tree whose codes all have the same length (e.g. 16 equiprobable byte values) never lets tracks merge -- and does not
-    // need to: the codeword boundaries are the multiples of that length
-    const bool fixed_len = !__syncthreads_or(tid < 128 && (tid & 15) >= 2 && (tid & 15) <= zc::HUF_MAX_BITS && wcnt[tid] != 0);
+    const bool fixed_len = huf_fixed_length(sm.wcnt);
 
     // ---- phase 1: transition map of every range -------------------------------------------------------------------------
-    // q = distance (in bits) from the top of the stream; smem bit position x = XTOP - q.
-    const int Z = (int)(16 + a) * 8;
-    const uint8_t last = ((const uint8_t*)scomp)[16 + a + it.src_size - 1];
-    if (last == 0) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); return; }
-    const int P0 = 8 * (int)(it.src_size - 1) + zc::highbit32(last);
-    const int XTOP = Z + P0;
-    int S = (P0 + HB_T - 1) / HB_T;
-    if (S < 2 * MAXC) S = 2 * MAXC;
+    const HufShape shape = huf_stream_shape((const uint8_t*)scomp, a, it.src_size, HB_T);
+    if (shape.last == 0) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); return; }
+    const int P0 = shape.P0, XTOP = shape.XTOP, S = shape.S;
     const int ck[HB_NLEG + 1] = {S < HB_CK0 ? S : HB_CK0, S < HB_CK1 ? S : HB_CK1, S < HB_CK2 ? S : HB_CK2, S};
     const int q0 = tid * S;
     const int qe = (q0 + S < P0) ? q0 + S : P0;
@@ -1625,30 +1717,12 @@ __global__ void HB_CLUSTER_ATTR __launch_bounds__(HB_T, 3) k_huf_decode_big(JobD
     const saddr_t s_comp = to_saddr(scomp), s_bm = to_saddr(bm);
     auto cp_at = [&](int rq0, int rqe, int j) { const int x = rq0 + ck[j]; return x < rqe ? x : rqe; };      // checkpoint j of a range
 
-    // (1) first stop: every candidate lands on its first codeword boundary at or past checkpoint 0 (one lookup each, out of one
-    //     64-bit window); candidates of the same codeword chain land together.
+    // (1) first stop at checkpoint 0 (one lookup per candidate, out of one 64-bit window)
     uint64_t first = ~0ull, fcnt = 0;                                   // candidate -> landing offset / symbols so far (4 bits each)
     uint32_t live = 0;                                                  // landing offsets in use at the current checkpoint
     if (active) {
-        const int l0 = cp_at(q0, qe, 0);
-        first = 0;
-        if (fixed_len) {
-            int q = q0 + (maxbits - q0 % maxbits) % maxbits, c = 0;     // the one candidate that is a boundary; the others follow it
-            track_advance(s_comp, s_bm, XTOP, q, c, l0);
-            first = (uint64_t)(uint32_t)(q - l0) * 0x1111111111111111ull;
-            fcnt = (uint64_t)(uint32_t)c * 0x1111111111111111ull;
-            live = 1u << (q - l0);
-        } else {
-            for (int k = 0; k < maxbits; k++) {
-                int q = q0 + k, c = 0;
-                track_advance(s_comp, s_bm, XTOP, q, c, l0);
-                const uint32_t o = (uint32_t)(q - l0);
-                first |= (uint64_t)o << (4 * k);
-                fcnt |= (uint64_t)c << (4 * k);
-                live |= 1u << o;
-            }
-        }
-        if (maxbits < 16) first |= ~0ull << (4 * maxbits);              // candidates that cannot occur: dead (15)
+        const auto advance = [&](int& q, int& c, int lim) { track_advance(s_comp, s_bm, XTOP, q, c, lim); };
+        hb_first_stop(q0, cp_at(q0, qe, 0), maxbits, fixed_len, advance, first, fcnt, live);
     }
     // (2) legs between checkpoints: the live tracks of ALL ranges are work items dealt out evenly over the CTA
     uint32_t leg_done = 0;
@@ -1691,27 +1765,8 @@ __global__ void HB_CLUSTER_ATTR __launch_bounds__(HB_T, 3) k_huf_decode_big(JobD
         for (int k = 0; k < maxbits; k++) fmap |= ((exit_of >> (4 * ((uint32_t)(first >> (4 * k)) & 15u))) & 15ull) << (4 * k);
         if (maxbits < 16) fmap |= ~0ull << (4 * maxbits);
     }
-    // ---- compose the maps along the stream: inclusive scan in the warp, then warp totals serially ------------------------------
-    // inc_map(lane) = f_lane o ... o f_(lane - 2^d + 1); a constant map absorbs everything before it, and after the first
-    // step nearly every lane holds one: the gather runs only when some lane of the warp still needs it.
-    uint64_t inc_map = fmap;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        const uint64_t o = __shfl_up_sync(0xFFFFFFFFu, inc_map, d);
-        const bool need = lane >= d && !map_is_const(inc_map, maxbits);
-        if (__any_sync(0xFFFFFFFFu, need)) { if (need) inc_map = map_compose(inc_map, o); }
-    }
-    uint64_t exc_map = __shfl_up_sync(0xFFFFFFFFu, inc_map, 1);
-    if (lane == 0) exc_map = MAP_IDENTITY;
-    if (lane == 31) wmap[warp] = inc_map;
-    __syncthreads();
-    if (tid == 0) {
-        uint32_t k = 0;
-        for (int w = 0; w < HB_NW; w++) { misc[16 + w] = k; k = (uint32_t)(wmap[w] >> (4 * k)) & 15u; }
-    }
-    __syncthreads();
-    const uint32_t kw = misc[16 + warp];
-    const uint32_t ktrue = (uint32_t)(exc_map >> (4 * kw)) & 15u;      // this thread's true candidate
+    // ---- compose the maps along the stream ----------------------------------------------------------------------------------
+    const uint32_t ktrue = hb_compose<HB_NW>(fmap, maxbits, (uint64_t*)sm.wcnt, misc + 16);      // this thread's true candidate
     // symbols of the true track, and where it lands
     uint32_t mycnt = 0;
     int myland = -1;
@@ -1733,56 +1788,10 @@ __global__ void HB_CLUSTER_ATTR __launch_bounds__(HB_T, 3) k_huf_decode_big(JobD
     if (any_bad || total != it.n_sym) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); return; }
     uint8_t* dst = J.lit + B.lit_base + it.dst_off;
     const uint32_t a2 = (uint32_t)((uintptr_t)dst & 15);
-    if (mycnt) {
-        // write pass: from the true start to the first boundary at or past the end of the range.  Bytes go out as aligned 4-byte
-        // words assembled in a register pair; the ragged head and tail (words shared with the neighbouring ranges) as bytes.
-        const saddr_t s_t3 = to_saddr(t3), s_t1 = to_saddr(t1);
-        saddr_t out = to_saddr(sout) + a2 + off;
-        int q = q0 + (int)ktrue;
-        int rem = qe - q;
-        Win w;
-        win_init(w, s_comp, XTOP - q);
-        const int sh1 = HUF_W - maxbits;
-        while ((out & 3u) && rem > 0) {                                 // head: single symbols up to a word boundary
-            const uint32_t e = lds16(s_t1 + 2 * (win_peek(w) >> sh1));
-            sts8(out, e >> 8); out++;
-            rem -= (int)(e & 0xFFu);
-            win_consume(w, (int)(e & 0xFFu));
-        }
-        uint32_t acc_lo = 0, acc_hi = 0;
-        int pc = 0;                                                     // bytes waiting in acc
-        while (rem > HUF_W) {
-            const uint32_t e = lds32(s_t3 + win_peek_x4(w));
-            const int n = (int)(e >> 28), len = (int)(e >> 24) & 15;
-            const uint32_t sy = e & 0xFFFFFFu;
-            acc_lo |= sy << (8 * pc);
-            acc_hi |= __funnelshift_l(sy, 0u, 8 * pc);                  // the bits that fall off the top of acc_lo
-            pc += n;
-            if (pc >= 4) { sts32(out, acc_lo); out += 4; acc_lo = acc_hi; acc_hi = 0; pc -= 4; }
-            rem -= len;
-            win_consume(w, len);
-        }
-        while (rem > 0) {                                               // the last symbols, one at a time
-            const uint32_t e = lds16(s_t1 + 2 * (win_peek(w) >> sh1));
-            acc_lo |= (e >> 8) << (8 * pc);
-            pc++;
-            if (pc == 4) { sts32(out, acc_lo); out += 4; acc_lo = 0; pc = 0; }
-            rem -= (int)(e & 0xFFu);
-            win_consume(w, (int)(e & 0xFFu));
-        }
-        for (int k = 0; k < pc; k++) sts8(out + k, acc_lo >> (8 * k));
-    }
+    // write pass: from the true start to the first boundary at or past the end of the range
+    if (mycnt) hb_write_range(s_comp, to_saddr(t3), to_saddr(t1), maxbits, XTOP, q0 + (int)ktrue, qe, to_saddr(sout) + a2 + off);
     __syncthreads();
-    {
-        // ---- flush: sout[a2 + k] -> dst[k]; aligned 16 B chunks in the middle, bytes at the ragged ends ----------------
-        const uint32_t n = it.n_sym, endb = a2 + n;
-        uint8_t* dal = dst - a2;
-        const uint32_t first_full = a2 ? 1u : 0u, last_full = endb >> 4;     // chunks [first_full, last_full) are complete
-        for (uint32_t c = first_full + tid; c < last_full; c += HB_T) ((uint4*)dal)[c] = ((const uint4*)sout)[c];
-        if (a2) { uint32_t hend = endb < 16 ? endb : 16; for (uint32_t k = a2 + tid; k < hend; k += HB_T) dal[k] = sout[k]; }
-        if (last_full >= first_full && (last_full << 4) < endb && !(a2 && last_full == 0))
-            for (uint32_t k = (last_full << 4) + tid; k < endb; k += HB_T) dal[k] = sout[k];
-    }
+    flush_image<HB_T>(dst, sout, a2, it.n_sym);
 }
 
 // The counting legs of k_huf_scout: like track_advance, but the steady state reads the count table (bits and number of all
@@ -1830,7 +1839,8 @@ constexpr int HS_F = HB_T / HS_C;                           // fine ranges per c
 constexpr int HS_NLEG = HB_NLEG + HS_F - 1;                 // legs after the first stop
 static_assert(HS_T == HB_T && HS_F > HB_NLEG, "k_huf_scout: one scan shape with k_huf_decode_block; slots 1..3 for the first fine range's legs");
 constexpr uint32_t HS_LEG_BYTES = HS_F * HS_T * MAXC * 2u, HS_Q_BYTES = HS_T * MAXC * 2u;
-constexpr uint32_t HS_FIXED = 4096u + 768u + 4096u + HS_LEG_BYTES + HS_Q_BYTES;   // t1 | weights, wcnt, misc | count table | leg tables | queue
+constexpr uint32_t HS_TC_AT = sizeof(HufSmem), HS_LEG_AT = HS_TC_AT + 4096u, HS_Q_AT = HS_LEG_AT + HS_LEG_BYTES;
+constexpr uint32_t HS_FIXED = HS_Q_AT + HS_Q_BYTES;                // HufSmem | count table | leg tables | queue
 __host__ __device__ constexpr uint32_t hs_image_bytes(uint32_t max_stream) { return (max_stream + 15u + 16u + 16u + 15u) & ~15u; }
 __host__ __device__ constexpr uint32_t hs_smem_bytes(uint32_t max_stream) { return HS_FIXED + 4u * hs_image_bytes(max_stream); }
 
@@ -1844,15 +1854,13 @@ __device__ __forceinline__ int hs_checkpoint(int ctop, int S, int P0, int j) {
 
 __global__ void __launch_bounds__(HS_T, 2) k_huf_scout(JobDev J) {
     NAF_DYN_SMEM(unsigned char, smem);
-    uint16_t* t1 = (uint16_t*)smem;
-    uint8_t* weights = smem + 4096;
-    uint16_t* wcnt = (uint16_t*)(smem + 4096 + 256);
-    uint32_t* misc = (uint32_t*)(smem + 4096 + 512);                    // [0..15] scan buffers, [16..23] warp start candidates,
+    HufSmem& sm = *(HufSmem*)smem;
+    uint16_t* t1 = sm.t1;
+    uint32_t* misc = sm.misc;                                           // [0..15] scan buffers, [16..23] warp start candidates,
                                                                         // [24..39] per stream: XTOP, P0, S; [56..57] mbarrier
-    uint64_t* wmap = (uint64_t*)(smem + 4096 + 256);                    // [8] composed map of each warp (reuses wcnt after the table build)
-    uint8_t* tc = smem + 4864;
-    uint16_t* legtab = (uint16_t*)(smem + 4864 + 4096);
-    uint16_t* qitems = (uint16_t*)(smem + 4864 + 4096 + HS_LEG_BYTES);  // range | offset << 8
+    uint8_t* tc = smem + HS_TC_AT;
+    uint16_t* legtab = (uint16_t*)(smem + HS_LEG_AT);
+    uint16_t* qitems = (uint16_t*)(smem + HS_Q_AT);                     // range | offset << 8
     uint8_t* images = smem + HS_FIXED;
     const uint32_t stride = hs_image_bytes(J.max_huf_stream);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -1863,83 +1871,39 @@ __global__ void __launch_bounds__(HS_T, 2) k_huf_scout(JobDev J) {
     const HufItem it = J.huf_items[item0 + s];
     const uint8_t* g = J.comp + B.src_off + it.src_off;
     const uint32_t a = (uint32_t)((uintptr_t)g & 15);
-    const uint32_t bytes = ((a + it.src_size + 15u) >> 4) << 4;
     uint8_t* img = images + s * stride;                                 // 16 zero bytes, then the 16 B-aligned image of global memory
-#if defined(__CUDA_ARCH__)
-    const uint32_t mbar = (uint32_t)__cvta_generic_to_shared(&misc[56]);
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(mbar), "r"(4));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    const saddr_t mbar = to_saddr(&misc[56]);
+    if (tid == 0) mbar_init(mbar, 4);
     __syncthreads();
-    if (c == 0) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(mbar), "r"(bytes) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     :: "r"((uint32_t)__cvta_generic_to_shared(img + 16)), "l"(g - a), "r"(bytes), "r"(mbar) : "memory");
-    }
-#else
-    for (uint32_t k = c; k < (bytes >> 4); k += HS_C) ((uint4*)(img + 16))[k] = ((const uint4*)(g - a))[k];
-#endif
-    for (int i = tid; i < 64; i += HS_T) ((uint32_t*)weights)[i] = ((const uint32_t*)(J.huf_weights + (size_t)B.huf_slot * 256))[i];
-    const int nsym = (int)J.huf_meta[(size_t)B.huf_slot * 2] + 1, maxbits = (int)J.huf_meta[(size_t)B.huf_slot * 2 + 1];
+    if (c == 0) stage_stream(img + 16, g - a, ((a + it.src_size + 15u) >> 4) << 4, mbar);
+    const HufTree tree = huf_tree<HS_T>(J, B, sm.weights);
+    const int maxbits = tree.maxbits;
     __syncthreads();
     if (maxbits != 0) {                                                 // (a bad tree was flagged by k_build_tables)
-        huf_build_t1<HS_T>(weights, nsym, maxbits, t1, wcnt);
+        huf_build_t1<HS_T>(sm.weights, tree.nsym, maxbits, t1, sm.wcnt);
         huf_build_wide<HS_T, false>(t1, maxbits, nullptr, nullptr, 0u, 1u << HUF_W, tc);
     }
-    // a tree whose codes all have the same length never lets tracks merge -- and does not need to: the codeword boundaries
-    // are the multiples of that length
-    const bool fixed_len = !__syncthreads_or(tid < 128 && (tid & 15) >= 2 && (tid & 15) <= zc::HUF_MAX_BITS && wcnt[tid] != 0);
+    const bool fixed_len = huf_fixed_length(sm.wcnt);
     // (one thread reads the flag: another stream's kernel may set it at any moment, and the decision must be the CTA's)
     const bool skip = __syncthreads_or(maxbits == 0 || (tid == 0 && J.frame_bad[B.frame] != 0));
-#if defined(__CUDA_ARCH__)
-    {   // the bulk copies have landed (also before an early exit: the shared memory must not be handed on under them)
-        uint32_t done;
-        do {
-            asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                         : "=r"(done) : "r"(mbar), "r"(0) : "memory");
-        } while (!done);
-    }
-#endif
+    mbar_wait(mbar, 0);
     if (skip) return;
     if ((uint32_t)c < 16 + a) img[c] = 0;                                // bits below the stream start read as zero
-    const uint8_t last = img[16 + a + it.src_size - 1];
-    if (__syncthreads_or(last == 0)) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); return; }
-
-    // q = distance (in bits) from the top of the stream; smem bit position x = XTOP - q
-    const int P0 = 8 * (int)(it.src_size - 1) + zc::highbit32(last);
-    const int XTOP = (int)(16 + a) * 8 + P0;
-    int S = (P0 + HB_T - 1) / HB_T;                                     // fine ranges: exactly k_huf_decode_block's
-    if (S < 2 * MAXC) S = 2 * MAXC;
+    const HufShape shape = huf_stream_shape(img, a, it.src_size, HB_T); // (the fine ranges are k_huf_decode_block's)
+    if (__syncthreads_or(shape.last == 0)) { if (tid == 0) flag_error(J, B.frame, zc::E_HUF_STREAM); return; }
+    const int P0 = shape.P0, XTOP = shape.XTOP, S = shape.S;
     if (c == 0) { misc[24 + 4 * s] = (uint32_t)XTOP; misc[25 + 4 * s] = (uint32_t)P0; misc[26 + 4 * s] = (uint32_t)S; }
     const int ctop = c * HS_F * S;
     const bool active = ctop < P0;
     const saddr_t s_images = to_saddr(images), s_tc = to_saddr(tc), s_t1 = to_saddr(t1);
     const saddr_t s_comp = s_images + s * stride;
 
-    // (1) first stop: every candidate lands on its first codeword boundary at or past checkpoint 0
+    // (1) first stop at checkpoint 0
     uint64_t first = ~0ull, fcnt = 0;                                   // candidate -> landing offset / symbols so far (4 bits each)
     uint32_t live = 0;                                                  // landing offsets in use at the current checkpoint
     if (active) {
-        const int l0 = hs_checkpoint(ctop, S, P0, 0);
-        first = 0;
-        if (fixed_len) {
-            int q = ctop + (maxbits - ctop % maxbits) % maxbits, n = 0;
-            track_count(s_comp, s_tc, s_t1, maxbits, XTOP, q, n, l0);
-            first = (uint64_t)(uint32_t)(q - l0) * 0x1111111111111111ull;
-            fcnt = (uint64_t)(uint32_t)n * 0x1111111111111111ull;
-            live = 1u << (q - l0);
-        } else {
-            for (int k = 0; k < maxbits; k++) {
-                int q = ctop + k, n = 0;
-                track_count(s_comp, s_tc, s_t1, maxbits, XTOP, q, n, l0);
-                const uint32_t o = (uint32_t)(q - l0);
-                first |= (uint64_t)o << (4 * k);
-                fcnt |= (uint64_t)n << (4 * k);
-                live |= 1u << o;
-            }
-        }
-        if (maxbits < 16) first |= ~0ull << (4 * maxbits);              // candidates that cannot occur: dead (15)
+        const auto count = [&](int& q, int& n, int lim) { track_count(s_comp, s_tc, s_t1, maxbits, XTOP, q, n, lim); };
+        hb_first_stop(ctop, hs_checkpoint(ctop, S, P0, 0), maxbits, fixed_len, count, first, fcnt, live);
     }
     // (2) legs between checkpoints: the live tracks of ALL coarse ranges are work items dealt out evenly over the CTA
     auto slot_of = [](int leg) { return leg <= HB_NLEG ? leg : leg - HB_NLEG; };
@@ -2005,25 +1969,9 @@ __global__ void __launch_bounds__(HS_T, 2) k_huf_scout(JobDev J) {
         }
         if (maxbits < 16) fmap |= ~0ull << (4 * maxbits);
     }
-    // ---- compose the maps along each stream: inclusive scan in the warp, then the stream's two warp totals ----------------
-    uint64_t inc_map = fmap;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-        const uint64_t o = __shfl_up_sync(0xFFFFFFFFu, inc_map, d);
-        const bool need = lane >= d && !map_is_const(inc_map, maxbits);
-        if (__any_sync(0xFFFFFFFFu, need)) { if (need) inc_map = map_compose(inc_map, o); }
-    }
-    uint64_t exc_map = __shfl_up_sync(0xFFFFFFFFu, inc_map, 1);
-    if (lane == 0) exc_map = MAP_IDENTITY;
-    if (lane == 31) wmap[warp] = inc_map;
-    __syncthreads();
+    // ---- compose the maps along each stream ----------------------------------------------------------------------------------
     constexpr int WPS = HS_C / 32;                                      // warps per stream
-    if (tid < 4) {
-        uint32_t k = 0;
-        for (int w = tid * WPS; w < (tid + 1) * WPS; w++) { misc[16 + w] = k; k = (uint32_t)(wmap[w] >> (4 * k)) & 15u; }
-    }
-    __syncthreads();
-    const uint32_t ktrue = (uint32_t)(exc_map >> (4 * misc[16 + warp])) & 15u;     // this coarse range's true candidate
+    const uint32_t ktrue = hb_compose<WPS>(fmap, maxbits, (uint64_t*)sm.wcnt, misc + 16);       // this coarse range's true candidate
     // ---- the chain of the true track through the fine ranges: start offsets and symbols ------------------------------------
     uint32_t start[HS_F], cnt[HS_F];
 #pragma unroll
@@ -2077,135 +2025,59 @@ __global__ void __launch_bounds__(HS_T, 2) k_huf_scout(JobDev J) {
 // next stream's bytes are fetched (bulk asynchronous copy) while the current stream's output is flushed.
 __global__ void __launch_bounds__(HB_T, 3) k_huf_decode_block(JobDev J) {
     NAF_DYN_SMEM(unsigned char, smem);
-    uint16_t* t1 = (uint16_t*)smem;
-    uint8_t* weights = smem + 4096;
-    uint16_t* wcnt = (uint16_t*)(smem + 4096 + 256);
-    uint32_t* misc = (uint32_t*)(smem + 4096 + 512);                    // [56..57] mbarrier
-    uint32_t* t3 = (uint32_t*)(smem + 4864);
-    uint8_t* sout = smem + 4864 + 16384;
+    HufSmem& sm = *(HufSmem*)smem;
+    uint32_t* t3 = (uint32_t*)(smem + HB_T3_AT);
+    uint8_t* sout = smem + HB_SOUT_AT;
     uint32_t* scomp = (uint32_t*)(smem + HB_FIXED);
     const int tid = threadIdx.x;
-    (void)misc;
 
     const uint32_t item0 = blockIdx.x * 4u;                              // the block's four streams are four consecutive items
     const BlockDesc& B = J.blocks[J.huf_items[item0].block];
-#if defined(__CUDA_ARCH__)
-    const uint32_t mbar = (uint32_t)__cvta_generic_to_shared(&misc[56]);
-#endif
-    // stages stream `sidx`: the 16 B-aligned image of global memory, behind 16 bytes that stay zero (one bulk asynchronous copy)
+    const saddr_t mbar = to_saddr(&sm.misc[56]);
+    // stages stream `sidx`: the 16 B-aligned image of global memory, behind 16 bytes that stay zero
     auto stage = [&](uint32_t sidx) {
         const HufItem si = J.huf_items[item0 + sidx];
         const uint8_t* sg = J.comp + B.src_off + si.src_off;
         const uint32_t sa = (uint32_t)((uintptr_t)sg & 15);
-        const uint32_t bytes = ((sa + si.src_size + 15u) >> 4) << 4;
-#if defined(__CUDA_ARCH__)
-        if (tid == 0) {
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(mbar), "r"(bytes) : "memory");
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         :: "r"((uint32_t)__cvta_generic_to_shared(scomp + 4)), "l"(sg - sa), "r"(bytes), "r"(mbar) : "memory");
-        }
-#else
-        for (uint32_t c = tid; c < (bytes >> 4); c += HB_T) ((uint4*)scomp)[1 + c] = ((const uint4*)(sg - sa))[c];
-#endif
+        if (tid == 0) stage_stream(scomp + 4, sg - sa, ((sa + si.src_size + 15u) >> 4) << 4, mbar);
     };
-#if defined(__CUDA_ARCH__)
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(mbar), "r"(1));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
+    if (tid == 0) mbar_init(mbar, 1);
     __syncthreads();
-#endif
     stage(0);
-    for (int i = tid; i < 64; i += HB_T) ((uint32_t*)weights)[i] = ((const uint32_t*)(J.huf_weights + (size_t)B.huf_slot * 256))[i];
-    const int nsym = (int)J.huf_meta[(size_t)B.huf_slot * 2] + 1, maxbits = (int)J.huf_meta[(size_t)B.huf_slot * 2 + 1];
+    const HufTree tree = huf_tree<HB_T>(J, B, sm.weights);
+    const int maxbits = tree.maxbits;
     __syncthreads();
     if (maxbits != 0) {                                                 // (a bad tree was flagged by k_build_tables)
-        huf_build_t1<HB_T>(weights, nsym, maxbits, t1, wcnt);
-        huf_build_wide<HB_T, true>(t1, maxbits, nullptr, t3, 0u, 1u << HUF_W);
+        huf_build_t1<HB_T>(sm.weights, tree.nsym, maxbits, sm.t1, sm.wcnt);
+        huf_build_wide<HB_T, true>(sm.t1, maxbits, nullptr, t3, 0u, 1u << HUF_W);
     }
     // (one thread reads the flag: k_huf_scout flags every stream it refuses, and another stream's kernel may set it at any
     // moment -- the decision must be the CTA's)
     const bool skip = __syncthreads_or(maxbits == 0 || (tid == 0 && J.frame_bad[B.frame] != 0));
     for (uint32_t sidx = 0; sidx < 4u; sidx++) {
-    const HufItem it = J.huf_items[item0 + sidx];
-    const uint32_t bound = skip ? 0u : J.huf_bounds[(size_t)(item0 + sidx) * HB_T + tid];     // output offset << 4 | start offset
-    const uint8_t* g = J.comp + B.src_off + it.src_off;
-    const uint32_t a = (uint32_t)((uintptr_t)g & 15);
-#if defined(__CUDA_ARCH__)
-    {   // the bulk copy of this stream has landed (also before an early exit: the shared memory must not be handed on under it)
-        uint32_t done;
-        do {
-            asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                         : "=r"(done) : "r"(mbar), "r"(sidx & 1u) : "memory");
-        } while (!done);
-    }
-#endif
-    if (skip) break;
-    if ((uint32_t)tid < 16 + a) ((uint8_t*)scomp)[tid] = 0;              // bits below the stream start read as zero
-    __syncthreads();
+        const HufItem it = J.huf_items[item0 + sidx];
+        const uint32_t bound = skip ? 0u : J.huf_bounds[(size_t)(item0 + sidx) * HB_T + tid];     // output offset << 4 | start offset
+        const uint8_t* g = J.comp + B.src_off + it.src_off;
+        const uint32_t a = (uint32_t)((uintptr_t)g & 15);
+        mbar_wait(mbar, sidx & 1u);                                     // the bulk copy of this stream has landed
+        if (skip) break;
+        if ((uint32_t)tid < 16 + a) ((uint8_t*)scomp)[tid] = 0;          // bits below the stream start read as zero
+        __syncthreads();
 
-    // q = distance (in bits) from the top of the stream; smem bit position x = XTOP - q.  (k_huf_scout refused a zero last byte.)
-    const uint8_t last = ((const uint8_t*)scomp)[16 + a + it.src_size - 1];
-    const int P0 = 8 * (int)(it.src_size - 1) + zc::highbit32(last);
-    const int XTOP = (int)(16 + a) * 8 + P0;
-    int S = (P0 + HB_T - 1) / HB_T;
-    if (S < 2 * MAXC) S = 2 * MAXC;
-    const int q0 = tid * S;
-    const int qe = (q0 + S < P0) ? q0 + S : P0;
-    uint8_t* dst = J.lit + B.lit_base + it.dst_off;
-    const uint32_t a2 = (uint32_t)((uintptr_t)dst & 15);
-    if (q0 < P0) {
-        // write pass: from the true start to the first boundary at or past the end of the range.  Bytes go out as aligned 4-byte
-        // words assembled in a register pair; the ragged head and tail (words shared with the neighbouring ranges) as bytes.
-        const saddr_t s_comp = to_saddr(scomp), s_t3 = to_saddr(t3), s_t1 = to_saddr(t1);
-        saddr_t out = to_saddr(sout) + a2 + (bound >> 4);
-        int q = q0 + (int)(bound & 15u);
-        int rem = qe - q;
-        Win w;
-        win_init(w, s_comp, XTOP - q);
-        const int sh1 = HUF_W - maxbits;
-        while ((out & 3u) && rem > 0) {                                 // head: single symbols up to a word boundary
-            const uint32_t e = lds16(s_t1 + 2 * (win_peek(w) >> sh1));
-            sts8(out, e >> 8); out++;
-            rem -= (int)(e & 0xFFu);
-            win_consume(w, (int)(e & 0xFFu));
-        }
-        uint32_t acc_lo = 0, acc_hi = 0;
-        int pc = 0;                                                     // bytes waiting in acc
-        while (rem > HUF_W) {
-            const uint32_t e = lds32(s_t3 + win_peek_x4(w));
-            const int n = (int)(e >> 28), len = (int)(e >> 24) & 15;
-            const uint32_t sy = e & 0xFFFFFFu;
-            acc_lo |= sy << (8 * pc);
-            acc_hi |= __funnelshift_l(sy, 0u, 8 * pc);                  // the bits that fall off the top of acc_lo
-            pc += n;
-            if (pc >= 4) { sts32(out, acc_lo); out += 4; acc_lo = acc_hi; acc_hi = 0; pc -= 4; }
-            rem -= len;
-            win_consume(w, len);
-        }
-        while (rem > 0) {                                               // the last symbols, one at a time
-            const uint32_t e = lds16(s_t1 + 2 * (win_peek(w) >> sh1));
-            acc_lo |= (e >> 8) << (8 * pc);
-            pc++;
-            if (pc == 4) { sts32(out, acc_lo); out += 4; acc_lo = 0; pc = 0; }
-            rem -= (int)(e & 0xFFu);
-            win_consume(w, (int)(e & 0xFFu));
-        }
-        for (int k = 0; k < pc; k++) sts8(out + k, acc_lo >> (8 * k));
-    }
-    __syncthreads();
-    if (sidx + 1 < 4u) stage(sidx + 1);                                 // the next stream's bytes travel while this one's output is flushed
-    {
-        // ---- flush: sout[a2 + k] -> dst[k]; aligned 16 B chunks in the middle, bytes at the ragged ends ----------------
-        const uint32_t n = it.n_sym, endb = a2 + n;
-        uint8_t* dal = dst - a2;
-        const uint32_t first_full = a2 ? 1u : 0u, last_full = endb >> 4;     // chunks [first_full, last_full) are complete
-        for (uint32_t c = first_full + tid; c < last_full; c += HB_T) ((uint4*)dal)[c] = ((const uint4*)sout)[c];
-        if (a2) { uint32_t hend = endb < 16 ? endb : 16; for (uint32_t k = a2 + tid; k < hend; k += HB_T) dal[k] = sout[k]; }
-        if (last_full >= first_full && (last_full << 4) < endb && !(a2 && last_full == 0))
-            for (uint32_t k = (last_full << 4) + tid; k < endb; k += HB_T) dal[k] = sout[k];
-    }
-    __syncthreads();                                                    // the output image is overwritten by the next stream
+        const HufShape shape = huf_stream_shape((const uint8_t*)scomp, a, it.src_size, HB_T);     // (k_huf_scout refused a zero last byte)
+        const int P0 = shape.P0, S = shape.S;
+        const int q0 = tid * S;
+        const int qe = (q0 + S < P0) ? q0 + S : P0;
+        uint8_t* dst = J.lit + B.lit_base + it.dst_off;
+        const uint32_t a2 = (uint32_t)((uintptr_t)dst & 15);
+        // write pass: from the exact start k_huf_scout found to the first boundary at or past the end of the range
+        if (q0 < P0)
+            hb_write_range(to_saddr(scomp), to_saddr(t3), to_saddr(sm.t1), maxbits, shape.XTOP, q0 + (int)(bound & 15u), qe,
+                           to_saddr(sout) + a2 + (bound >> 4));
+        __syncthreads();
+        if (sidx + 1 < 4u) stage(sidx + 1);                             // the next stream's bytes travel while this one's output is flushed
+        flush_image<HB_T>(dst, sout, a2, it.n_sym);
+        __syncthreads();                                                // the output image is overwritten by the next stream
     }
 }
 
@@ -3336,7 +3208,7 @@ Launch choose_paths(JobDev& J, const fw::JobPlan& pl, const Overrides& ov, uint3
     // archive): one CTA per STREAM, the four of a block as a thread-block cluster that shares the table construction through
     // DSMEM -- four times the CTAs in flight and no second launch, which is what latency wants (k_huf_decode_big).
     L.huf_per_block = J.n_huf_big / 4 >= (J.huf_block_min ? J.huf_block_min : 296u);
-    L.huf_small_smem = huf_fixed_smem(HUF_T_SMALL) + ((J.max_huf_small + 15 + 16 + 16 + 15) & ~15u);
+    L.huf_small_smem = HUF_SMALL_FIXED + ((J.max_huf_small + 15 + 16 + 16 + 15) & ~15u);
     L.huf_big_smem = hb_smem_bytes(J.max_huf_stream);
     L.huf_scout_smem = hs_smem_bytes(J.max_huf_stream);
     // a job with both kinds of blocks (a FASTQ archive: 2 x 10^6 tiny blocks and the ~130 big blocks of the ids, each one chain of
@@ -3377,7 +3249,7 @@ int launch_zstd_stage(const JobDev& J, const Launch& L, const Streams& S, StageE
         const bool side = st2 && st3 && L.huf_side;
         if (side) {
             cudaEventRecord(S.fork[1], sb); cudaStreamWaitEvent(st3, S.fork[1], 0);
-            NAF_LAUNCH((k_huf_decode<HUF_T_SMALL>), J.n_huf_items - J.n_huf_big, HUF_T_SMALL, L.huf_small_smem, st3, J, J.huf_items + J.n_huf_big); launches++;
+            NAF_LAUNCH(k_huf_decode_small, J.n_huf_items - J.n_huf_big, HUF_T_SMALL, L.huf_small_smem, st3, J, J.huf_items + J.n_huf_big); launches++;
             cudaEventRecord(S.join[1], st3);
         }
         if (J.n_huf_big) {   // items [0, n_huf_big): the streams of 4-stream blocks, four consecutive items (= one cluster) per block
@@ -3396,7 +3268,7 @@ int launch_zstd_stage(const JobDev& J, const Launch& L, const Streams& S, StageE
         }
         if (side) cudaStreamWaitEvent(sb, S.join[1], 0);
         else if (J.n_huf_items > J.n_huf_big) {
-            NAF_LAUNCH((k_huf_decode<HUF_T_SMALL>), J.n_huf_items - J.n_huf_big, HUF_T_SMALL, L.huf_small_smem, sb, J, J.huf_items + J.n_huf_big); launches++;
+            NAF_LAUNCH(k_huf_decode_small, J.n_huf_items - J.n_huf_big, HUF_T_SMALL, L.huf_small_smem, sb, J, J.huf_items + J.n_huf_big); launches++;
         }
     }
     if (st2) cudaEventRecord(S.join[0], st2);

@@ -39,8 +39,7 @@ struct JobDev {
     uint32_t* lz_blocker;             // per match: the unfinished match it was last found waiting for (0xFFFFFFFF: none yet)
     uint32_t* frame_bad;              // per frame: non-zero once anything in it failed validation
     uint32_t* status;                 // OR of zc::E_* bits
-    unsigned long long* debug;        // optional per-CTA phase clocks of k_huf_decode (NAFGPU_DEBUG_HUF=1), else null
-    unsigned long long* debug_seq;    // optional cycle accounting of k_decode_sequences (8 counters), else null
+    unsigned long long* debug_seq;    // optional cycle accounting of k_decode_sequences and k_lz_small (8 counters), else null
     uint32_t* lz_list[3];             // rotating worklists of matches still pending (n_seq entries each)
     uint32_t* lz_count;               // [3] their lengths
     uint32_t* lz_rounds;              // rounds k_lz_first + k_lz_resolve ran (statistics)
@@ -64,7 +63,7 @@ struct JobDev {
     const zf::HufItem* huf_items;     // one per Huffman bitstream
     uint32_t* huf_bounds;             // [n_huf_big x 256] k_huf_scout -> k_huf_decode_block: output offset << 4 | start offset of every range
     uint32_t huf_block_min;           // host: launch configuration: jobs with at least this many big blocks use k_huf_decode_block (0: default)
-    uint32_t n_huf_items, n_huf_big;  // items [0, n_huf_big): streams of 4-stream blocks, four per block (k_huf_decode_big, one cluster per block); the rest: k_huf_decode<128>
+    uint32_t n_huf_items, n_huf_big;  // items [0, n_huf_big): streams of 4-stream blocks, four per block (k_huf_scout + k_huf_decode_block, or k_huf_decode_big); the rest: k_huf_decode_small
     uint32_t max_huf_stream, max_huf_small;   // largest stream (bytes) in each class
     const zf::FsTile* fs_tiles;       // tiles of the frames with more than FS_BIG_FRAME blocks (host-filled)
     const zf::FsBigFrame* fs_big;
@@ -111,7 +110,7 @@ static_assert(sizeof(JobWords) == 42 * 4, "JobWords: 42 fixed words");
 //                             test_parity, test_zstd_sequences, test_job_plan
 //   NAFGPU_WALK_SPLIT=n       n > 0: walk sections in parts of n blocks, even short ones; n <= 0: never in parts
 //                             test_parity, test_zstd_sequences, test_job_plan
-//   NAFGPU_DEBUG_HUF          any value: cycle counters of the Huffman and sequence kernels on stderr at fetch (tools/dbg_huf.py)
+//   NAFGPU_DEBUG_HUF          any value: cycle counters of k_decode_sequences and k_lz_small on stderr at fetch (tools/lat_debug.py)
 //   NAFGPU_DEBUG_PREP         any value: phase times of the job's preparation on stderr (tools/prep_probe.py)
 struct Overrides {
     std::optional<uint32_t> tiny_blocks, lz_small, lz_flow, lz_flow_early, fin_cost_us, huf_block_min, fs_tile;

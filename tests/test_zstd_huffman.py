@@ -1,9 +1,9 @@
-"""The Huffman literal decoders (k_build_tables<1>, k_huf_decode<128>, k_huf_decode_block, k_huf_decode_big) on literals
+"""The Huffman literal decoders (k_build_tables<1>, k_huf_decode_small, k_huf_decode_block, k_huf_decode_big) on literals
 sections built to order (tests/_zhuf.py): trees of every depth, fixed-length trees, both weight forms at their count limits,
 stream lengths around the kernels' range and size boundaries, treeless reuse, and the sections a decoder must refuse.
 Each case reads its section back with the plain reader to prove that its edge is there, then checks that the reader,
 libzstd and the device agree on every byte, under both big-stream kernels (NAFGPU_HUF_BLOCK_MIN=1: one CTA per block;
-1000000: four clustered CTAs).  Streams of at most 2048 symbols go to k_huf_decode<128> whatever the setting."""
+1000000: four clustered CTAs).  Streams of at most 2048 symbols go to k_huf_decode_small whatever the setting."""
 import numpy as np
 import pytest
 
@@ -15,7 +15,7 @@ import nafcodec_b200 as N
 from _harness import BACKENDS, assert_same_as_oracle, library
 from conftest import read_golden
 
-SMALL_MAX = 2048                           # symbols per stream up to which a 4-stream block is decoded by k_huf_decode<128>
+SMALL_MAX = 2048                           # symbols per stream up to which a 4-stream block is decoded by k_huf_decode_small
 RANGE_MIN_BITS = 256 * 2 * H.MAX_BITS      # big-stream kernels: 256 ranges of at least 2 * 11 bits
 ASCII0 = 48                                # trees over printable symbols 48.. (up to 64 of them) make valid TEXT payloads
 
@@ -152,8 +152,8 @@ def test_writer_sections_decode_under_libzstd():
 
 # ---- depths and fixed-length trees ----------------------------------------------------------------------------------
 def _depth_sections(rng, w, **kw):
-    """One tree in three sections: a 1-stream section (k_huf_decode<128>), a 4-stream section of short streams (also
-    k_huf_decode<128>) and one of 6000 symbols per stream (a big-stream kernel)."""
+    """One tree in three sections: a 1-stream section (k_huf_decode_small), a 4-stream section of short streams (also
+    k_huf_decode_small) and one of 6000 symbols per stream (a big-stream kernel)."""
     out = []
     for n, streams in ((700, 1), (4000, 4), (24_000, 4)):
         d = _data(rng, w, n)
@@ -262,7 +262,7 @@ def _bits_stream(seg, target_bits):
 def test_stream_geometry(backend, huf_env):
     rng = np.random.default_rng(14)
     w = GEO_TREE
-    # symbols per stream at the small/big classification: 2047, 2048 (k_huf_decode<128>), 2049 (big); regen 8193 is big too
+    # symbols per stream at the small/big classification: 2047, 2048 (k_huf_decode_small), 2049 (big); regen 8193 is big too
     for regen in (4 * 2047, 4 * 2048, 4 * 2048 + 1, 4 * 2049):
         d = _data(rng, w, regen)
         (lit,) = _lits(backend, [(d, H.literals_section(d, w))], f"regen {regen}")
